@@ -2,6 +2,7 @@
 """Benchmark of the B200-native hyper-greco proving path (contract: see the task statement / DESIGN.md "Measurement").
 
     python bench.py --gpus 1 --steps K --warmup W                 # our arm
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # + the outputs of the last timed step, to compare two builds
     python bench.py --impl reference --gpus 1 --steps K --warmup W   # CPU arm: the oracle port on the host cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # one rank per GPU, weak scaling
 
@@ -32,6 +33,7 @@ UNIT = "proofs/s"
 DEFAULT_CONFIG = "32768_16x59_65537"
 NOMINAL_HBM_GBS = 8000.0   # the ~8 TB/s the north star quotes; the measured copy bandwidth is in MEASURED_PEAKS.json
 WITNESS_POOL = 8           # distinct synthetic witnesses per rank (generated on the device, hg_bfv_witness_generate)
+DUMP_LIMIT_BYTES = 64 << 20   # --dump-outputs writes at most this much
 
 
 def bench_config(args, P, nv, m):
@@ -234,10 +236,11 @@ class ProofSlot:
         return [(self.np.zeros((0, el), self.np.uint64), self.np.zeros(el, self.np.uint64)), (point, value)]
 
     def resident(self):
-        """the `GKR prove` span: gkr::prove_gkr on device-resident circuit values"""
+        """the `GKR prove` span: gkr::prove_gkr on device-resident circuit values. What its caller receives (the transcript holding
+        the proof, the input claims) is kept in `last` until the next proof of this slot."""
         tr = self.api.Keccak256Transcript(self.field_id)
         tr.squeeze_challenges(self.prover.ct0is_log2_size)
-        self.prover.circuit.prove_gkr(self.out_claims, tr, self.api.MODE_PREFETCH)
+        self.last = (tr, self.prover.circuit.prove_gkr(self.out_claims, tr, self.api.MODE_PREFETCH))
         return tr
 
     def e2e(self, which=None):
@@ -471,6 +474,7 @@ def run_ours(args):
     wall = time.perf_counter() - w0
     clocks = sampler.stop()
     ms = e0.elapsed_time(e1)
+    last_step = [s.last for s in slots]
     t = torch.tensor([ms, wall * 1000.0], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -590,6 +594,8 @@ def run_ours(args):
                 "gpu_launches": int(launches_per_proof * args.steps * B), "gpu_launches_per_proof": int(launches_per_proof),
                 "single_proof_latency_ms": latency_ms, "interactive_mode": interactive_ms, "wall_ms_per_step": wall_ms / args.steps, "proof_bytes": proof_len, "spin_up_steps": spin_up, "witness_gen_ms_per_witness": witness_gen_ms,
                 "host_phases_us": host_phases, "roofline": roofline, "cpu_baseline": cpu, "shard": shard}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step, f"rank{rank}_" if world > 1 else "")
     barrier()
     for s in slots:
         s.close()
@@ -597,6 +603,32 @@ def run_ours(args):
         dist.destroy_process_group()
     if line is not None:
         print(json.dumps(line))
+
+
+def u64_as_f64(words):
+    """uint64 limbs -> float64 [n, 2] (low, high 32 bits of each limb): exact, so two dumps can be compared value for value"""
+    import numpy as np
+    w = np.ascontiguousarray(words, dtype=np.uint64).reshape(-1)
+    return np.stack([w & np.uint64(0xFFFFFFFF), w >> np.uint64(32)], -1).astype(np.float64)
+
+
+def dump_outputs(out_dir, last_step, prefix=""):
+    """--dump-outputs: what every in-flight proof of the last timed step handed to its caller, as <prefix>proof_<slot>.npy (the proof
+    bytes, float32) and <prefix>input_claims_<slot>.npy (point then value of every claim on every input node, in node order, through
+    u64_as_f64). Slots are written in order while the total stays within DUMP_LIMIT_BYTES."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for k, (tr, claims) in enumerate(last_step):
+        proof = np.frombuffer(tr.into_proof(), np.uint8).astype(np.float32)
+        words = [a.reshape(-1) for node in claims for pt, val in node for a in (pt, val)]
+        cl = u64_as_f64(np.concatenate(words) if words else np.zeros(0, np.uint64))
+        if total + proof.nbytes + cl.nbytes > DUMP_LIMIT_BYTES:
+            print(f"bench.py: --dump-outputs stops after {k} of {len(last_step)} slots ({DUMP_LIMIT_BYTES >> 20} MB)", file=sys.stderr)
+            break
+        np.save(os.path.join(out_dir, f"{prefix}proof_{k}.npy"), proof)
+        np.save(os.path.join(out_dir, f"{prefix}input_claims_{k}.npy"), cl)
+        total += proof.nbytes + cl.nbytes
 
 
 def run_shard(args):
@@ -650,7 +682,13 @@ def main():
     ap.add_argument("--no-shard", action="store_true", help="skip the sharded measurement that a multi-GPU run adds to its line")
     ap.add_argument("--field", default="goldilocks", choices=["goldilocks", "bn254"], help="BASELINE.json config 5: --field bn254")
     ap.add_argument("--pool", type=int, default=WITNESS_POOL, help="distinct witnesses per rank (<= %d)" % WITNESS_POOL)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what every proof of the last timed step returned "
+                    "as DIR/proof_<slot>.npy and DIR/input_claims_<slot>.npy (the inputs are the same from run to run with the same arguments)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.shard):
+        ap.error("--dump-outputs writes the outputs of the default GPU run, not of --impl reference or --shard")
     if args.impl == "reference":
         run_reference(args)
     elif args.shard:
