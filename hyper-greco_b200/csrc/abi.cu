@@ -523,6 +523,9 @@ template <class FP> struct FieldOpsT : IFieldOps {
     }
     void mle_eval_batch(DeviceCtx* dev, const void* d_tables, size_t n_tables, size_t stride, size_t num_vars, const uint64_t* point_ext, uint64_t* out_ext) override {
         const size_t n = (size_t)1 << num_vars;
+        // k_dot_eq reads a table four entries at a time with 16-byte vector loads from its first entry on (num_vars >= 2)
+        if (num_vars >= 2 && (((uintptr_t)d_tables | (stride * sizeof(B))) & 15) != 0)
+            throw std::runtime_error("hg_mle_eval_batch: every table must start 16-byte aligned (d_tables and stride * element size)");
         cudaStream_t s = dev->stream;
         // work buffers persist across calls (a cudaMalloc / cudaFree pair per buffer costs more than the evaluation)
         DevBuf<X>&pt = mle_pt_, &eq = mle_eq_, &partials = mle_partials_, &out = mle_out_;

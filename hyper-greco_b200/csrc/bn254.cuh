@@ -52,6 +52,12 @@ HG_HD void fr_sub_mod_inplace(u64* a) {
 #if defined(__CUDACC__)
 // ---- device arithmetic with PTX carry chains (the portable C below compiles to compare/select sequences: 724 vs 481
 // instructions per multiplication). Same results: Montgomery CIOS, fully reduced outputs.
+// Contracts (raw Montgomery limbs; tests/test_field_probe.py checks each one at its boundaries):
+//   fr_cond_sub_dev(t)           t < 2r as 5 limbs; output t mod r (t == r gives 0).
+//   fr_add_dev, fr_sub_dev       a, b < r; output < r. No input may be lazy: a + b < 2r < 2^255 is what fr_cond_sub_dev takes.
+//   fr_mul_dev, fr_mul_dev32     a, b < r; output a b R^-1 mod r, < r. In fr_mul_dev the running value stays below 2r, so
+//                                t + a b_i + m r < 2^65 r < 2^320 never carries into t5 (r < 2^254): t5 and the t4 handed to
+//                                fr_cond_sub_dev are 0 for inputs in contract.
 __device__ __forceinline__ fr fr_cond_sub_dev(u64 t0, u64 t1, u64 t2, u64 t3, u64 t4) {  // (t4:t3:t2:t1:t0) < 2r  ->  mod r
     u64 s0, s1, s2, s3, bw;
     asm("sub.cc.u64 %0, %5, %9; subc.cc.u64 %1, %6, %10; subc.cc.u64 %2, %7, %11; subc.cc.u64 %3, %8, %12; subc.u64 %4, %13, 0;"

@@ -26,7 +26,7 @@ constexpr u64 GL_EPS = 0xFFFFFFFFULL;  // 2^64 mod p
 HG_HD u64 gl_add(u64 a, u64 b) {
     u64 s = a + b;
 #if defined(__CUDA_ARCH__)
-    if (s < a) s += GL_EPS;       // wrapped: + 2^64 = + EPS (result < p, see DESIGN.md)
+    if (s < a) s += GL_EPS;       // wrapped: + 2^64 = + EPS. a, b < p gives s = a + b - 2^64 <= p - 2 - EPS, so s + EPS < p
     else if (s >= GL_P) s -= GL_P;
 #else
     s += (0 - (u64)(s < a)) & GL_EPS;   // after a wrap the sum is < p - EPS, so at most one of the two corrections applies
@@ -137,13 +137,26 @@ HG_HD gl2 gl2_inv(gl2 a) {
 //   * table elements in memory are always CANONICAL (< p);
 //   * products are accumulated UNREDUCED in a 160-bit accumulator (lo, hi, carry word) and reduced once;
 //   * subtraction needs only its subtrahend canonical; results are "lazy" (any representative in [0, 2^64)).
+// Contracts, per primitive ("lazy" = any u64, "canonical" = < p). tests/test_field_probe.py checks each one at its limit.
+//   acc_mad(a, x, y), acc_add(a, x)   x, y lazy. acc_mad adds at most 1 to e4 and at most 2 to o2, acc_add at most 1 to e4.
+//   acc_reduce                        exact and canonical for any e01, e23, o01, o2 and e4 <= 2^32 - 3. From acc_zero / acc_from
+//                                     that is n acc_mad and m acc_add with 2n <= 2^32 - 1 and n + m <= 2^32 - 3: 2^31 - 1 products.
+//   xacc_mad, xacc_mad_base           x, y lazy. xacc_mad adds one product to a00 and a11 and two to ax, xacc_mad_base one to
+//                                     a00 and ax. xacc_reduce adds one more product to (a copy of) a00, which must have room
+//                                     for it. Output canonical.
+//   gl_sub_cs(a, b)                   b canonical, a lazy; output lazy, canonical when a is.
+//   gl_add_cs(a, b)                   a canonical, b lazy; output lazy (may be p, a non-canonical zero).
+//   gl_canon(r)                       r lazy; output canonical.
+//   gl_mul_fast, gl2_mul_fast, GlField::fmul_any   operands lazy; output canonical.
+//   gl2_fold, GlField::fold_scaled    canonical in (a0, a1, r, c, cr and fold_aux's r7), canonical out.
+//   GlField::slope                    canonical in; output canonical. at_m1, q_at_m1: canonical in, lazy out.
 #if defined(__CUDACC__)
 // Unreduced sum of 64x64-bit products, kept as TWO column accumulators so that every 32x32 partial product lands on an
 // aligned 64-bit register pair and one IMAD.WIDE.U32 (with carry) adds it:
 //     value = (e01 + 2^64 e23 + 2^128 e4)  +  2^32 (o01 + 2^64 o2)
 // "even" columns take x0*y0 (weight 2^0) and x1*y1 (2^64), "odd" columns the cross products (2^32). acc_mad is
 // 4 IMAD.WIDE.U32 + 3 carry adds (the single-accumulator form needed 15 instructions); the columns are merged once, in
-// acc_reduce. Capacity: 2^31 products.
+// acc_reduce. Capacity: 2^31 - 1 products (o2 takes up to 2 carries per product), e4 <= 2^32 - 3 at acc_reduce.
 struct acc192 {
     u64 e01, e23, o01;
     u32 e4, o2;
@@ -200,20 +213,22 @@ __device__ __forceinline__ u64 gl_canon(u64 r) {
 }
 // value mod p, canonical.  2^64 = 2^32 - 1, 2^96 = -1, 2^128 = -2^32 (mod p)
 __device__ __forceinline__ u64 acc_reduce(const acc192& a) {
-    // merge the odd columns: (lo, hi, c) = E + 2^32 O, c < 2^31
+    // merge the odd columns: (lo, hi, c) = E + 2^32 O. (e1, e2, e3) + (o0, o1, o2) < 2^97 carries at most 1 into c, so
+    // c <= e4 + 1 <= 2^32 - 2
     u32 e0 = (u32)a.e01, e1 = (u32)(a.e01 >> 32), e2 = (u32)a.e23, e3 = (u32)(a.e23 >> 32), c = a.e4;
     const u32 o0 = (u32)a.o01, o1 = (u32)(a.o01 >> 32);
     asm("add.cc.u32 %0, %0, %4; addc.cc.u32 %1, %1, %5; addc.cc.u32 %2, %2, %6; addc.u32 %3, %3, 0;"
         : "+r"(e1), "+r"(e2), "+r"(e3), "+r"(c) : "r"(o0), "r"(o1), "r"(a.o2));
     const u64 lo = e0 | ((u64)e1 << 32);
-    const u64 s1 = e3 | ((u64)c << 32);  // hi_hi + c * 2^32, canonical (< 2^63)
+    const u64 s1 = e3 | ((u64)c << 32);  // hi_hi + c * 2^32 <= (2^32 - 2) 2^32 + 2^32 - 1 = p - 2: canonical, as gl_sub_cs needs
     u64 t0 = gl_sub_cs(lo, s1);
-    const u64 t1 = ((u64)e2 << 32) - e2;  // hi_lo * (2^32 - 1) < 2^64 - 2^33 + 2
+    const u64 t1 = ((u64)e2 << 32) - e2;  // hi_lo * (2^32 - 1) <= 2^64 - 2^33 + 1
     u64 r;
     u32 cy;
     asm("add.cc.u64 %0, %2, %3; addc.u32 %1, 0, 0;" : "=l"(r), "=r"(cy) : "l"(t0), "l"(t1));
-    r += (u64)(0u - cy);  // cannot wrap twice (see DESIGN.md)
-    return gl_canon(r);
+    // on a carry r = t0 + t1 - 2^64 <= t1 - 1 <= 2^64 - 2^33, so r + EPS < 2^64 - 2^32 < p cannot wrap twice
+    r += (u64)(0u - cy);
+    return gl_canon(r);  // r < 2^64 < 2p: one conditional subtract makes it canonical
 }
 // extension-field accumulator: sum of products x*y kept as three unreduced base accumulators
 struct xacc {

@@ -208,7 +208,8 @@ int hg_sumcheck_prove(hg_ctx* ctx, int arity, size_t n_terms, size_t num_vars, c
                       const uint64_t* claim_ext, hg_transcript* t, int mode, uint64_t* out_point, uint64_t* out_evals);
 
 /* ---- batched multilinear evaluation: MultilinearPoly::evaluate (lasso/src/memory_checking/mod.rs:80-93) ---------
- *      d_tables: n_tables base tables of 2^num_vars elements (stride elements apart); point: num_vars ext elements (host). */
+ *      d_tables: n_tables base tables of 2^num_vars elements (stride elements apart); point: num_vars ext elements (host).
+ *      For num_vars >= 2 every table must start 16-byte aligned (Goldilocks: an even stride); otherwise this is an error. */
 int hg_mle_eval_batch(hg_ctx* ctx, const void* d_tables, size_t n_tables, size_t stride, size_t num_vars, const uint64_t* point_ext,
                       uint64_t* out_ext);
 

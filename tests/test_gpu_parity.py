@@ -51,13 +51,42 @@ def test_device_field_arithmetic(api, ctx, oracle):
         assert (api.field_selftest(ctx, 2, a[i:i + 1], b[i:i + 1])[0] == oracle.field_op(0, 2, a[i], b[i])).all()
 
 
-@pytest.mark.parametrize("arity,nterms,nv", [(1, 2, 1), (1, 7, 4), (2, 1, 1), (2, 3, 2), (2, 5, 3), (2, 12, 11), (1, 25, 12), (2, 50, 9)])
+FILLS = ("random", "max", "lazy_pairs")
+
+
+def fill_params(shapes, fills=FILLS):
+    """shape x fill; the random fill keeps the shape's own test id."""
+    return [pytest.param(*sh, f, id="-".join(map(str, sh)) + ("" if f == "random" else "-" + f)) for f in fills for sh in shapes]
+
+
+def fill_tables(rng, fill, shape, consts, rand):
+    """Sumcheck inputs at the extremes, from consts = the elements (0, p - 2, p - 1) in the field's limb layout: `max` is every
+    entry p - 1; `lazy_pairs` makes every pair (lo, hi) either (p - 1, p - 2) or (0, p - 1), whose line through the pair is p
+    (a non-canonical zero) at X = -1 resp. takes the borrow at X = -1 and at infinity."""
+    if fill == "random":
+        return rand(shape)
+    idx = np.full(shape, 2)
+    if fill == "lazy_pairs":
+        kind = rng.integers(0, 2, size=shape[:-1] + (shape[-1] // 2,))
+        idx[..., 0::2] = np.where(kind == 0, 2, 0)
+        idx[..., 1::2] = np.where(kind == 0, 1, 2)
+    return consts[idx]
+
+
+# the last shapes give more pairs than k_sc_round's grid (8 blocks of 256 threads per SM): every thread loops
+SC_SHAPES = [(1, 2, 1), (1, 7, 4), (2, 1, 1), (2, 3, 2), (2, 5, 3), (2, 12, 11), (1, 25, 12), (2, 50, 9), (2, 2, 20), (1, 3, 20)]
+
+
+@pytest.mark.parametrize("arity,nterms,nv,fill", fill_params(SC_SHAPES))
 @pytest.mark.parametrize("mode", [0, 1])
-def test_sumcheck_matches_oracle(api, ctx, oracle, arity, nterms, nv, mode):
+def test_sumcheck_matches_oracle(api, ctx, oracle, arity, nterms, nv, fill, mode):
     rng = np.random.default_rng(nv * 100 + nterms)
-    tables = rng.integers(0, GL_P, size=(nterms * arity, 1 << nv), dtype=np.uint64)
+    tables = fill_tables(rng, fill, (nterms * arity, 1 << nv), np.array([0, GL_P - 2, GL_P - 1], np.uint64),
+                         lambda sh: rng.integers(0, GL_P, size=sh, dtype=np.uint64))
     coeffs = rand_ext(rng, nterms)
     claim = rand_ext(rng, 1)[0]
+    if fill == "max":
+        coeffs[:], claim[:] = GL_P - 1, GL_P - 1
     oproof, te, orr, ofe = oracle.sumcheck_prove(0, arity, coeffs, tables, nv, claim)
     d = api.DeviceBuffer.from_numpy(ctx, tables)
     t = api.Keccak256Transcript()
@@ -91,16 +120,38 @@ def test_sumcheck_wire_variants(api, oracle, opts):
         c.close()
 
 
+def _mle_cases(rng, rand_table, top_table, rand_point, edge_point):
+    """(label, num_vars, n_tables, stride, tables [n_tables, stride], point). nv = 12 is where the low half of the eq split
+    covers the whole table, nv = 21 where k_dot_eq's grid is capped at 2 blocks per SM; stride > 2^nv leaves gaps between
+    the tables; several tables run as grid.y."""
+    cases = []
+    for nv in (1, 5, 13):
+        cases.append((f"random nv={nv}", nv, 3, 1 << nv, rand_table((3, 1 << nv)), rand_point(nv)))
+    for nv, nt, extra in ((12, 2, 0), (21, 2, 0), (7, 5, 10), (13, 4, 4096)):
+        stride = (1 << nv) + extra
+        cases.append((f"nv={nv} tables={nt} stride={stride}", nv, nt, stride, rand_table((nt, stride)), rand_point(nv)))
+    for nv in (3, 12, 14):
+        cases.append((f"max nv={nv}", nv, 2, 1 << nv, top_table((2, 1 << nv)), rand_point(nv)))
+        cases.append((f"max at 0/1/p-1 point nv={nv}", nv, 2, 1 << nv, top_table((2, 1 << nv)), edge_point(rng, nv)))
+        cases.append((f"random at 0/1/p-1 point nv={nv}", nv, 1, 1 << nv, rand_table((1, 1 << nv)), edge_point(rng, nv)))
+    return cases
+
+
 def test_mle_eval_batch_matches_oracle(api, ctx, oracle):
     rng = np.random.default_rng(9)
-    for nv in (1, 5, 13):
-        tables = rng.integers(0, GL_P, size=(3, 1 << nv), dtype=np.uint64)
-        pt = rand_ext(rng, nv)
+    edge = lambda rng, nv: rng.choice(np.array([0, 1, GL_P - 1], np.uint64), size=(nv, 2))
+    for label, nv, nt, stride, tables, pt in _mle_cases(rng, lambda sh: rng.integers(0, GL_P, size=sh, dtype=np.uint64),
+                                                        lambda sh: np.full(sh, GL_P - 1, np.uint64), lambda nv: rand_ext(rng, nv), edge):
         d = api.DeviceBuffer.from_numpy(ctx, tables)
-        got = api.mle_eval_batch(ctx, d, 3, nv, pt)
-        for i in range(3):
-            assert (got[i] == oracle.mle_eval(0, tables[i], nv, pt)).all()
+        got = api.mle_eval_batch(ctx, d, nt, nv, pt, stride=stride)
+        for i in range(nt):
+            assert (got[i] == oracle.mle_eval(0, tables[i, :1 << nv], nv, pt)).all(), (label, i)
         d.free()
+    # the tables are read with 16-byte vector loads: an odd stride is refused before any launch
+    d = api.DeviceBuffer.from_numpy(ctx, np.zeros(2 * 17, np.uint64))
+    with pytest.raises(api.HgError, match="aligned"):
+        api.mle_eval_batch(ctx, d, 2, 4, rand_ext(rng, 4), stride=17)
+    d.free()
 
 
 def _prove_gpu(api, ctx, bounds, segs, nv, inp, mode=0, device_resident=False):
@@ -309,11 +360,29 @@ def test_bn254_lasso_node_sharded(api, ctx_bn, oracle, golden_dir):
     assert proof == oproof
 
 
-@pytest.mark.parametrize("log_n,batch", [(1, 3), (2, 1), (5, 4), (8, 2), (11, 3), (13, 2), (16, 3), (17, 1)])
-def test_ntt_matches_oracle(api, ctx, oracle, log_n, batch):
+def ntt_fill(rng, fill, shape, top, rand):
+    """NTT inputs at the extremes: all top (= p - 1), a single top in zeros, or the powers of 2^32 mod p (0, 2^32, 2^64 - 2^32 ...)."""
+    if fill == "random":
+        return rand(shape)
+    x = np.zeros(shape, dtype=object)
+    if fill == "max":
+        x[...] = top
+    elif fill == "single_max":
+        x[..., rng.integers(0, shape[-1])] = top
+    else:
+        x[...] = [pow(2, 32 * (j % 6), top + 1) for j in range(shape[-1])]
+    return x
+
+
+NTT_SHAPES = [(1, 3), (2, 1), (5, 4), (8, 2), (11, 3), (13, 2), (16, 3), (17, 1)]
+
+
+@pytest.mark.parametrize("log_n,batch,fill", fill_params(NTT_SHAPES, ("random",)) +
+                         fill_params([(1, 3), (5, 4), (11, 3), (16, 3)], ("max", "single_max", "pow2_32")))
+def test_ntt_matches_oracle(api, ctx, oracle, log_n, batch, fill):
     """FftNode forward / inverse evaluation (assumption A9: natural order, inverse scaled by 1/n)."""
     rng = np.random.default_rng(log_n)
-    x = rng.integers(0, GL_P, size=(batch, 1 << log_n), dtype=np.uint64)
+    x = ntt_fill(rng, fill, (batch, 1 << log_n), GL_P - 1, lambda sh: rng.integers(0, GL_P, size=sh, dtype=np.uint64)).astype(np.uint64)
     for inverse in (False, True):
         d = api.DeviceBuffer.from_numpy(ctx, x)
         api.ntt(ctx, d, log_n, inverse, batch)
@@ -470,8 +539,19 @@ def ctx_bn(api):
     c.close()
 
 
+def rand_fr_limbs(rng, shape):
+    """Canonical limbs of uniform-ish elements (a top limb below r's is enough), vectorised for large tables."""
+    t = rng.integers(0, 2**64, size=tuple(shape) + (4,), dtype=np.uint64)
+    t[..., 3] %= np.uint64(BN_R >> 192)
+    return t
+
+
+def rand_fr_int(rng, shape):
+    return np.array([int.from_bytes(rng.bytes(40), "little") % BN_R for _ in range(int(np.prod(shape)))], dtype=object).reshape(shape)
+
+
 def rand_fr(rng, shape):
-    vals = [int.from_bytes(rng.bytes(40), "little") % BN_R for _ in range(int(np.prod(shape)))]
+    vals = rand_fr_int(rng, shape).reshape(-1)
     return np.array([[(v >> (64 * j)) & 0xFFFFFFFFFFFFFFFF for j in range(4)] for v in vals], dtype=np.uint64).reshape(*shape, 4)
 
 
@@ -487,12 +567,15 @@ def test_bn254_device_field_arithmetic(api, ctx_bn, oracle):
         assert got == [f(x, y) for x, y in zip(ai, bi)], op
 
 
-@pytest.mark.parametrize("arity,nterms,nv", [(1, 3, 4), (2, 1, 1), (2, 4, 7), (2, 6, 3)])
+@pytest.mark.parametrize("arity,nterms,nv,fill", fill_params([(1, 3, 4), (2, 1, 1), (2, 4, 7), (2, 6, 3), (2, 1, 20)]))
 @pytest.mark.parametrize("mode", [0, 1])
-def test_bn254_sumcheck_matches_oracle(api, ctx_bn, oracle, arity, nterms, nv, mode):
+def test_bn254_sumcheck_matches_oracle(api, ctx_bn, oracle, arity, nterms, nv, fill, mode):
     rng = np.random.default_rng(nv * 10 + nterms)
-    tables = rand_fr(rng, (nterms * arity, 1 << nv))
+    tables = fill_tables(rng, fill, (nterms * arity, 1 << nv), _bn_limbs([0, BN_R - 2, BN_R - 1]),
+                         lambda sh: rand_fr(rng, sh) if np.prod(sh) <= 1 << 16 else rand_fr_limbs(rng, sh))
     coeffs, claim = rand_fr(rng, (nterms,)), rand_fr(rng, (1,))[0]
+    if fill == "max":
+        coeffs, claim = _bn_limbs([BN_R - 1] * nterms), _bn_limbs([BN_R - 1])[0]
     oproof, te, orr, ofe = oracle.sumcheck_prove(1, arity, coeffs, tables, nv, claim)
     d = api.DeviceBuffer.from_field(ctx_bn, tables)
     t = api.Keccak256Transcript(api.BN254)
@@ -589,14 +672,27 @@ def test_device_proofs_equal_committed_oracle_generated_golden_bytes(api, ctx, c
 
 def test_bn254_ntt_matches_oracle(api, ctx_bn, oracle):
     rng = np.random.default_rng(2)
-    for log_n in (3, 10, 13):
-        x = rand_fr(rng, (2, 1 << log_n))
+    cases = [(log_n, "random") for log_n in (3, 10, 13)] + [(log_n, f) for log_n in (3, 10) for f in ("max", "single_max", "pow2_32")]
+    for log_n, fill in cases:
+        x = _bn_limbs(ntt_fill(rng, fill, (2, 1 << log_n), BN_R - 1, lambda sh: rand_fr_int(rng, sh)).reshape(-1)).reshape(2, 1 << log_n, 4)
         for inverse in (False, True):
             d = api.DeviceBuffer.from_field(ctx_bn, x)
             api.ntt(ctx_bn, d, log_n, inverse, 2)
             got = d.to_field(2 << log_n).reshape(x.shape)
-            assert (got == oracle.ntt(1, x, log_n, inverse).reshape(x.shape)).all(), (log_n, inverse)
+            assert (got == oracle.ntt(1, x, log_n, inverse).reshape(x.shape)).all(), (log_n, fill, inverse)
             d.free()
+
+
+def test_bn254_mle_eval_batch_matches_oracle(api, ctx_bn, oracle):
+    rng = np.random.default_rng(19)
+    edge = lambda rng, nv: _bn_limbs(rng.choice(np.array([0, 1, BN_R - 1], dtype=object), size=nv))
+    top = lambda sh: np.broadcast_to(_bn_limbs([BN_R - 1])[0], sh + (4,)).copy()
+    for label, nv, nt, stride, tables, pt in _mle_cases(rng, lambda sh: rand_fr_limbs(rng, sh), top, lambda nv: rand_fr(rng, (nv,)), edge):
+        d = api.DeviceBuffer.from_field(ctx_bn, tables)
+        got = api.mle_eval_batch(ctx_bn, d, nt, nv, pt, stride=stride)
+        for i in range(nt):
+            assert (got[i] == oracle.mle_eval(1, tables[i, :1 << nv], nv, pt)).all(), (label, i)
+        d.free()
 
 
 # ------------------------------------------------------------------------------------------------ full-size byte parity
