@@ -19,6 +19,8 @@ MODE_PREFETCH, MODE_INTERACTIVE = 0, 1
 OPT_A3_WIRE, OPT_A3_H1, OPT_A5_ASCENDING = 3, 31, 5
 LIMBS = {GOLDILOCKS: 1, BN254: 4}
 DEGREE = {GOLDILOCKS: 2, BN254: 1}
+GL_P = 2**64 - 2**32 + 1                                                          # Goldilocks prime
+BN_R = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001  # BN254 scalar field order
 
 # every symbol include/hg_b200.h declares (tests check the library exports all of them)
 SYMBOLS = [
@@ -954,6 +956,31 @@ class Circuit:
         i = C.c_int(-1)
         _chk(lib().hg_circuit_insert_vanilla(self.h, arity, log2_sub, num_reps, ng, *[_p(x) for x in arrs], C.byref(i)))
         return i.value
+
+    def insert_vanilla(self, arity, log2_sub, gates, num_reps=1):
+        """VanillaNode::new(input_arity, log2_sub_input_size, gates, num_reps) from a list of VanillaGate. A coefficient or constant is
+        a Python int (reduced modulo the field's prime); a coefficient None is one, as Option<F> is in the reference."""
+        limbs = LIMBS[self.field]
+        p = GL_P if self.field == GOLDILOCKS else BN_R
+
+        def felts(vals):
+            out = np.zeros((len(vals), limbs), np.uint64)
+            for i, v in enumerate(vals):
+                v = (1 if v is None else int(v)) % p
+                for j in range(limbs):
+                    out[i, j] = (v >> (64 * j)) & 0xFFFFFFFFFFFFFFFF
+            return out
+        ng = len(gates)
+        add_ptr, mul_ptr = np.zeros(ng + 1, np.uint64), np.zeros(ng + 1, np.uint64)
+        adds = [a for g in gates for a in g.adds]
+        muls = [m for g in gates for m in g.muls]
+        add_ptr[1:] = np.cumsum([len(g.adds) for g in gates])
+        mul_ptr[1:] = np.cumsum([len(g.muls) for g in gates])
+        return self.insert_vanilla_arrays(
+            arity, log2_sub, num_reps, [g.const is not None for g in gates], felts([0 if g.const is None else g.const for g in gates]),
+            add_ptr, felts([c for c, _ in adds]), [w[0] for _, w in adds], [w[1] for _, w in adds],
+            mul_ptr, felts([c for c, _, _ in muls]), [a[0] for _, a, _ in muls], [a[1] for _, a, _ in muls],
+            [b[0] for _, _, b in muls], [b[1] for _, _, b in muls])
 
     def connect(self, frm, to):
         _chk(lib().hg_circuit_connect(self.h, frm, to))

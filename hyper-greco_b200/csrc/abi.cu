@@ -1101,13 +1101,8 @@ int hg_circuit_insert_vanilla(hg_circuit* c, size_t input_arity, size_t log2_sub
                               const uint64_t* add_wire, const uint64_t* mul_ptr, const uint64_t* mul_coef, const uint32_t* mul_in0, const uint64_t* mul_w0,
                               const uint32_t* mul_in1, const uint64_t* mul_w1, int* out_id) {
     HG_TRY({
-        if (c->ctx) circuit_use_device(c);
-        const size_t L = c->c->field_id == HG_FIELD_BN254 ? 4 : 1;  // limbs per coefficient
-        VanillaDesc d;
-        d.arity = input_arity; d.log2_sub = log2_sub_input_size; d.num_reps = num_reps; d.n_gates = n_gates;
-        d.has_const.assign(has_const, has_const + n_gates);
-        d.consts.assign(consts, consts + n_gates * L);
-        if (!has_const || !consts || !add_ptr || !mul_ptr || !out_id || n_gates < 1) throw std::runtime_error("hg_circuit_insert_vanilla: NULL argument or no gates");
+        // every argument is checked before anything is read through it
+        if (!c || !has_const || !consts || !add_ptr || !mul_ptr || !out_id || n_gates < 1) throw std::runtime_error("hg_circuit_insert_vanilla: NULL argument or no gates");
         // the edge arrays are sized by the CSR pointers: check those before anything is read through them
         if (add_ptr[0] != 0 || mul_ptr[0] != 0) throw std::runtime_error("hg_circuit_insert_vanilla: CSR pointers must start at 0");
         for (size_t g = 0; g < n_gates; g++)
@@ -1115,6 +1110,12 @@ int hg_circuit_insert_vanilla(hg_circuit* c, size_t input_arity, size_t log2_sub
         if (add_ptr[n_gates] > ((uint64_t)1 << 40) || mul_ptr[n_gates] > ((uint64_t)1 << 40)) throw std::runtime_error("hg_circuit_insert_vanilla: implausible edge count");
         if ((add_ptr[n_gates] && (!add_coef || !add_input || !add_wire)) || (mul_ptr[n_gates] && (!mul_coef || !mul_in0 || !mul_w0 || !mul_in1 || !mul_w1)))
             throw std::runtime_error("hg_circuit_insert_vanilla: NULL edge array");
+        if (c->ctx) circuit_use_device(c);
+        const size_t L = c->c->field_id == HG_FIELD_BN254 ? 4 : 1;  // limbs per coefficient
+        VanillaDesc d;
+        d.arity = input_arity; d.log2_sub = log2_sub_input_size; d.num_reps = num_reps; d.n_gates = n_gates;
+        d.has_const.assign(has_const, has_const + n_gates);
+        d.consts.assign(consts, consts + n_gates * L);
         d.add_ptr.assign(add_ptr, add_ptr + n_gates + 1);
         const size_t na = d.add_ptr[n_gates];
         d.add_coef.assign(add_coef, add_coef + na * L); d.add_in.assign(add_input, add_input + na); d.add_wire.assign(add_wire, add_wire + na);

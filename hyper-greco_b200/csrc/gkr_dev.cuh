@@ -2,9 +2,10 @@
 // (call sites /root/reference/bfv-gkr/src/sk_encryption_circuit.rs:102-290, :442, :455-457). The engine is the un-vendored `gkr`
 // crate (PARITY UNPINNED); the protocol restated here is specified in DESIGN.md section 3 (the parity tests check it against an independent CPU restatement):
 //     per node, in reverse topological order: [T > 1 claims: squeeze alpha] -> product sumcheck rounds -> write input evaluations
-// Node shapes: Input, Vanilla with linear gates (relay / scale / add-const / sum), the element-wise product layer, FFT
-// forward / inverse, Lasso. In PREFETCH mode every node's sumcheck is independent (claim POINTS are transcript challenges,
-// only claim VALUES flow between nodes, and those are needed on the host only), so round j of all nodes is one launch.
+// Node shapes: Input, Vanilla with linear gates (relay / scale / add-const / sum), the element-wise product layer, general
+// Vanilla layers (any other product terms: two sumchecks, DESIGN.md section 7b, A11), FFT forward / inverse, Lasso. In
+// PREFETCH mode every node's sumcheck is independent (claim POINTS are transcript challenges, only claim VALUES flow between
+// nodes, and those are needed on the host only), so round j of all nodes is one launch.
 #pragma once
 #include <algorithm>
 #include <map>
@@ -87,8 +88,8 @@ template <class FP> class GkrCircuitDev {
                 ok = !d.has_const[g] && d.mul_ptr[g] == g && d.mul_in0[g] == 0 && d.mul_in1[g] == 1 && d.mul_w0[g] == g && d.mul_w1[g] == g &&
                      FP::b_eq(FP::b_from_limbs(&d.mul_coef[g * FP::B_LIMBS]), FP::b_one());
             }
-            if (!ok) throw std::runtime_error("VanillaNode: only linear gates and the element-wise product layer are supported on the device");
-            n.is_elemmul = true;
+            n.is_elemmul = ok;
+            n.is_general = !ok;  // any other product term: the two-phase layer sumcheck (DESIGN.md section 3, A11)
         }
         auto up = [](auto& buf, const auto& v) { buf.alloc(std::max<size_t>(v.size(), 1)); if (!v.empty()) HG_CUDA(cudaMemcpy(buf.p, v.data(), v.size() * sizeof(v[0]), cudaMemcpyHostToDevice)); };
         std::vector<B> addc(n_add), mulc(n_mul), cg(ng);
@@ -125,7 +126,7 @@ template <class FP> class GkrCircuitDev {
             }
             if (!ok) n.fwd_runs.clear();
         }
-        if (n.is_linear) {
+        if (!n.is_elemmul) {
             // reverse wiring: for every element x of the concatenated inputs, the (output, coefficient) pairs that read it
             const size_t S = n.a_pad * n.n_in;
             std::vector<uint64_t> rp(S + 1, 0);
@@ -168,6 +169,32 @@ template <class FP> class GkrCircuitDev {
                 for (size_t r = 0; r < d.num_reps; r++) for (size_t g = 0; g < ng; g++) cf[r * ng + g] = cg[g];
                 up(n.consts_full, cf);
             }
+        }
+        if (n.is_general) {
+            // the product terms keyed by either side: row x of the x-keyed CSR = (y, output, coefficient) of every term that reads x as
+            // its first factor, row y of the y-keyed CSR = (x, output, coefficient); indices are positions in the concatenated inputs
+            const size_t S = n.a_pad * n.n_in;
+            if (S > ((size_t)1 << 32) || n.out_len > ((size_t)1 << 32) || n_mul * d.num_reps > ((size_t)1 << 32)) throw std::runtime_error("VanillaNode: general layer too large");
+            auto pos = [&](uint32_t in, size_t r, uint64_t w) { return (size_t)in * n.n_in + r * sub + w; };
+            std::vector<uint64_t> px(S + 1, 0), py(S + 1, 0);
+            for (size_t r = 0; r < d.num_reps; r++)
+                for (size_t e = 0; e < n_mul; e++) { px[pos(d.mul_in0[e], r, d.mul_w0[e]) + 1]++; py[pos(d.mul_in1[e], r, d.mul_w1[e]) + 1]++; }
+            for (size_t x = 0; x < S; x++) { px[x + 1] += px[x]; py[x + 1] += py[x]; }
+            const size_t ne = px[S];
+            std::vector<uint32_t> xo(ne), xout(ne), yo(ne), yout(ne);
+            std::vector<B> xc(ne), yc(ne);
+            std::vector<uint64_t> fx(px.begin(), px.end() - 1), fy(py.begin(), py.end() - 1);
+            for (size_t r = 0; r < d.num_reps; r++)
+                for (size_t g = 0; g < ng; g++)
+                    for (uint64_t e = d.mul_ptr[g]; e < d.mul_ptr[g + 1]; e++) {
+                        const size_t x = pos(d.mul_in0[e], r, d.mul_w0[e]), y = pos(d.mul_in1[e], r, d.mul_w1[e]);
+                        const uint32_t o = (uint32_t)(r * ng + g);
+                        xo[fx[x]] = (uint32_t)y; xout[fx[x]] = o; xc[fx[x]] = mulc[e]; fx[x]++;
+                        yo[fy[y]] = (uint32_t)x; yout[fy[y]] = o; yc[fy[y]] = mulc[e]; fy[y]++;
+                    }
+            up(n.gx_ptr, px); up(n.gx_other, xo); up(n.gx_out, xout); up(n.gx_coef, xc);
+            up(n.gy_ptr, py); up(n.gy_other, yo); up(n.gy_out, yout); up(n.gy_coef, yc);
+            n.n_terms = ne;
         }
         n.value.alloc(n.out_len);
         HG_CUDA(cudaDeviceSynchronize());  // blocking uploads from pageable memory vs non-blocking streams (see LassoNodeDev's constructor)
@@ -429,7 +456,7 @@ template <class FP> class GkrCircuitDev {
                 std::vector<std::shared_ptr<X>> vals;
                 for (auto& c : cl) vals.push_back(c.value);
                 const size_t aidx = job.alpha_idx, coff = job.const_off;
-                const bool has_c = n.kind == GKR_VANILLA && n.is_linear && n.has_consts;
+                const bool has_c = lin(n) && n.has_consts;
                 ch.emit([chp, st, vals, aidx, coff, has_c]() {
                     X a = aidx == (size_t)-1 ? FP::x_one() : chp->chal(aidx), p = FP::x_one(), comb = FP::x_zero();
                     for (auto& v : vals) { comb = FP::x_add(comb, FP::x_mul(p, *v)); p = FP::x_mul(p, a); }
@@ -437,35 +464,30 @@ template <class FP> class GkrCircuitDev {
                     st->claim = comb;
                 });
             }
-            const int n_ev = n.kind == GKR_FFT ? 1 : (n.is_elemmul ? 2 : n.arity);
-            if (mode == kModeInteractive) prepare_jobs(ch, {job}, wo);
-            for (int j = 0; j < job.nv; j++) {
-                size_t off = ch.alloc_msg(4);
-                if (j == 0) job.msg_off = off;
-                if (mode == kModeInteractive) launch_round(ch, {job}, j);
-                const size_t next_idx = ch.next_index();
-                if (job.nt == 1) emit_round_slots<FP, 2>(ch, st, off, wo, j == 0, next_idx);
-                else emit_round_slots<FP, 3>(ch, st, off, wo, j == 0, next_idx);
-                size_t idx = ch.squeeze(1);
-                if (j == 0) job.r0_idx = idx;
-            }
-            job.evals_off = ch.alloc_msg(n_ev);  // after the rounds: in interactive mode earlier slots have already been downloaded
-            if (mode == kModeInteractive) launch_finals(ch, {job});
-            // new claims on the predecessors: (point = the round challenges restricted to the input's variables, value = its evaluation)
-            const int in_vars = n.kind == GKR_VANILLA && n.is_linear ? log2sz(n.n_in) : job.nv;
-            std::vector<std::shared_ptr<X>> outv;
-            for (int k = 0; k < n_ev; k++) {
-                Claim c; c.by_index = true; c.idx = job.r0_idx; c.nvars = in_vars; c.value = std::make_shared<X>(FP::x_zero());
-                outv.push_back(c.value);
-                claims[n.preds.at(k)].push_back(c);
-            }
-            {
-                const size_t eo = job.evals_off;
-                ch.emit([chp, outv, eo]() {
-                    for (size_t k = 0; k < outv.size(); k++) { *outv[k] = chp->msg(eo + k); chp->transcript().write_felt_ext(*outv[k]); }
+            run_job(ch, mode, wo, job, st, jobs);
+            if (n.is_general) {
+                // phase 2 over y: sum_y (X(u) M(u, y)) X(y) = X(u) H(u), u = phase 1's challenges. The device samples the rounds with the
+                // unscaled M_u and reduces H(u) = sum_y M_u[y] X[y] into slot hu_off; X(u) = sum_k eq(u_hi, k) X_k(u_lo) comes from phase 1's
+                // input evaluations. The claim thus depends on message slots and challenges only, not on phase 1's host state.
+                const Job& p1 = jobs.back();
+                Job j2;
+                j2.node = id; j2.phase = 1; j2.nt = 1; j2.S = p1.S; j2.nv = p1.nv; j2.u_idx = p1.r0_idx;
+                j2.hu_off = ch.alloc_msg(1);
+                auto st2 = std::make_shared<ScHostState<FP>>();
+                const size_t eo = p1.evals_off, hu = j2.hu_off, u0 = p1.r0_idx;
+                const int m = log2sz(n.n_in), nvh = p1.nv - m, ar = n.arity;
+                ch.emit([chp, st2, eo, hu, u0, m, nvh, ar]() {
+                    X xu = FP::x_zero();
+                    for (int k = 0; k < ar; k++) {
+                        X e = FP::x_one();
+                        for (int i = 0; i < nvh; i++) { const X r = chp->chal(u0 + m + i); e = FP::x_mul(e, ((k >> i) & 1) ? r : FP::x_sub(FP::x_one(), r)); }
+                        xu = FP::x_add(xu, FP::x_mul(e, chp->msg(eo + k)));
+                    }
+                    st2->scaled = true; st2->scale = xu;
+                    st2->claim = FP::x_mul(xu, chp->msg(hu));
                 });
+                run_job(ch, mode, wo, j2, st2, jobs);
             }
-            jobs.push_back(job);
         }
         const double t3 = now();
         bool early = false;
@@ -480,7 +502,11 @@ template <class FP> class GkrCircuitDev {
                 }
             } swap(ctx_, fork);
             std::vector<Job> mine;  // the node sumchecks this device runs (all of them unless the proof is sharded)
-            for (size_t q = 0; q < jobs.size(); q++) if (!sharded || (int)(q % (size_t)world) == rank) mine.push_back(jobs[q]);
+            size_t q = 0;           // both phases of a general layer go to one device: phase 2 needs the weights and tables of phase 1
+            for (const Job& j : jobs) {
+                if (!sharded || (int)(q % (size_t)world) == rank) mine.push_back(j);
+                if (!(j.phase == 0 && nodes_[j.node]->is_general)) q++;
+            }
             prepare_jobs(ch, mine, wo);
             use_tail_ = true;
             struct TailOff { bool* f; ~TailOff() { *f = false; } } tail_off{&use_tail_};
@@ -498,10 +524,11 @@ template <class FP> class GkrCircuitDev {
         timing_[0] = t1 - t0; timing_[1] = t2 - t1; timing_[2] = t3 - t2; timing_[3] = t4 - t3;
     }
 
+    struct Work { DevBuf<X> wbuf0, wbuf1, tbuf0, tbuf1, capture, midpart; };
     struct Node {
         int kind = GKR_INPUT, log2_size = 0, num_reps = 1, arity = 0, log2_sub = 0;
-        bool fft_inverse = false, is_linear = false, is_elemmul = false, has_consts = false;
-        size_t ng = 0, out_len = 0, n_in = 0, a_pad = 1;
+        bool fft_inverse = false, is_linear = false, is_elemmul = false, is_general = false, has_consts = false;
+        size_t ng = 0, out_len = 0, n_in = 0, a_pad = 1, n_terms = 0;  // n_terms: product terms of a general layer, num_reps expanded
         std::vector<int> preds, succs;
         struct FwdRun { uint64_t g0, len; int ne; uint32_t in[HG_FWD_MAXE]; uint64_t w0[HG_FWD_MAXE]; B coef[HG_FWD_MAXE]; B cst; };
         std::vector<FwdRun> fwd_runs;    // non-empty: the gates come in runs (k_vanilla_runs evaluates the layer)
@@ -514,15 +541,57 @@ template <class FP> class GkrCircuitDev {
         PinnedBuf<const B*> h_in_ptrs;  // what in_ptrs holds (uploaded again only when an input pointer changes)
         const B* value_ptr = nullptr;
         LassoNodeDev<FP>* lasso = nullptr;
-        // per-node work buffers of the layer sumcheck
-        DevBuf<X> W, A, wbuf0, wbuf1, tbuf0, tbuf1, capture, midpart;
+        // general layers: the product terms as two reverse CSRs over the concatenated inputs, num_reps expanded. Row x of the
+        // x-keyed one lists (y, output, coefficient) of every term that reads x on its first side; the y-keyed one (x, output, coefficient).
+        DevBuf<u64> gx_ptr, gy_ptr;
+        DevBuf<u32> gx_other, gx_out, gy_other, gy_out;
+        DevBuf<B> gx_coef, gy_coef;
+        // per-node work buffers of the layer sumcheck (wk[1]: phase 2 of a general layer, which runs next to phase 1)
+        DevBuf<X> W, A, Mu;
+        Work wk[2];
         DevBuf<B> Xcat;
     };
+    // phase: 0 = the node's (first) sumcheck, 1 = phase 2 of a general layer (weights M_u, claim X(u) H(u), u = phase 1's challenges)
     struct Job {
-        int node = 0, nt = 1, nv = 0;
-        size_t S = 0, alpha_idx = (size_t)-1, const_off = 0, msg_off = 0, r0_idx = 0, evals_off = 0;
+        int node = 0, nt = 1, nv = 0, phase = 0;
+        size_t S = 0, alpha_idx = (size_t)-1, const_off = 0, msg_off = 0, r0_idx = 0, evals_off = 0, u_idx = 0, hu_off = 0;
         std::vector<const X*> points;
     };
+    // the rounds of one node sumcheck (launched here in interactive mode, batched by the caller in prefetch mode), its input
+    // evaluations and the claims they put on the node's predecessors; appends the job to `jobs`
+    void run_job(Channel<FP>& ch, ProveMode mode, const WireOptions& wo, Job& job, std::shared_ptr<ScHostState<FP>> st, std::vector<Job>& jobs) {
+        Node& n = *nodes_[job.node];
+        Channel<FP>* chp = &ch;
+        const int n_ev = n.kind == GKR_FFT ? 1 : (n.is_elemmul ? 2 : n.arity);
+        if (mode == kModeInteractive) prepare_jobs(ch, {job}, wo);
+        for (int j = 0; j < job.nv; j++) {
+            size_t off = ch.alloc_msg(4);
+            if (j == 0) job.msg_off = off;
+            if (mode == kModeInteractive) launch_round(ch, {job}, j);
+            const size_t next_idx = ch.next_index();
+            if (job.nt == 1) emit_round_slots<FP, 2>(ch, st, off, wo, j == 0, next_idx);
+            else emit_round_slots<FP, 3>(ch, st, off, wo, j == 0, next_idx);
+            size_t idx = ch.squeeze(1);
+            if (j == 0) job.r0_idx = idx;
+        }
+        job.evals_off = ch.alloc_msg(n_ev);  // after the rounds: in interactive mode earlier slots have already been downloaded
+        if (mode == kModeInteractive) launch_finals(ch, {job});
+        // new claims on the predecessors: (point = the round challenges restricted to the input's variables, value = its evaluation)
+        const int in_vars = lin(n) ? log2sz(n.n_in) : job.nv;
+        std::vector<std::shared_ptr<X>> outv;
+        for (int k = 0; k < n_ev; k++) {
+            Claim c; c.by_index = true; c.idx = job.r0_idx; c.nvars = in_vars; c.value = std::make_shared<X>(FP::x_zero());
+            outv.push_back(c.value);
+            pending_claims_[n.preds.at(k)].push_back(c);
+        }
+        {
+            const size_t eo = job.evals_off;
+            ch.emit([chp, outv, eo]() {
+                for (size_t k = 0; k < outv.size(); k++) { *outv[k] = chp->msg(eo + k); chp->transcript().write_felt_ext(*outv[k]); }
+            });
+        }
+        jobs.push_back(job);
+    }
 
     struct FftGroup { std::vector<int> nodes; std::unique_ptr<DevBuf<B>> arena; };
     struct EvalLevel {
@@ -608,16 +677,22 @@ template <class FP> class GkrCircuitDev {
             size_t edges = 0;
             for (int sx : n.succs) for (int p : nodes_[sx]->preds) if (p == id) edges++;
             n_claims = std::max<size_t>(1, edges);
-            chal += (n_claims > 1 ? 1 : 0) + nv;
-            msg += 1 + 4 * (size_t)nv + 8 + n.a_pad;
+            const int phases = n.is_general ? 2 : 1;
+            chal += (n_claims > 1 ? 1 : 0) + phases * nv;
+            msg += phases * (1 + 4 * (size_t)nv + 8 + n.a_pad);
             eq_elems += n_claims * (((size_t)1 << eq_lo_bits(log2sz(n.out_len))) + (n.out_len >> eq_lo_bits(log2sz(n.out_len))) + 2);
-            items += n_claims + 4;
+            if (n.is_general) eq_elems += ((size_t)1 << eq_lo_bits(nv)) + (S >> eq_lo_bits(nv)) + 2;  // eq(u, .) of phase 2
+            items += n_claims + 4 * phases;
             n.W.alloc(n.out_len);
             if (!(n.kind == GKR_VANILLA && n.is_elemmul)) n.A.alloc(S);
-            n.wbuf0.alloc(std::max<size_t>(S / 2, 1)); n.wbuf1.alloc(std::max<size_t>(S / 4, 1));
-            n.tbuf0.alloc(std::max<size_t>(nt * (S / 2), 1)); n.tbuf1.alloc(std::max<size_t>(nt * (S / 4), 1));
+            for (int ph = 0; ph < phases; ph++) {
+                Work& w = n.wk[ph];
+                w.wbuf0.alloc(std::max<size_t>(S / 2, 1)); w.wbuf1.alloc(std::max<size_t>(S / 4, 1));
+                w.tbuf0.alloc(std::max<size_t>(nt * (S / 2), 1)); w.tbuf1.alloc(std::max<size_t>(nt * (S / 4), 1));
+                w.capture.alloc(n.a_pad + 2);
+            }
+            if (n.is_general) n.Mu.alloc(S);
             if (n.kind == GKR_VANILLA) n.Xcat.alloc(n.is_elemmul ? 2 * S : S);
-            n.capture.alloc(n.a_pad + 2);
         }
         total_chal_ = chal;
         msg_budget_ = msg + 64;
@@ -657,6 +732,20 @@ template <class FP> class GkrCircuitDev {
         for (size_t q = 0; q < jobs.size(); q++) {
             const Job& j = jobs[q];
             Node& n = *nodes_[j.node];
+            if (j.phase == 1) {  // eq(u, .) over the S entries of the concatenated inputs, in two factors
+                const int lo = eq_lo_bits(j.nv);
+                const size_t need = ((size_t)1 << lo) + ((size_t)1 << (j.nv - lo));
+                if (eq_off_ + need > d_eq_.n) throw std::runtime_error("gkr: eq table pool too small");
+                X* elo = d_eq_.p + eq_off_;
+                eq_off_ += need;
+                EqSplitItem<FP> si; si.point = ch.d_chal(j.u_idx); si.eq_lo = elo; si.eq_hi = elo + ((size_t)1 << lo); si.nv = j.nv; si.lo_bits = lo;
+                si.blk_start = split_blk; si.alpha = nullptr; si.t = 0;
+                split_blk += (int)((need + HG_BLOCK - 1) / HG_BLOCK);
+                split_bytes += need * sizeof(X);
+                splits.push_back(si);
+                eqs[q].push_back({elo, si.eq_hi, lo});
+                continue;
+            }
             const int nvw = log2sz(n.out_len), lo = eq_lo_bits(nvw);
             max_claims = std::max(max_claims, j.points.size());
             for (size_t t = 0; t < j.points.size(); t++) {
@@ -710,8 +799,34 @@ template <class FP> class GkrCircuitDev {
             cat_bytes += cnt * sizeof(B) * 2;
             cats.push_back(c);
         };
-        for (const Job& j : jobs) {
+        std::vector<GeneralItem<FP>> gitems, mitems;  // general layers: phase 1's G gather, phase 2's M_u gather
+        int g_blk = 0, m_blk = 0;
+        size_t g_bytes = 0, m_bytes = 0;
+        std::vector<const Job*> hu_jobs;
+        auto general_item = [&](const Node& n, bool phase2, int& blk, size_t& bytes) {
+            GeneralItem<FP> gi;
+            const size_t S = n.a_pad * n.n_in;
+            gi.ptr = phase2 ? n.gy_ptr.p : n.gx_ptr.p; gi.other = phase2 ? n.gy_other.p : n.gx_other.p; gi.out = phase2 ? n.gy_out.p : n.gx_out.p;
+            gi.coef = phase2 ? n.gy_coef.p : n.gx_coef.p; gi.w = n.W.p; gi.tab = tables(n); gi.dst = phase2 ? n.Mu.p : n.A.p;
+            gi.eq_lo = gi.eq_hi = nullptr; gi.lo_bits = 0; gi.n = S; gi.blk_start = blk;
+            blk += (int)((S + HG_BLOCK * HG_GENERAL_PER_THREAD - 1) / (HG_BLOCK * HG_GENERAL_PER_THREAD));
+            // algorithmic bytes: the row pointers, every term (index, output, coefficient, W[output], X[y] or two eq factors), A read and G
+            // written (phase 1) or M_u written (phase 2)
+            bytes += (S + 1) * sizeof(u64) + n.n_terms * (2 * sizeof(u32) + sizeof(B) + sizeof(X) + (phase2 ? 2 * sizeof(X) : sizeof(B))) +
+                     S * sizeof(X) * (phase2 ? 1 : 2);
+            return gi;
+        };
+        for (size_t q = 0; q < jobs.size(); q++) {
+            const Job& j = jobs[q];
             Node& n = *nodes_[j.node];
+            if (j.phase == 1) {
+                GeneralItem<FP> gi = general_item(n, true, m_blk, m_bytes);
+                gi.eq_lo = eqs[q][0].lo; gi.eq_hi = eqs[q][0].hi; gi.lo_bits = eqs[q][0].lo_bits;
+                mitems.push_back(gi);
+                hu_jobs.push_back(&j);
+                continue;
+            }
+            if (n.is_general) gitems.push_back(general_item(n, false, g_blk, g_bytes));
             if (n.kind == GKR_FFT) { fft_groups[{n.log2_size, n.fft_inverse ? 1 : 0}].push_back(j.node); continue; }
             if (n.is_elemmul) {
                 // tables = [in0 | in1]
@@ -745,6 +860,16 @@ template <class FP> class GkrCircuitDev {
         if (!runs.empty()) HG_K(ctx_, KC_GKR_PREP, run_bytes, k_wiring_runs<FP><<<run_blk, HG_BLOCK, 0, s>>>(stage(runs), (int)runs.size()));
         if (!wires.empty()) HG_K(ctx_, KC_GKR_PREP, wire_bytes, k_wiring_gather<FP><<<wire_blk, HG_BLOCK, 0, s>>>(stage(wires), (int)wires.size()));
         if (!cats.empty()) HG_K(ctx_, KC_GKR_PREP, cat_bytes, k_concat_items<FP><<<cat_blk, HG_BLOCK, 0, s>>>(stage(cats), (int)cats.size()));
+        // general layers, after W, A and the concatenated inputs: G = A + H in place of A (phase 1), M_u and H(u) (phase 2)
+        if (!gitems.empty()) HG_K(ctx_, KC_GKR_PREP, g_bytes, k_general_g<FP><<<g_blk, HG_BLOCK, 0, s>>>(stage(gitems), (int)gitems.size()));
+        if (!mitems.empty()) HG_K(ctx_, KC_GKR_PREP, m_bytes, k_general_mu<FP><<<m_blk, HG_BLOCK, 0, s>>>(stage(mitems), (int)mitems.size()));
+        for (const Job* j : hu_jobs) {
+            const Node& n = *nodes_[j->node];
+            const size_t S = n.a_pad * n.n_in;
+            int blocks = (int)std::min<size_t>((S + HG_BLOCK - 1) / HG_BLOCK, (size_t)ctx_->sm_count * 2);
+            HG_K(ctx_, KC_GKR_PREP, S * (sizeof(X) + sizeof(B)),
+                 k_dot_wconst<FP><<<blocks, HG_BLOCK, 0, s>>>(n.Mu.p, tables(n), S, d_partials_.p, d_counters_.p, ch.d_msg(j->hu_off)));
+        }
         // FFT-matrix weights: A = transform(W) plane by plane, batched over all FFT nodes of the same size and direction
         for (auto& kv : fft_groups) {
             const int lg = kv.first.first;
@@ -762,11 +887,19 @@ template <class FP> class GkrCircuitDev {
         (void)wo;
     }
 
-    const X* weights(const Node& n) const { return n.kind == GKR_VANILLA && n.is_elemmul ? n.W.p : n.A.p; }
+    const X* weights(const Job& j) const {
+        const Node& n = *nodes_[j.node];
+        if (j.phase == 1) return n.Mu.p;
+        return n.kind == GKR_VANILLA && n.is_elemmul ? n.W.p : n.A.p;
+    }
     const B* tables(const Node& n) const {
-        if (n.kind == GKR_FFT || (n.kind == GKR_VANILLA && n.is_linear && n.arity == 1)) return nodes_[n.preds.at(0)]->value_ptr;
+        if (n.kind == GKR_FFT || (lin(n) && n.arity == 1)) return nodes_[n.preds.at(0)]->value_ptr;
         return n.Xcat.p;
     }
+    // sumchecks over the concatenated inputs (linear and general layers): the input evaluations are read off the table folded
+    // over the low log2(n_in) variables
+    static bool lin(const Node& n) { return n.kind == GKR_VANILLA && !n.is_elemmul; }
+    Work& wk(const Job& j) { return nodes_[j.node]->wk[j.phase]; }
 
     // round r of every job that still has one
     void launch_round(Channel<FP>& ch, const std::vector<Job>& jobs, int r) {
@@ -786,16 +919,17 @@ template <class FP> class GkrCircuitDev {
             const bool fuse = r == 1 && fused0(j);
             any_fused = any_fused || fuse;
             Node& n = *nodes_[j.node];
+            Work& wb = wk(j);
             ProdItem<FP> it;
             it.nt = j.nt;
             if (r == 0) {
-                it.w_in = weights(n); it.w_out = nullptr; it.tab_in = tables(n); it.tab_out = nullptr; it.n_in = j.S; it.r_prev = nullptr;
+                it.w_in = weights(j); it.w_out = nullptr; it.tab_in = tables(n); it.tab_out = nullptr; it.n_in = j.S; it.r_prev = nullptr;
             } else {
                 it.n_in = j.S >> (r - 1);
-                it.w_in = r == 1 ? weights(n) : ((r - 1) & 1 ? n.wbuf0.p : n.wbuf1.p);
-                it.w_out = (r & 1) ? n.wbuf0.p : n.wbuf1.p;
-                it.tab_in = r == 1 ? (const void*)tables(n) : (const void*)((r - 1) & 1 ? n.tbuf0.p : n.tbuf1.p);
-                it.tab_out = (r & 1) ? n.tbuf0.p : n.tbuf1.p;
+                it.w_in = r == 1 ? weights(j) : ((r - 1) & 1 ? wb.wbuf0.p : wb.wbuf1.p);
+                it.w_out = (r & 1) ? wb.wbuf0.p : wb.wbuf1.p;
+                it.tab_in = r == 1 ? (const void*)tables(n) : (const void*)((r - 1) & 1 ? wb.tbuf0.p : wb.tbuf1.p);
+                it.tab_out = (r & 1) ? wb.tbuf0.p : wb.tbuf1.p;
                 it.r_prev = ch.d_chal(j.r0_idx + r - 1);
             }
             it.msg = ch.d_msg(j.msg_off + 4 * (size_t)(fuse ? 0 : r));
@@ -827,10 +961,11 @@ template <class FP> class GkrCircuitDev {
         std::vector<CopyItem<FP>> copies;
         for (const Job& j : jobs) {
             Node& n = *nodes_[j.node];
-            if (!(n.kind == GKR_VANILLA && n.is_linear)) continue;
+            Work& wb = wk(j);
+            if (!lin(n)) continue;
             const int m = log2sz(n.n_in);
             if (m != r || m >= j.nv || r == 0 || m >= stream_end(j)) continue;
-            CopyItem<FP> c; c.src = (m & 1) ? n.tbuf0.p : n.tbuf1.p; c.dst = n.capture.p; c.n = n.arity;
+            CopyItem<FP> c; c.src = (m & 1) ? wb.tbuf0.p : wb.tbuf1.p; c.dst = wb.capture.p; c.n = n.arity;
             copies.push_back(c);
         }
         if (!copies.empty()) HG_K(ctx_, KC_GKR_SC, copies.size() * 64, k_copy_items<FP><<<(unsigned)copies.size(), 32, 0, s>>>(stage(copies)));
@@ -856,20 +991,21 @@ template <class FP> class GkrCircuitDev {
         for (const Job& j : jobs) {
             if (!has_mid(j)) continue;
             Node& n = *nodes_[j.node];
+            Work& wb = wk(j);
             const int se = stream_end(j);
             ProdMidItem<FP> it;
             it.n_in = j.S >> (se - 1);
             if (it.n_in < 2 * (size_t)HG_PROD_MID_SEG || (it.n_in % HG_PROD_MID_SEG)) throw std::runtime_error("gkr: mid stage on a table that is too small");
             it.nt = j.nt; it.nseg = (int)(it.n_in / HG_PROD_MID_SEG); it.blk_start = blk;
-            it.w_in = ((se - 1) & 1) ? n.wbuf0.p : n.wbuf1.p;  it.tab_in = ((se - 1) & 1) ? n.tbuf0.p : n.tbuf1.p;
-            it.w_out = (se & 1) ? n.wbuf0.p : n.wbuf1.p;       it.tab_out = (se & 1) ? n.tbuf0.p : n.tbuf1.p;
+            it.w_in = ((se - 1) & 1) ? wb.wbuf0.p : wb.wbuf1.p;  it.tab_in = ((se - 1) & 1) ? wb.tbuf0.p : wb.tbuf1.p;
+            it.w_out = (se & 1) ? wb.wbuf0.p : wb.wbuf1.p;       it.tab_out = (se & 1) ? wb.tbuf0.p : wb.tbuf1.p;
             it.chal = ch.d_chal(j.r0_idx + se - 1);
-            if (n.midpart.n < (size_t)HG_PROD_MID_K * it.nseg * 4) { HG_CUDA(cudaStreamSynchronize(s)); n.midpart.alloc((size_t)HG_PROD_MID_K * it.nseg * 4); }
-            it.part = n.midpart.p;
+            if (wb.midpart.n < (size_t)HG_PROD_MID_K * it.nseg * 4) { HG_CUDA(cudaStreamSynchronize(s)); wb.midpart.alloc((size_t)HG_PROD_MID_K * it.nseg * 4); }
+            it.part = wb.midpart.p;
             it.capture = nullptr; it.cap_round = -1; it.arity = n.arity;
-            if (n.kind == GKR_VANILLA && n.is_linear) {
+            if (lin(n)) {
                 const int m = log2sz(n.n_in);
-                if (m >= se && m < se + HG_PROD_MID_K) { it.capture = n.capture.p; it.cap_round = m - se; }
+                if (m >= se && m < se + HG_PROD_MID_K) { it.capture = wb.capture.p; it.cap_round = m - se; }
             }
             blk += it.nseg;
             nt_max = std::max(nt_max, j.nt);
@@ -889,27 +1025,28 @@ template <class FP> class GkrCircuitDev {
             const int rt = tail_start(j);
             if (rt >= j.nv) continue;
             Node& n = *nodes_[j.node];
+            Work& wb = wk(j);
             ProdTailItem<FP> t;
             t.n_in = (int)(j.S >> (rt - 1)); t.nt = j.nt; t.rounds = j.nv - rt;
-            t.w_in = ((rt - 1) & 1) ? n.wbuf0.p : n.wbuf1.p;
-            t.tab_in = ((rt - 1) & 1) ? n.tbuf0.p : n.tbuf1.p;
+            t.w_in = ((rt - 1) & 1) ? wb.wbuf0.p : wb.wbuf1.p;
+            t.tab_in = ((rt - 1) & 1) ? wb.tbuf0.p : wb.tbuf1.p;
             t.mid_part = nullptr; t.mid_msg = nullptr; t.mid_nseg = 0; t.mid_rounds = 0;
             if (has_mid(j)) {  // the mid stage wrote its pairs where streaming round stream_end would have written
                 const int se = stream_end(j);
-                t.w_in = (se & 1) ? n.wbuf0.p : n.wbuf1.p;
-                t.tab_in = (se & 1) ? n.tbuf0.p : n.tbuf1.p;
-                t.mid_part = n.midpart.p; t.mid_nseg = (int)((j.S >> (se - 1)) / HG_PROD_MID_SEG); t.mid_rounds = HG_PROD_MID_K;
+                t.w_in = (se & 1) ? wb.wbuf0.p : wb.wbuf1.p;
+                t.tab_in = (se & 1) ? wb.tbuf0.p : wb.tbuf1.p;
+                t.mid_part = wb.midpart.p; t.mid_nseg = (int)((j.S >> (se - 1)) / HG_PROD_MID_SEG); t.mid_rounds = HG_PROD_MID_K;
                 t.mid_msg = ch.d_msg(j.msg_off + 4 * (size_t)se);
             }
             t.chal = ch.d_chal(j.r0_idx + rt - 1);
             t.msg = ch.d_msg(j.msg_off + 4 * (size_t)rt);
             t.evals = ch.d_msg(j.evals_off);
-            t.linear = n.kind == GKR_VANILLA && n.is_linear;
+            t.linear = lin(n);
             t.arity = n.arity; t.capture = nullptr; t.cap_round = -1;
             if (t.linear) {
                 const int m = log2sz(n.n_in);
                 if (m == 0) throw std::runtime_error("gkr: empty input tables");
-                if (m < rt) t.capture = n.capture.p;
+                if (m < rt) t.capture = wb.capture.p;
                 else if (m < j.nv) t.cap_round = m - rt;
             }
             smem = std::max(smem, ((size_t)(j.nt + 1) * (t.n_in + t.n_in / 2) + 96) * sizeof(X));
@@ -929,11 +1066,12 @@ template <class FP> class GkrCircuitDev {
         for (const Job& j : jobs) {
             if (tail_start(j) < j.nv) continue;  // done by launch_tail
             Node& n = *nodes_[j.node];
+            Work& wb = wk(j);
             // state after the last round launch (round nv-1): tables folded by r_0..r_{nv-2}, length 2
             const int last = j.nv - 1;
-            const void* tab_last = last == 0 ? (const void*)tables(n) : (const void*)((last & 1) ? n.tbuf0.p : n.tbuf1.p);
+            const void* tab_last = last == 0 ? (const void*)tables(n) : (const void*)((last & 1) ? wb.tbuf0.p : wb.tbuf1.p);
             const bool base_last = last == 0;
-            if (n.kind == GKR_VANILLA && n.is_linear) {
+            if (lin(n)) {
                 const int m = log2sz(n.n_in);  // the table folded by r_0..r_{m-1} has a_pad entries: the evaluations of the inputs
                 if (m == j.nv) {
                     FoldItem<FP> f; f.in = tab_last; f.out = ch.d_msg(j.evals_off); f.r = ch.d_chal(j.r0_idx + j.nv - 1); f.n_out = 1; f.in_base = base_last;
@@ -941,7 +1079,7 @@ template <class FP> class GkrCircuitDev {
                 } else if (m == 0) {
                     throw std::runtime_error("gkr: empty input tables");
                 } else {  // captured by launch_round(m) into the node's staging buffer
-                    CopyItem<FP> c; c.src = n.capture.p; c.dst = ch.d_msg(j.evals_off); c.n = n.arity;
+                    CopyItem<FP> c; c.src = wb.capture.p; c.dst = ch.d_msg(j.evals_off); c.n = n.arity;
                     copies.push_back(c);
                 }
             } else {

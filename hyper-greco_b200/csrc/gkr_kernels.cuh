@@ -193,6 +193,64 @@ template <class FP> __global__ void k_wiring_runs(const WireRunItem<FP>* __restr
         it.A[i] = v[k];
     }
 }
+// ---- general layers (the two-phase layer sumcheck, DESIGN.md section 3, A11). The product terms are two reverse CSRs over the
+// S entries of the concatenated inputs X (num_reps expanded): row x of the x-keyed CSR holds (y, output, coefficient) of every term
+// W-weighted as W[output] coef X[x] X[y], row y of the y-keyed CSR the same terms with their x. Gathers: no atomics.
+template <class FP> struct GeneralItem {
+    const u64* ptr; const u32* other; const u32* out; const typename FP::B* coef;
+    const typename FP::X* w;                                       // W: weights of the outputs
+    const typename FP::B* tab;                                     // X (phase 1)
+    const typename FP::X* eq_lo; const typename FP::X* eq_hi;      // eq(u, .) = eq_lo[x mod 2^lo_bits] eq_hi[x >> lo_bits] (phase 2)
+    typename FP::X* dst;                                           // phase 1: A, turned into G = A + H in place; phase 2: M_u
+    u64 n; int lo_bits, blk_start;
+};
+constexpr int HG_GENERAL_PER_THREAD = 4;  // independent row chains per thread (ptr -> term -> W): memory-level parallelism
+// phase 1: G[x] = A[x] + H[x],  H[x] = sum_{(y, o, c) in row x} W[o] c X[y]
+template <class FP> __global__ void k_general_g(const GeneralItem<FP>* __restrict__ items, int nitems) {
+    const GeneralItem<FP> it = items[find_item(items, nitems)];
+    const size_t base = (size_t)(blockIdx.x - it.blk_start) * blockDim.x * HG_GENERAL_PER_THREAD + threadIdx.x;
+    u64 e0[HG_GENERAL_PER_THREAD], e1[HG_GENERAL_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < HG_GENERAL_PER_THREAD; k++) {
+        const size_t x = base + (size_t)k * blockDim.x;
+        e0[k] = e1[k] = 0;
+        if (x < it.n) { e0[k] = it.ptr[x]; e1[k] = it.ptr[x + 1]; }
+    }
+#pragma unroll
+    for (int k = 0; k < HG_GENERAL_PER_THREAD; k++) {
+        const size_t x = base + (size_t)k * blockDim.x;
+        if (x >= it.n || e0[k] == e1[k]) continue;
+        typename FP::XAcc acc = FP::xacc_zero_();
+        for (u64 e = e0[k]; e < e1[k]; e++) FP::xacc_mad_b(acc, it.w[it.out[e]], FP::fmul(it.coef[e], it.tab[it.other[e]]));
+        it.dst[x] = FP::x_add(it.dst[x], FP::xacc_reduce_(acc));
+    }
+}
+// phase 2: M_u[y] = sum_{(x, o, c) in row y} eq(u, x) W[o] c
+template <class FP> __global__ void k_general_mu(const GeneralItem<FP>* __restrict__ items, int nitems) {
+    typedef typename FP::X X;
+    const GeneralItem<FP> it = items[find_item(items, nitems)];
+    const size_t base = (size_t)(blockIdx.x - it.blk_start) * blockDim.x * HG_GENERAL_PER_THREAD + threadIdx.x;
+    const size_t mask = ((size_t)1 << it.lo_bits) - 1;
+    u64 e0[HG_GENERAL_PER_THREAD], e1[HG_GENERAL_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < HG_GENERAL_PER_THREAD; k++) {
+        const size_t y = base + (size_t)k * blockDim.x;
+        e0[k] = e1[k] = 0;
+        if (y < it.n) { e0[k] = it.ptr[y]; e1[k] = it.ptr[y + 1]; }
+    }
+#pragma unroll
+    for (int k = 0; k < HG_GENERAL_PER_THREAD; k++) {
+        const size_t y = base + (size_t)k * blockDim.x;
+        if (y >= it.n) continue;
+        typename FP::XAcc acc = FP::xacc_zero_();
+        for (u64 e = e0[k]; e < e1[k]; e++) {
+            const size_t x = it.other[e];
+            const X eqx = FP::fmul(it.eq_lo[x & mask], it.eq_hi[x >> it.lo_bits]);
+            FP::xacc_mad_b(acc, FP::fmul(eqx, it.w[it.out[e]]), it.coef[e]);
+        }
+        it.dst[y] = FP::xacc_reduce_(acc);
+    }
+}
 // concatenated input tables of the layer sumchecks: dst[0..n) = src[0..n) (src = nullptr: zeros), every node's pieces in one launch
 template <class FP> struct ConcatItem { const typename FP::B* src; typename FP::B* dst; u64 n; int blk_start; };
 constexpr int HG_CONCAT_PER_THREAD = 8;

@@ -8,6 +8,7 @@
 //     final check   W(r) * prod_k in_k(r) == last sumcheck claim,   W = the weights the claims induce on the node's inputs
 //       Vanilla, additive gates   W = sum_t alpha^t eq(z_t, .) pushed through the wiring (plus the constant part of the gates)
 //       element-wise product      W = sum_t alpha^t eq(z_t, .)
+//       Vanilla, general gates    two product sumchecks (x, then y), final check X(u) M(u, v) X(v) == last claim (DESIGN.md section 3, A11)
 //       FFT forward / inverse     W = transform of sum_t alpha^t eq(z_t, .)   (the DFT matrix is symmetric)
 //       Lasso                     LassoVerifier (lasso_verify.hpp)
 // It returns the claims that reach the input nodes; the caller compares them with the MLEs of the inputs (hg_mle_eval_host).
@@ -82,6 +83,8 @@ template <class FP> class GkrVerifierHost {
         const size_t n_add = d.add_ptr[ng], n_mul = d.mul_ptr[ng];
         for (size_t g = 0; g < ng; g++) if (d.add_ptr[g + 1] < d.add_ptr[g] || d.mul_ptr[g + 1] < d.mul_ptr[g]) throw VerifyError("VanillaNode: CSR pointers must be non-decreasing");
         for (size_t e = 0; e < n_add; e++) if (d.add_in[e] >= d.arity || d.add_wire[e] >= sub) throw VerifyError("VanillaNode: edge outside the inputs");
+        for (size_t e = 0; e < n_mul; e++)
+            if (d.mul_in0[e] >= d.arity || d.mul_in1[e] >= d.arity || d.mul_w0[e] >= sub || d.mul_w1[e] >= sub) throw VerifyError("VanillaNode: edge outside the inputs");
         Node n;
         n.kind = GKR_VANILLA; n.arity = (int)d.arity; n.log2_sub = (int)d.log2_sub; n.num_reps = (int)d.num_reps; n.ng = ng;
         n.out_len = pad2(ng * d.num_reps);
@@ -93,11 +96,9 @@ template <class FP> class GkrVerifierHost {
             for (size_t g = 0; ok && g < ng; g++)
                 ok = !d.has_const[g] && d.mul_ptr[g] == g && d.mul_in0[g] == 0 && d.mul_in1[g] == 1 && d.mul_w0[g] == g && d.mul_w1[g] == g &&
                      FP::b_eq(FP::b_from_limbs(&d.mul_coef[g * FP::B_LIMBS]), FP::b_one());
-            if (!ok) throw VerifyError("VanillaNode: only linear gates and the element-wise product layer are supported");
-            n.is_elemmul = true;
-        } else {
-            n.desc.reset(new VanillaDesc(d));
+            n.is_elemmul = ok;  // otherwise a general layer (two-phase layer sumcheck)
         }
+        if (!n.is_elemmul) n.desc.reset(new VanillaDesc(d));
         nodes_.push_back(std::move(n));
         return (int)nodes_.size() - 1;
     }
@@ -197,7 +198,7 @@ template <class FP> class GkrVerifierHost {
         bool fft_inverse = false, is_linear = false, is_elemmul = false;
         size_t ng = 0, out_len = 0, n_in = 0, a_pad = 1;
         std::vector<int> preds, succs;
-        std::shared_ptr<VanillaDesc> desc;            // linear layers: the gates (CSR)
+        std::shared_ptr<VanillaDesc> desc;            // linear and general layers: the gates (CSR)
         std::shared_ptr<LassoPreprocessing> pp;
     };
     static size_t pad2(size_t n) { size_t p = 1; while (p < n) p <<= 1; return p; }
@@ -296,8 +297,50 @@ template <class FP> class GkrVerifierHost {
                 out[k].push_back({lo, e});
             }
             if (!FP::x_eq(FP::x_mul(mle_eval_ext(std::move(A), pt), x), fc)) throw VerifyError("InvalidSumCheck: linear layer final evaluation mismatch");
-        } else {
-            throw VerifyError("verify_gkr: unsupported gate shape");
+        } else {  // general layer: phase 1 over x (claim c - const), phase 2 over y (claim fc1 - A(u) X(u)), DESIGN.md section 3 (A11)
+            if ((int)n.preds.size() != n.arity) throw VerifyError("Vanilla node arity does not match its connections");
+            const VanillaDesc& d = *n.desc;
+            const size_t S = n.a_pad * n.n_in, sub = (size_t)1 << n.log2_sub;
+            const int nv = log2sz(S), lo_vars = log2sz(n.n_in);
+            X constant = FP::x_zero();
+            for (size_t r = 0; r < (size_t)n.num_reps; r++)
+                for (size_t g = 0; g < n.ng; g++)
+                    if (d.has_const[g]) constant = FP::x_add(constant, FP::x_mul_b(w[r * n.ng + g], FP::b_from_limbs(&d.consts[g * FP::B_LIMBS])));
+            auto read_evals = [&](const std::vector<X>& p) {  // X(p) = sum_k eq(p_hi, k) X_k(p_lo) from the written X_k(p_lo)
+                const std::vector<X> lo(p.begin(), p.begin() + lo_vars), hi(p.begin() + lo_vars, p.end());
+                const std::vector<X> eqhi = eq_table(hi);
+                X x = FP::x_zero();
+                for (int k = 0; k < n.arity; k++) {
+                    const X e = tr.read_felt_ext();
+                    x = FP::x_add(x, FP::x_mul(eqhi[k], e));
+                    out[k].push_back({lo, e});
+                }
+                return x;
+            };
+            std::vector<X> u, v;
+            X fc1, fc2;
+            verify_sum_check_host<FP>(2, nv, FP::x_sub(combined, constant), tr, wo, &fc1, &u);
+            const X xu = read_evals(u);
+            const std::vector<X> equ = eq_table(u);
+            // A(u) and M(u, v), sparsely from the edges
+            X au = FP::x_zero();
+            for (size_t r = 0; r < (size_t)n.num_reps; r++)
+                for (size_t g = 0; g < n.ng; g++)
+                    for (uint64_t e = d.add_ptr[g]; e < d.add_ptr[g + 1]; e++) {
+                        const size_t x = (size_t)d.add_in[e] * n.n_in + r * sub + d.add_wire[e];
+                        au = FP::x_add(au, FP::x_mul_b(FP::x_mul(w[r * n.ng + g], equ[x]), FP::b_from_limbs(&d.add_coef[e * FP::B_LIMBS])));
+                    }
+            verify_sum_check_host<FP>(2, nv, FP::x_sub(fc1, FP::x_mul(au, xu)), tr, wo, &fc2, &v);
+            const X xv = read_evals(v);
+            const std::vector<X> eqv = eq_table(v);
+            X muv = FP::x_zero();
+            for (size_t r = 0; r < (size_t)n.num_reps; r++)
+                for (size_t g = 0; g < n.ng; g++)
+                    for (uint64_t e = d.mul_ptr[g]; e < d.mul_ptr[g + 1]; e++) {
+                        const size_t x = (size_t)d.mul_in0[e] * n.n_in + r * sub + d.mul_w0[e], y = (size_t)d.mul_in1[e] * n.n_in + r * sub + d.mul_w1[e];
+                        muv = FP::x_add(muv, FP::x_mul_b(FP::x_mul(w[r * n.ng + g], FP::x_mul(equ[x], eqv[y])), FP::b_from_limbs(&d.mul_coef[e * FP::B_LIMBS])));
+                    }
+            if (!FP::x_eq(FP::x_mul(FP::x_mul(xu, muv), xv), fc2)) throw VerifyError("InvalidSumCheck: general layer final evaluation mismatch");
         }
         return out;
     }

@@ -432,6 +432,8 @@ template <class FP> struct ScHostState {
     X pending_true[4];               // coefficients of the TRUE round polynomial of the last round
     int pending_deg = 0;
     size_t pending_chal = 0;
+    bool scaled = false;             // the device samples h / scale (phase 2 of a general layer: h = X(u) * the sampled polynomial)
+    X scale;
 };
 
 struct ScScratch {
@@ -471,15 +473,16 @@ void emit_round(Channel<FP>& ch, std::shared_ptr<ScHostState<FP>> st, size_t off
         const int slot_h1 = o.slot_h1;
         typedef RoundPoly<FP> RP;
         auto horner = [](const X* c, int deg, X x) { X r = c[deg]; for (int i = deg; i-- > 0;) r = FP::x_add(FP::x_mul(r, x), c[i]); return r; };
+        auto sample = [&](size_t i) { const X v = chp->msg(i); return st->scaled ? FP::x_mul(v, st->scale) : v; };
         X s;
         if (round0) {
-            s = FP::x_add(chp->msg(off), chp->msg(off + slot_h1));
+            s = FP::x_add(sample(off), sample(off + slot_h1));
         } else {
             X rprev = chp->chal(st->pending_chal);
             s = horner(st->pending_true, st->pending_deg, rprev);
             st->claim = horner(st->pending_wire, st->pending_deg, rprev);
         }
-        const X h0 = chp->msg(off), hinf = chp->msg(off + 1);
+        const X h0 = sample(off), hinf = sample(off + 1);
         X tc[D + 1];
         tc[0] = h0;
         tc[D] = hinf;
@@ -487,7 +490,7 @@ void emit_round(Channel<FP>& ch, std::shared_ptr<ScHostState<FP>> st, size_t off
         if (D == 2) {
             tc[1] = a;
         } else {
-            X bv = FP::x_add(FP::x_sub(chp->msg(off + 2), h0), hinf);  // c2 - c1
+            X bv = FP::x_add(FP::x_sub(sample(off + 2), h0), hinf);  // c2 - c1
             X inv2 = RP::inv_small(2);
             tc[2] = FP::x_mul(FP::x_add(a, bv), inv2);
             tc[1] = FP::x_mul(FP::x_sub(a, bv), inv2);

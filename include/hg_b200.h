@@ -231,7 +231,10 @@ int hg_circuit_insert_lasso(hg_circuit* c, hg_lasso_node* node, int* out_id);   
 /* VanillaNode::new(input_arity, log2_sub_input_size, gates, num_reps); gates in CSR form:
  *   gate g = consts[g] (if has_const[g]) + sum_{e in [add_ptr[g], add_ptr[g+1])} add_coef[e] * input[add_input[e]][rep*2^sub + add_wire[e]]
  *                                        + sum_{e in [mul_ptr[g], mul_ptr[g+1])} mul_coef[e] * input[mul_in0[e]][.. + mul_w0[e]] * input[mul_in1[e]][.. + mul_w1[e]]
- * Supported on the device: layers with additive gates only, and the element-wise product layer (VanillaGate::mul((0,i),(1,i))). */
+ * Every gate shape is supported, on the device and by the host verifier: layers with additive gates only and the element-wise
+ * product layer (VanillaGate::mul((0,i),(1,i)), num_reps = 1) keep their own layer sumcheck; any other layer with a product term
+ * (squares, products of any two wires, with coefficients, mixed with constants and sums, num_reps > 1) is proved by the two-phase
+ * layer sumcheck of DESIGN.md section 3. The CSR arrays are validated before they are used; a NULL array is an error. */
 int hg_circuit_insert_vanilla(hg_circuit* c, size_t input_arity, size_t log2_sub_input_size, size_t num_reps, size_t n_gates, const uint8_t* has_const,
                               const uint64_t* consts, const uint64_t* add_ptr, const uint64_t* add_coef, const uint32_t* add_input,
                               const uint64_t* add_wire, const uint64_t* mul_ptr, const uint64_t* mul_coef, const uint32_t* mul_in0, const uint64_t* mul_w0,
