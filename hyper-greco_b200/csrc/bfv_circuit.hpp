@@ -3,7 +3,7 @@
 // calls the C ABI exposes (hg_circuit_insert_* / hg_circuit_connect). A Rust caller that keeps `configure` as it is binds those
 // calls one by one; a caller that only wants the finished circuit (bench, tests, the verifier) calls hg_bfv_configure.
 // Works on any circuit type with insert_input / insert_fft / insert_vanilla(VanillaDesc) / connect: the device circuit
-// (GkrCircuitDev, through ICircuit) and the host-only description (GkrVerifierHost).
+// (GkrCircuitDev) and the host-only description (GkrVerifierHost).
 #pragma once
 #include <functional>
 

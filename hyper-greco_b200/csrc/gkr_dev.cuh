@@ -328,7 +328,7 @@ template <class FP> class GkrCircuitDev {
         return ch_->copy_partial_to(d_out, cap);
     }
     std::vector<std::vector<InputClaim>> emit_shard_dev(const X* d_merged, size_t count) {
-        ch_->emit_merged_device(d_merged, count);
+        ch_->emit_merged(d_merged, count);
         return collect();
     }
     // the same with the serialisation split over the devices: device `part` returns the bytes of its range of the proof (the caller

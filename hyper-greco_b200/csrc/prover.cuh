@@ -280,24 +280,18 @@ template <class FP> class Channel {
     // ---- a proof split over several devices (LassoNodeDev::prove_shard): every device fills the message slots of the terms
     // it owns and leaves the others zero; the element-wise sum over devices is the message buffer of the whole proof
     void zero_messages() { HG_CUDA(cudaMemsetAsync(d_msg_.p, 0, d_msg_.bytes(), ctx_->stream)); }
-    // bring every message to the host WITHOUT serialising (the serialisers stay queued for emit_merged)
-    const X* download_partial(size_t* count) {
-        HG_CUDA(cudaMemcpyAsync(h_msg_.p, d_msg_.p, msg_cursor_ * sizeof(X), cudaMemcpyDeviceToHost, ctx_->stream));
-        HG_CUDA(cudaStreamSynchronize(ctx_->stream));
-        *count = msg_cursor_;
-        return h_msg_.p;
-    }
-    // the same without leaving the device: copy this device's partial message buffer into a caller-owned device buffer
-    // (stream-ordered, no host synchronisation); the caller sums the buffers of all devices (k_shard_merge after an NCCL
-    // all-gather) and rank 0 hands the sum back to emit_merged_device
-    size_t copy_partial_to(X* d_out, size_t cap) {
+    // copy this device's partial message buffer to `out`, host or device memory of the caller, WITHOUT serialising (the
+    // serialisers stay queued for emit_merged). Stream-ordered, no host synchronisation. The caller sums the buffers of all
+    // devices (hg_shard_merge, or k_shard_merge after an NCCL all-gather) and rank 0 hands the sum back to emit_merged
+    size_t copy_partial_to(X* out, size_t cap) {
         if (msg_cursor_ > cap) throw std::runtime_error("Channel: shard message buffer too small");
-        HG_CUDA(cudaMemcpyAsync(d_out, d_msg_.p, msg_cursor_ * sizeof(X), cudaMemcpyDeviceToDevice, ctx_->stream));
+        HG_CUDA(cudaMemcpyAsync(out, d_msg_.p, msg_cursor_ * sizeof(X), cudaMemcpyDefault, ctx_->stream));
         return msg_cursor_;
     }
-    void emit_merged_device(const X* d_merged, size_t count) {
+    // replace the host copy of the messages by the merged one (host or device memory) and serialise
+    void emit_merged(const X* merged, size_t count) {
         if (count != msg_cursor_) throw std::runtime_error("Channel: merged message count does not match this proof");
-        HG_CUDA(cudaMemcpyAsync(h_msg_.p, d_merged, count * sizeof(X), cudaMemcpyDeviceToHost, ctx_->stream));
+        HG_CUDA(cudaMemcpyAsync(h_msg_.p, merged, count * sizeof(X), cudaMemcpyDefault, ctx_->stream));
         HG_CUDA(cudaStreamSynchronize(ctx_->stream));
         msg_ready_ = msg_cursor_;
         for (; deferred_done_ < deferred_.size(); deferred_done_++) deferred_[deferred_done_](*this);
@@ -312,7 +306,7 @@ template <class FP> class Channel {
         if (count != msg_cursor_) throw std::runtime_error("Channel: merged message count does not match this proof");
         if (nparts < 1 || part < 0 || part >= nparts) throw std::runtime_error("Channel: bad part index");
         if (tr_->hooked()) throw std::runtime_error("Channel: a sharded proof is serialised into the library's own transcript");
-        HG_CUDA(cudaMemcpyAsync(h_msg_.p, d_merged, count * sizeof(X), cudaMemcpyDeviceToHost, ctx_->stream));
+        HG_CUDA(cudaMemcpyAsync(h_msg_.p, d_merged, count * sizeof(X), cudaMemcpyDefault, ctx_->stream));
         // cut points: serialiser i may start a range if it is a plain one directly followed by a round record; weights = round records
         const size_t nd = deferred_.size();
         std::vector<size_t> cuts{0};
@@ -344,13 +338,6 @@ template <class FP> class Channel {
         out = local.proof();
     }
     bool dry() const { return dry_; }
-    // replace the host copy of the messages by the merged one and serialise
-    void emit_merged(const X* merged, size_t count) {
-        if (count != msg_cursor_) throw std::runtime_error("Channel: merged message count does not match this proof");
-        memcpy(h_msg_.p, merged, count * sizeof(X));
-        msg_ready_ = msg_cursor_;
-        for (; deferred_done_ < deferred_.size(); deferred_done_++) deferred_[deferred_done_](*this);
-    }
     size_t msg_used() const { return msg_cursor_; }
     const X* d_chal(size_t i) const { return d_chal_.p + i; }
     X* d_msg(size_t i) { return d_msg_.p + i; }
@@ -959,8 +946,9 @@ template <class FP> class LassoNodeDev {
     // stays zero, and the element-wise field sum of the message buffers over devices is the buffer a single device would
     // have produced. The challenges do not depend on the messages (SURVEY F3), so no device waits for another; the only
     // exchange is that one sum of `shard_message_count()` elements, after which rank 0 serialises (emit_shard).
-    // Returns this device's partial message buffer (pinned host memory, valid until the next prove).
-    const X* prove_shard(const B* d_inputs, size_t n_inputs, Keccak256Transcript<FP>& tr, const WireOptions& wo, int rank, int world, size_t* count) {
+    // Copies this device's partial message buffer to `out` (host or device memory of the caller, room for `cap` elements) on the
+    // context's stream and returns its length; nothing waits for the device.
+    size_t prove_shard(const B* d_inputs, size_t n_inputs, Keccak256Transcript<FP>& tr, const WireOptions& wo, int rank, int world, X* out, size_t cap) {
         if (world < 1 || rank < 0 || rank >= world || world > 2 * m_) throw std::runtime_error("LassoNode: bad shard rank / world size");
         if (!tr.prefetch_legal()) throw std::runtime_error("LassoNode: a sharded proof needs a transcript whose challenges do not depend on the messages");
         Channel<FP>& ch = *ch_;
@@ -971,9 +959,9 @@ template <class FP> class LassoNodeDev {
         ch.begin(&tr, kModePrefetch, total_chal_);
         enqueue_protocol(ch, kModePrefetch, wo, &shard_r_idx_, &shard_sum_off_);
         if (ch.chal_used() != total_chal_) throw std::runtime_error("LassoNode: challenge count mismatch");
-        return ch.download_partial(count);
+        return ch.copy_partial_to(out, cap);
     }
-    // rank 0, after prove_shard on the same node: write the proof from the merged message buffer
+    // rank 0, after prove_shard on the same node: write the proof from the merged message buffer (host or device memory)
     void emit_shard(const X* merged, size_t count, std::vector<X>* out_point, X* out_value) {
         Channel<FP>& ch = *ch_;
         ch.emit_merged(merged, count);
@@ -981,27 +969,6 @@ template <class FP> class LassoNodeDev {
         if (out_value) *out_value = ch.msg(shard_sum_off_);
     }
     size_t shard_message_count() const { return msg_budget_; }
-    // device-resident variant: the partial buffer is copied into d_out (device memory of the caller) on the context's stream,
-    // nothing waits for the device
-    size_t prove_shard_dev(const B* d_inputs, size_t n_inputs, Keccak256Transcript<FP>& tr, const WireOptions& wo, int rank, int world, X* d_out, size_t cap) {
-        if (world < 1 || rank < 0 || rank >= world || world > 2 * m_) throw std::runtime_error("LassoNode: bad shard rank / world size");
-        if (!tr.prefetch_legal()) throw std::runtime_error("LassoNode: a sharded proof needs a transcript whose challenges do not depend on the messages");
-        Channel<FP>& ch = *ch_;
-        set_shard(rank, world);
-        struct Reset { LassoNodeDev* n; ~Reset() { n->set_shard(0, 1); } } reset{this};
-        enqueue_witness(d_inputs, n_inputs, wo);
-        ch.zero_messages();
-        ch.begin(&tr, kModePrefetch, total_chal_);
-        enqueue_protocol(ch, kModePrefetch, wo, &shard_r_idx_, &shard_sum_off_);
-        if (ch.chal_used() != total_chal_) throw std::runtime_error("LassoNode: challenge count mismatch");
-        return ch.copy_partial_to(d_out, cap);
-    }
-    void emit_shard_dev(const X* d_merged, size_t count, std::vector<X>* out_point, X* out_value) {
-        Channel<FP>& ch = *ch_;
-        ch.emit_merged_device(d_merged, count);
-        if (out_point) { out_point->resize(num_vars_); for (int i = 0; i < num_vars_; i++) (*out_point)[i] = ch.chal(shard_r_idx_ + i); }
-        if (out_value) *out_value = ch.msg(shard_sum_off_);
-    }
     // which device of a sharded proof this node works for (GkrCircuitDev::enqueue sets it around the node's two enqueue calls)
     void set_shard(int rank, int world) { shard_rank_ = rank; shard_world_ = world; }
 
