@@ -534,10 +534,9 @@ struct FrField {
     static constexpr int FIELD_ID = 1;
     static constexpr int B_LIMBS = 4, X_LIMBS = 4;
     static constexpr int PLANES = 1;  // base planes per extension element
-    static constexpr int GP_TAIL_LOG = 5, GP_MIN_BLOCKS = 1, GP_R0_U = 2, GP_R0A_QPT = 1, GP_BLOCK = 128;
+    static constexpr int GP_TAIL_LOG = 5, GP_MIN_BLOCKS = 1, GP_BLOCK = 128;
     static constexpr int GP_FOLD_CTAS = 3;      // CTAs of GP_BLOCK threads per SM the fold kernels are compiled for
     static constexpr int FUSED_MIN_BLOCKS = 2;
-    static constexpr int GP_MID_LOG = 0;
     static constexpr int GP_TAIL_GROUPS = 4;
     static constexpr int GP_BALANCE = 0;
     static constexpr double GP_TARGET = 2.0;

@@ -24,11 +24,9 @@ struct GlField {
     HG_HD static B root_of_unity() { return 0x185629dcda58878cULL; }  // 7^((p-1)/2^32), goldilocks ROOT_OF_UNITY (A9)
     static constexpr int TWO_ADICITY = 32;
     static constexpr int PLANES = 2;  // base planes per extension element
-    static constexpr int GP_TAIL_LOG = 7, GP_MIN_BLOCKS = 2, GP_R0_U = 4, GP_R0A_QPT = 4, GP_BLOCK = 128;
+    static constexpr int GP_TAIL_LOG = 7, GP_MIN_BLOCKS = 2, GP_BLOCK = 128;
     static constexpr int GP_FOLD_CTAS = 4;      // CTAs of GP_BLOCK threads per SM the fold kernels are compiled for (5: 96 registers, 430-530 B of spills, GP class 1.97 instead of 1.66 ms)
     static constexpr int FUSED_MIN_BLOCKS = 4;  // CTAs of HG_FUSED_BLOCK threads per SM the fused tree builders are compiled for (gp_fused.cuh)
-    static constexpr int GP_MID_LOG = 0;        // tables of at most 2^GP_MID_LOG entries: the remaining rounds run in mid stages (k_gp_mid); 0 = off.
-                                                // Measured slower on B200 (profiles/r2_experiments.md: GP class 1.69 ms off, 1.90 ms at 11, 2.42 ms at 13), kept for experiments
     static constexpr int GP_TAIL_GROUPS = 8;    // CTAs a layer is split over (by terms) in the tail kernel (profiles/r2_experiments.md)
     static constexpr int GP_BALANCE = 1;        // work-balanced term groups in the batched layer sumchecks (prover.cuh run_gp_batch)
     static constexpr double GP_TARGET = 0.25;  // CTAs per SM (of 256 threads) from which a layer runs with one term group (prover.cuh)

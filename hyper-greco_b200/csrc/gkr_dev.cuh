@@ -102,14 +102,13 @@ template <class FP> class GkrCircuitDev {
         up(n.consts, cg);
         {   // forward runs (k_vanilla_runs): maximal stretches of gates with the same number of edge slots, every slot walking one input
             // wire by wire with one coefficient, and the same constant
-            static const bool env_fwd = getenv("HG_FWD_RUNS") ? atoi(getenv("HG_FWD_RUNS")) != 0 : true;
             typedef typename Node::FwdRun FwdRun;
-            bool ok = env_fwd;
-            if (ok && n.is_elemmul) {
+            bool ok = true;
+            if (n.is_elemmul) {
                 FwdRun r; r.g0 = 0; r.len = ng; r.ne = -2; r.cst = FP::b_zero();
                 r.in[0] = 0; r.in[1] = 1; r.w0[0] = r.w0[1] = 0; r.coef[0] = r.coef[1] = FP::b_one();
                 n.fwd_runs.push_back(r);
-            } else if (ok && n.is_linear) {
+            } else if (n.is_linear) {
                 for (size_t g = 0; ok && g < ng; g++) {
                     const uint64_t e0 = d.add_ptr[g], ne = d.add_ptr[g + 1] - e0;
                     if (ne > (uint64_t)HG_FWD_MAXE) { ok = false; break; }
@@ -145,8 +144,7 @@ template <class FP> class GkrCircuitDev {
                     }
             up(n.rev_ptr, rp); up(n.rev_out, ro); up(n.rev_coef, rc);
             // piecewise-identity wiring (k_wiring_runs): maximal runs of elements with one reader each, consecutive outputs, one coefficient
-            static const bool env_runs = getenv("HG_WIRE_RUNS") ? atoi(getenv("HG_WIRE_RUNS")) != 0 : true;
-            bool compressible = env_runs;
+            bool compressible = true;
             typedef typename Node::WireRun WireRun;
             for (size_t x = 0; compressible && x < S; x++) {
                 const uint64_t deg = rp[x + 1] - rp[x];
@@ -513,18 +511,16 @@ template <class FP> class GkrCircuitDev {
             int maxv = 0;
             for (auto& j : mine) maxv = std::max(maxv, std::min(j.nv, stream_end(j)));
             for (int r = 0; r < maxv; r++) launch_round(ch, mine, r);
-            launch_mid(ch, mine);
             launch_tail(ch, mine);
             launch_finals(ch, mine);
             early = fork && !sharded;
         }
-        static const bool env_early = getenv("HG_EARLY_FLUSH") ? atoi(getenv("HG_EARLY_FLUSH")) != 0 : true;
-        if (early && env_early) ch.arm_early(ctx_->ev_join);  // after the StreamSwap scope: ev_join marks the end of every node sumcheck
+        if (early) ch.arm_early(ctx_->ev_join);  // after the StreamSwap scope: ev_join marks the end of every node sumcheck
         const double t4 = now();
         timing_[0] = t1 - t0; timing_[1] = t2 - t1; timing_[2] = t3 - t2; timing_[3] = t4 - t3;
     }
 
-    struct Work { DevBuf<X> wbuf0, wbuf1, tbuf0, tbuf1, capture, midpart; };
+    struct Work { DevBuf<X> wbuf0, wbuf1, tbuf0, tbuf1, capture; };
     struct Node {
         int kind = GKR_INPUT, log2_size = 0, num_reps = 1, arity = 0, log2_sub = 0;
         bool fft_inverse = false, is_linear = false, is_elemmul = false, is_general = false, has_consts = false;
@@ -909,8 +905,7 @@ template <class FP> class GkrCircuitDev {
         size_t part_off = 0, bytes = 0;
         size_t round_pairs = 0;  // small rounds get one pair per thread (more CTAs), large ones up to 16 (fewer block-level reductions)
         // prefetch mode: round 0 of every job with a streamed round 1 is sampled by that round's launch (k_prod_round_multi FUSE0)
-        static const bool env_fuse0 = getenv("HG_PROD_FUSE0") ? atoi(getenv("HG_PROD_FUSE0")) != 0 : true;
-        auto fused0 = [&](const Job& j) { return env_fuse0 && use_tail_ && j.nv >= 2 && stream_end(j) >= 2; };
+        auto fused0 = [&](const Job& j) { return use_tail_ && j.nv >= 2 && stream_end(j) >= 2; };
         for (const Job& j : jobs) if (r < j.nv && r < stream_end(j) && !(r == 0 && fused0(j))) round_pairs += r == 0 ? j.S / 2 : (j.S >> (r - 1)) / 4;
         bool any_fused = false;
         for (const Job& j : jobs) {
@@ -935,7 +930,7 @@ template <class FP> class GkrCircuitDev {
             it.msg = ch.d_msg(j.msg_off + 4 * (size_t)(fuse ? 0 : r));
             const size_t npairs = r == 0 ? it.n_in / 2 : it.n_in / 4;
             // several pairs per thread: the block-level reduction that ends every block costs about as much as eight pairs (measured optimum 8-16)
-            static const size_t ppt_max = getenv("HG_PROD_PPT") ? (size_t)atoi(getenv("HG_PROD_PPT")) : 16;
+            constexpr size_t ppt_max = 16;
             const size_t ppt = std::max<size_t>(1, std::min<size_t>(ppt_max, round_pairs / ((size_t)HG_PROD_BLOCK * ctx_->sm_count * 4)));
             size_t b = std::max<size_t>(1, std::min<size_t>((npairs + HG_PROD_BLOCK * ppt - 1) / (HG_PROD_BLOCK * ppt), (size_t)ctx_->sm_count * 16 * (HG_BLOCK / HG_PROD_BLOCK)));
             it.nblk = (int)b; it.bx = (int)b; it.blk_start = blk;
@@ -972,57 +967,19 @@ template <class FP> class GkrCircuitDev {
     }
 
     // first round that is NOT streamed: the tail kernel takes over there (prefetch mode only; nv when the job has no tail)
-    // Round schedule of a job in prefetch mode (use_tail_): rounds [0, stream_end) are streamed, one launch per round for all jobs;
-    // sumchecks with nv >= 12 then run HG_PROD_MID_K rounds in ONE launch on 1024-entry segments in shared memory (k_prod_mid),
-    // and the rest (tables of <= 2^10 entries) in the one-CTA-per-job tail kernel. Without use_tail_ every round is streamed.
-    static constexpr int HG_PROD_MID_LOG = 15;  // the mid stage starts when the tables are down to 2^(HG_PROD_MID_LOG+1) entries
-    bool has_mid(const Job& j) const { return use_tail_ && use_mid_ && j.nv >= 12; }
+    // Round schedule of a job in prefetch mode (use_tail_): rounds [0, stream_end) are streamed, one launch per round for all jobs,
+    // and the rest (tables of <= 2^10 entries) run in the one-CTA-per-job tail kernel. Without use_tail_ every round is streamed.
     int stream_end(const Job& j) const {
         if (!use_tail_ || j.nv < 3) return j.nv;
-        return has_mid(j) ? std::max(2, j.nv - HG_PROD_MID_LOG) : std::max(2, j.nv - HG_PROD_TAIL_LOG);
+        return std::max(2, j.nv - HG_PROD_TAIL_LOG);
     }
-    int tail_start(const Job& j) const { return stream_end(j) + (has_mid(j) ? HG_PROD_MID_K : 0); }
-    // mid stage of every job that has one: input = output of streaming round stream_end - 1, K rounds, output 2 entries per segment
-    void launch_mid(Channel<FP>& ch, const std::vector<Job>& jobs) {
-        cudaStream_t s = ctx_->stream;
-        std::vector<ProdMidItem<FP>> items;
-        int blk = 0, nt_max = 1;
-        size_t bytes = 0;
-        for (const Job& j : jobs) {
-            if (!has_mid(j)) continue;
-            Node& n = *nodes_[j.node];
-            Work& wb = wk(j);
-            const int se = stream_end(j);
-            ProdMidItem<FP> it;
-            it.n_in = j.S >> (se - 1);
-            if (it.n_in < 2 * (size_t)HG_PROD_MID_SEG || (it.n_in % HG_PROD_MID_SEG)) throw std::runtime_error("gkr: mid stage on a table that is too small");
-            it.nt = j.nt; it.nseg = (int)(it.n_in / HG_PROD_MID_SEG); it.blk_start = blk;
-            it.w_in = ((se - 1) & 1) ? wb.wbuf0.p : wb.wbuf1.p;  it.tab_in = ((se - 1) & 1) ? wb.tbuf0.p : wb.tbuf1.p;
-            it.w_out = (se & 1) ? wb.wbuf0.p : wb.wbuf1.p;       it.tab_out = (se & 1) ? wb.tbuf0.p : wb.tbuf1.p;
-            it.chal = ch.d_chal(j.r0_idx + se - 1);
-            if (wb.midpart.n < (size_t)HG_PROD_MID_K * it.nseg * 4) { HG_CUDA(cudaStreamSynchronize(s)); wb.midpart.alloc((size_t)HG_PROD_MID_K * it.nseg * 4); }
-            it.part = wb.midpart.p;
-            it.capture = nullptr; it.cap_round = -1; it.arity = n.arity;
-            if (lin(n)) {
-                const int m = log2sz(n.n_in);
-                if (m >= se && m < se + HG_PROD_MID_K) { it.capture = wb.capture.p; it.cap_round = m - se; }
-            }
-            blk += it.nseg;
-            nt_max = std::max(nt_max, j.nt);
-            bytes += (size_t)(j.nt + 1) * it.n_in * sizeof(X);
-            items.push_back(it);
-        }
-        if (items.empty()) return;
-        prod_mid_set_smem<FP>();
-        HG_K(ctx_, KC_GKR_SC, bytes, k_prod_mid<FP><<<blk, 256, prod_mid_smem<FP>(nt_max), s>>>(stage(items), (int)items.size()));
-    }
-    // rounds tail_start .. nv-1 and the input evaluations of every job that has a tail, one CTA per job
+    // rounds stream_end .. nv-1 and the input evaluations of every job that has a tail, one CTA per job
     void launch_tail(Channel<FP>& ch, const std::vector<Job>& jobs) {
         cudaStream_t s = ctx_->stream;
         std::vector<ProdTailItem<FP>> items;
         size_t smem = 0, bytes = 0;
         for (const Job& j : jobs) {
-            const int rt = tail_start(j);
+            const int rt = stream_end(j);
             if (rt >= j.nv) continue;
             Node& n = *nodes_[j.node];
             Work& wb = wk(j);
@@ -1031,13 +988,6 @@ template <class FP> class GkrCircuitDev {
             t.w_in = ((rt - 1) & 1) ? wb.wbuf0.p : wb.wbuf1.p;
             t.tab_in = ((rt - 1) & 1) ? wb.tbuf0.p : wb.tbuf1.p;
             t.mid_part = nullptr; t.mid_msg = nullptr; t.mid_nseg = 0; t.mid_rounds = 0;
-            if (has_mid(j)) {  // the mid stage wrote its pairs where streaming round stream_end would have written
-                const int se = stream_end(j);
-                t.w_in = (se & 1) ? wb.wbuf0.p : wb.wbuf1.p;
-                t.tab_in = (se & 1) ? wb.tbuf0.p : wb.tbuf1.p;
-                t.mid_part = wb.midpart.p; t.mid_nseg = (int)((j.S >> (se - 1)) / HG_PROD_MID_SEG); t.mid_rounds = HG_PROD_MID_K;
-                t.mid_msg = ch.d_msg(j.msg_off + 4 * (size_t)se);
-            }
             t.chal = ch.d_chal(j.r0_idx + rt - 1);
             t.msg = ch.d_msg(j.msg_off + 4 * (size_t)rt);
             t.evals = ch.d_msg(j.evals_off);
@@ -1064,7 +1014,7 @@ template <class FP> class GkrCircuitDev {
         std::vector<FoldItem<FP>> folds;
         std::vector<CopyItem<FP>> copies;
         for (const Job& j : jobs) {
-            if (tail_start(j) < j.nv) continue;  // done by launch_tail
+            if (stream_end(j) < j.nv) continue;  // done by launch_tail
             Node& n = *nodes_[j.node];
             Work& wb = wk(j);
             // state after the last round launch (round nv-1): tables folded by r_0..r_{nv-2}, length 2
@@ -1098,10 +1048,6 @@ template <class FP> class GkrCircuitDev {
     std::vector<std::unique_ptr<Node>> nodes_;
     std::vector<int> topo_;
     bool evaluated_ = false, planned_ = false, eval_planned_ = false, use_tail_ = false;
-    // measured on B200 (n = 32768): for the ~70 node sumchecks the mid stage is SLOWER than the streamed rounds it replaces (0.86 vs 0.76 ms
-    // for the class: ~2000 CTAs that each run 9 serial rounds), so it is off here; the Lasso collation sumcheck (one job, 18 us per
-    // streamed round whatever the size) uses it (sumcheck_dev: 0.24 -> 0.19 ms, 13 -> 5 launches)
-    bool use_mid_ = getenv("HG_PROD_MID_LAYERS") ? atoi(getenv("HG_PROD_MID_LAYERS")) != 0 : false;
     size_t tail_smem_ = 0;
     std::vector<EvalLevel> eval_levels_;
     size_t total_chal_ = 0, desc_off_ = 0, eq_off_ = 0;

@@ -414,7 +414,7 @@ template <class FP> struct ProdTailItem {
     typename FP::X* evals;
     const typename FP::X* capture;                               // linear layers whose capture round ran in the streaming part, else nullptr
     int n_in, nt, rounds, linear, arity, cap_round;              // cap_round: index (0-based within the tail) of the round whose folded table holds the input evaluations, -1: none
-    const typename FP::X* mid_part;                              // rounds done by k_prod_mid before this tail: CTA partial sums [mid_rounds][mid_nseg][4] ...
+    const typename FP::X* mid_part;                              // rounds done by k_prod_mid_one before this tail: CTA partial sums [mid_rounds][mid_nseg][4] ...
     typename FP::X* mid_msg;                                     // ... summed into the 4 message slots of each of those rounds (nullptr: no mid stage)
     int mid_nseg, mid_rounds;
 };
@@ -427,7 +427,7 @@ template <class FP> __device__ __forceinline__ void prod_tail_body(const ProdTai
     X* red = nxt + (size_t)ntab * (it.n_in / 2);        // [32][3]
     for (int e = threadIdx.x; e < len; e += blockDim.x) cur[e] = it.w_in[e];
     for (int e = threadIdx.x; e < nt * len; e += blockDim.x) cur[len + e] = it.tab_in[e];
-    if (it.mid_msg)  // the messages of the rounds k_prod_mid ran: add up its CTA partials (field addition is exact: any order)
+    if (it.mid_msg)  // the messages of the rounds k_prod_mid_one ran: add up its CTA partials (field addition is exact: any order)
         for (int t = threadIdx.x; t < 4 * it.mid_rounds; t += blockDim.x) {
             const int rd = t >> 2, p = t & 3;
             X s = FP::x_zero();
@@ -488,7 +488,7 @@ template <class FP> struct ProdMidItem {
     typename FP::X* part;                                        // [K][nseg][4]
     typename FP::X* capture;                                     // linear layers whose capture round falls into this stage (else nullptr)
     unsigned long long n_in;
-    int nt, nseg, blk_start, cap_round, arity;
+    int nt, nseg, cap_round, arity;
 };
 template <class FP> __device__ __forceinline__ void prod_mid_body(const ProdMidItem<FP>& it, const int seg, unsigned char* smem_raw) {
     typedef typename FP::X X;
@@ -552,11 +552,6 @@ template <class FP> __device__ __forceinline__ void prod_mid_body(const ProdMidI
     }
 }
 
-template <class FP> __global__ void __launch_bounds__(256) k_prod_mid(const ProdMidItem<FP>* __restrict__ items, int nitems) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const ProdMidItem<FP> it = items[find_item(items, nitems)];
-    prod_mid_body<FP>(it, blockIdx.x - it.blk_start, smem_raw);
-}
 // a single sumcheck (the Lasso collation sumcheck): descriptor by value
 template <class FP> __global__ void __launch_bounds__(256) k_prod_mid_one(const ProdMidItem<FP> it) {
     extern __shared__ __align__(16) unsigned char smem_raw[];

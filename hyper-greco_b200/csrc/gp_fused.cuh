@@ -7,7 +7,7 @@
 // get the layer above: q_i(b; 0) = l_i(2b) r_i(2b) and q_i(b; 1) = l_i(2b+1) r_i(2b+1) ARE the two tree entries it writes.
 // With all challenges known up front (c_i = gamma_layer^i, transcript.rs:156,183-203) the builder therefore emits the four
 // samples h(0), h(inf), h(-1), h(1) itself and the layer is never re-read for round 0 (2.6 GB less traffic per proof at
-// n = 32768: the two former round-0 launches, k_gp_r0a_multi and k_gp_r0_multi, are gone from the prefetch path).
+// n = 32768 than a separate round-0 pass).
 //   * q_i(b; X) = l_i r_i is quadratic in X: q(inf) costs one product of slopes, q(-1) = 2 q(0) - q(1) + 2 q(inf) none;
 //   * per vector i the base-field sums D_i(p) = sum_b t_0(b; p) q_i(b; p) are accumulated unreduced and multiplied by the
 //     extension coefficient c_i once per thread;

@@ -203,8 +203,7 @@ constexpr int HG_GP_TAIL_MAXR = 10;  // most rounds the tail kernel runs (tables
 #endif
 
 template <class FP> struct GpItem {
-    const void* in;                  // tables read this round (base in rounds 0/1, extension later): [2*nvec][n_in]
-    const void* parent;              // round 0, first half: the tree layer above, [nvec][n_in] base elements = l_i * r_i
+    const void* in;                  // tables read this round (base in round 1, extension later): [2*nvec][n_in]
     typename FP::X* out;             // folded tables written this round: [2*nvec][n_in/2]
     unsigned long long n_in;
     const typename FP::X* c;         // c_i
@@ -221,7 +220,7 @@ template <class FP> struct GpItem {
 
 template <class FP, int NP>
 __device__ __forceinline__ void block_reduce_finalize_ex(typename FP::X (&acc)[NP], typename FP::X* partials, unsigned* counter,
-                                                         typename FP::X* out, unsigned nblk, unsigned bid, int out_stride = 1) {
+                                                         typename FP::X* out, unsigned nblk, unsigned bid) {
     typedef typename FP::X X;
     __shared__ X sm[32][NP];
     __shared__ bool is_last;
@@ -272,7 +271,7 @@ __device__ __forceinline__ void block_reduce_finalize_ex(typename FP::X (&acc)[N
             X v = lane < nwarps ? sm[lane][p] : FP::x_zero();
 #pragma unroll
             for (int off = 16; off > 0; off >>= 1) v = FP::x_add(v, FP::x_shfl_down(v, off));
-            if (lane == 0) out[p * out_stride] = v;
+            if (lane == 0) out[p] = v;
         }
         if (lane == 0) *counter = 0;
     }
@@ -288,112 +287,6 @@ template <class ITEM> __device__ __forceinline__ int find_item(const ITEM* items
     return lo;
 }
 template <class FP> __device__ __forceinline__ int gp_find_item(const GpItem<FP>* items, int nitems) { return find_item(items, nitems); }
-
-// Round 0 is split in two launches.
-// (a) h(0) and h(1): l_i(2b) * r_i(2b) and l_i(2b+1) * r_i(2b+1) are entries 2b, 2b+1 of the tree layer ABOVE (Layer::up,
-//     prover.rs:332-354, already in memory), so these two samples need no product of l and r:
-//         h(0) = sum_b t_0(2b) * sum_i c_i parent_i(2b),   h(1) the same at 2b+1         -> msg[0], msg[3]
-//     computed as sum_i c_i * D_i with the base-field dot products D_i = sum_b t_0(2b) parent_i(2b) (resp. 2b+1): per entry
-//     one unreduced 64x64 multiply-add; c_i is applied once per term and thread.
-template <class FP>
-__global__ void __launch_bounds__(FP::GP_BLOCK, 2 * (HG_BLOCK / FP::GP_BLOCK)) k_gp_r0a_multi(const GpItem<FP>* __restrict__ items, int nitems) {
-    typedef typename FP::B B;
-    typedef typename FP::X X;
-    constexpr int QPT = FP::GP_R0A_QPT;  // quads (4 consecutive entries = two pairs) per thread and term
-    const GpItem<FP> it = items[gp_find_item<FP>(items, nitems)];
-    const unsigned lb = blockIdx.x - it.blk_start;
-    const unsigned bxi = lb % it.bx, grp = lb / it.bx;
-    const B* tables = (const B*)it.in;
-    const B* parent = (const B*)it.parent;
-    const size_t n = it.n_in, nquads = n / 4;
-    const int i0 = it.i_begin + grp * it.tpg, i1 = min(it.i_end, i0 + it.tpg);
-    typename FP::XAcc accx[2] = {FP::xacc_zero_(), FP::xacc_zero_()};
-    for (size_t q0 = (size_t)bxi * (blockDim.x * QPT) + threadIdx.x; q0 < nquads; q0 += (size_t)it.bx * blockDim.x * QPT) {
-        for (int i = i0; i < i1; i++) {
-            const B* pi = parent + (size_t)i * n;
-            B p[QPT][4];
-#pragma unroll
-            for (int k = 0; k < QPT; k++) {
-                const size_t q = q0 + (size_t)k * blockDim.x;
-#pragma unroll
-                for (int e = 0; e < 4; e++) p[k][e] = FP::b_zero();
-                if (q < nquads) load4(pi + 4 * q, p[k]);
-            }
-            typename FP::BAcc d0 = FP::bacc_zero(), d1 = FP::bacc_zero();
-#pragma unroll
-            for (int k = 0; k < QPT; k++) {
-                const size_t q = q0 + (size_t)k * blockDim.x;
-                if (q < nquads) {
-                    const B* t = tables + 4 * q;  // t_0: the same addresses for every term, served by L1
-                    FP::bacc_mad(d0, t[0], p[k][0]);
-                    FP::bacc_mad(d1, t[1], p[k][1]);
-                    FP::bacc_mad(d0, t[2], p[k][2]);
-                    FP::bacc_mad(d1, t[3], p[k][3]);
-                }
-            }
-            const X c = it.c[i];
-            FP::xacc_mad_b(accx[0], c, FP::bacc_reduce(d0));
-            FP::xacc_mad_b(accx[1], c, FP::bacc_reduce(d1));
-        }
-    }
-    X acc[2] = {FP::xacc_reduce_(accx[0]), FP::xacc_reduce_(accx[1])};
-    block_reduce_finalize_ex<FP, 2>(acc, it.partials, it.counter, it.msg, it.nblk, lb, 3);
-}
-// (b) h(inf) and h(-1) from the slopes / values at -1 of t_0, l_i, r_i                       -> msg[1], msg[2]
-template <class FP, int U>
-__global__ void __launch_bounds__(FP::GP_BLOCK, FP::GP_MIN_BLOCKS * (HG_BLOCK / FP::GP_BLOCK)) k_gp_r0_multi(const GpItem<FP>* __restrict__ items, int nitems) {
-    typedef typename FP::B B;
-    typedef typename FP::X X;
-    constexpr int NP = 2;
-    const GpItem<FP> it = items[gp_find_item<FP>(items, nitems)];
-    const unsigned lb = blockIdx.x - it.blk_start;
-    const unsigned bxi = lb % it.bx, grp = lb / it.bx;
-    const B* tables = (const B*)it.in;
-    const size_t n = it.n_in, npairs = n / 2, stride = (size_t)it.bx * blockDim.x;
-    const int i0 = it.i_begin + grp * it.tpg, i1 = min(it.i_end, i0 + it.tpg);
-    typename FP::XAcc accx[NP];
-#pragma unroll
-    for (int p = 0; p < NP; p++) accx[p] = FP::xacc_zero_();
-    for (size_t b0 = (size_t)bxi * blockDim.x + threadIdx.x; b0 < npairs; b0 += stride * U) {
-        B t0[U][NP];
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const size_t b = b0 + u * stride;
-            B p[2] = {FP::b_zero(), FP::b_zero()};
-            if (b < npairs) load2(tables + 2 * b, p);
-            t0[u][0] = FP::slope(p[0], p[1]); t0[u][1] = FP::at_m1(p[0], p[1]);
-        }
-        for (int i = i0; i < i1; i++) {
-            const B* li = tables + (size_t)i * 2 * n;
-            const B* ri = li + n;
-            B l[U][2], r[U][2];
-#pragma unroll
-            for (int u = 0; u < U; u++) {
-                const size_t b = b0 + u * stride;
-                l[u][0] = l[u][1] = r[u][0] = r[u][1] = FP::b_zero();
-                if (b < npairs) {
-                    load2(li + 2 * b, l[u]); load2(ri + 2 * b, r[u]);
-                    if (i + HG_GP_PREFETCH < i1) { prefetch_l2(li + (size_t)HG_GP_PREFETCH * 2 * n + 2 * b); prefetch_l2(ri + (size_t)HG_GP_PREFETCH * 2 * n + 2 * b); }
-                }
-            }
-            typename FP::BAcc s[NP];
-#pragma unroll
-            for (int p = 0; p < NP; p++) s[p] = FP::bacc_zero();
-#pragma unroll
-            for (int u = 0; u < U; u++) {
-                FP::bacc_mad(s[0], t0[u][0], FP::fmul(FP::slope(l[u][0], l[u][1]), FP::slope(r[u][0], r[u][1])));
-                FP::bacc_mad(s[1], t0[u][1], FP::fmul(FP::at_m1(l[u][0], l[u][1]), FP::at_m1(r[u][0], r[u][1])));
-            }
-            const X c = it.c[i];
-#pragma unroll
-            for (int p = 0; p < NP; p++) FP::xacc_mad_b(accx[p], c, FP::bacc_reduce(s[p]));
-        }
-    }
-    X acc[NP];
-#pragma unroll
-    for (int p = 0; p < NP; p++) acc[p] = FP::xacc_reduce_(accx[p]);
-    block_reduce_finalize_ex<FP, NP>(acc, it.partials, it.counter, it.msg + 1, it.nblk, lb);
-}
 
 template <class FP, class TIN, bool SCALE>
 __global__ void __launch_bounds__(FP::GP_BLOCK, FP::GP_FOLD_CTAS) k_gp_fold_multi(const GpItem<FP>* __restrict__ items, int nitems) {
@@ -485,10 +378,6 @@ template <class FP> __global__ void k_gp_coeffs_multi(const GpCoeffItem<FP>* __r
 }
 
 // ---- tail: one CTA per layer, tables in shared memory, all remaining rounds + the final evaluations
-constexpr int HG_GP_MID_STAGES = 3;   // mid stages per layer (each folds up to HG_GP_MID_MAXK rounds)
-constexpr int HG_GP_MID_SEG = 64;     // entries of a table one mid CTA owns
-constexpr int HG_GP_MID_MAXK = 5;     // 64 -> 2 entries
-constexpr int HG_GP_MID_THREADS = 256;
 template <class FP> struct GpTailItem {
     const void* in;                 // from_base: base tables [nvec][2n]; else extension tables [2*nvec][n] (already scaled)
     const typename FP::X* c;
@@ -500,11 +389,6 @@ template <class FP> struct GpTailItem {
     int i_begin, i_end;             // owned terms (see GpItem)
     const typename FP::X* r0part;   // !from_base: round-0 partial sums of the fused tree builders (gp_fused.cuh), [r0n][4], summed into msg0
     int r0n;
-    // rounds that ran in mid stages (k_gp_mid): stage s left mid_K[s] x mid_n[s] CTA partial sums, [K][n][3]; their sums are the
-    // messages mid_msg[s][3 * q + p]
-    const typename FP::X* mid_part[HG_GP_MID_STAGES];
-    typename FP::X* mid_msg[HG_GP_MID_STAGES];
-    int mid_n[HG_GP_MID_STAGES], mid_K[HG_GP_MID_STAGES];
     // the layer's terms are split over `groups` CTAs of tpg terms; gpart: [groups][1 + HG_GP_TAIL_MAXR][4] partial sums
     int tpg, groups;
     typename FP::X* gpart;
@@ -590,23 +474,12 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
             const size_t tab = slot ? (size_t)(2 * i0 + slot - 1) : 0;
             A[e] = src[tab * len + k];
         }
-        if (g == 0) {
-            if (it.r0n > 0) {  // round 0 was sampled while the tree was built: add up the CTA partials
-                X acc[4] = {FP::x_zero(), FP::x_zero(), FP::x_zero(), FP::x_zero()};
-                for (int b = threadIdx.x; b < it.r0n; b += blockDim.x)
+        if (g == 0 && it.r0n > 0) {  // round 0 was sampled while the tree was built: add up the CTA partials
+            X acc[4] = {FP::x_zero(), FP::x_zero(), FP::x_zero(), FP::x_zero()};
+            for (int b = threadIdx.x; b < it.r0n; b += blockDim.x)
 #pragma unroll
-                    for (int p = 0; p < 4; p++) acc[p] = FP::x_add(acc[p], it.r0part[(size_t)b * 4 + p]);
-                tail_block_sum<FP, 4>(acc, red, it.msg0);
-            }
-            for (int st = 0; st < HG_GP_MID_STAGES; st++)  // rounds that ran in mid stages: add up the CTA partials of every round
-                for (int q = 0; q < it.mid_K[st]; q++) {
-                    X acc[3] = {FP::x_zero(), FP::x_zero(), FP::x_zero()};
-                    const X* part = it.mid_part[st] + (size_t)q * it.mid_n[st] * 3;
-                    for (int b = threadIdx.x; b < it.mid_n[st]; b += blockDim.x)
-#pragma unroll
-                        for (int p = 0; p < 3; p++) acc[p] = FP::x_add(acc[p], part[(size_t)b * 3 + p]);
-                    tail_block_sum<FP, 3>(acc, red, it.mid_msg[st] + 3 * q);
-                }
+                for (int p = 0; p < 4; p++) acc[p] = FP::x_add(acc[p], it.r0part[(size_t)b * 4 + p]);
+            tail_block_sum<FP, 4>(acc, red, it.msg0);
         }
         __syncthreads();
     }
@@ -667,93 +540,6 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
         if (slot == 0) it.msg0[p] = v; else it.msg[3 * (slot - 1) + p] = v;
     }
     if (threadIdx.x == 0) *it.counter = 0;
-}
-
-}  // namespace hg
-
-namespace hg {
-// ---- mid stage: K (<= 5) consecutive rounds of a layer in ONE launch, for the rounds whose tables are too short to fill the GPU
-// (profiles/r2_launch_list.md: the streamed rounds 8..14 take 11-26 us each for < 30 MB). Folding pairs (2b, 2b+1) is local to a
-// segment of 2^K consecutive entries, so a CTA that owns HG_GP_MID_SEG = 64 consecutive entries of its tables runs the K rounds in
-// shared memory; only its partial sums per round leave it, and the tables come back 2^K times shorter (64 >> K entries per segment).
-// h is linear in the terms: a segment's terms are split over `groups` CTAs, each with its own copy of t_0. The tail kernel adds the
-// partial sums up (GpTailItem::mid_part). Same arithmetic as k_gp_tail, so the messages are the same field elements.
-template <class FP> struct GpMidItem {
-    const typename FP::X* in;    // [2*nvec][n_in], already scaled (a streamed round >= 1 ran before)
-    typename FP::X* out;         // [2*nvec][n_in >> K]
-    unsigned long long n_in;
-    const typename FP::X* chal;  // chal[q]: the challenge folded in the q-th round of the stage
-    typename FP::X* part;        // [K][nseg * groups][3]
-    int nvec, K, nseg, groups, tpg, blk_start;
-    int i_begin, i_end, write_t0;  // owned terms (see GpItem); table 0 is written by group 0 when term 0 is not owned
-};
-template <class FP> inline size_t gp_mid_smem(int tpg) {
-    return ((size_t)(1 + 2 * tpg) * (HG_GP_MID_SEG + HG_GP_MID_SEG / 2) + 32 * 4) * sizeof(typename FP::X);
-}
-template <class FP> __global__ void __launch_bounds__(HG_GP_MID_THREADS) k_gp_mid(const GpMidItem<FP>* __restrict__ items, int nitems) {
-    typedef typename FP::X X;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    constexpr int SEG = HG_GP_MID_SEG;
-    const GpMidItem<FP> it = items[find_item(items, nitems)];
-    const int lb = (int)blockIdx.x - it.blk_start;
-    const int seg = lb % it.nseg, grp = lb / it.nseg;
-    const int i0 = it.i_begin + grp * it.tpg, i1 = min(it.i_end, i0 + it.tpg);
-    const int nt = i1 - i0, ntab = 1 + 2 * nt;  // slot 0: t_0 (table 0); slots 1 + 2k, 2 + 2k: l, r of term i0 + k
-    const int cap = 1 + 2 * it.tpg;
-    X* A = reinterpret_cast<X*>(smem_raw);   // [cap][SEG]
-    X* Bf = A + (size_t)cap * SEG;            // [cap][SEG / 2]
-    X* red = Bf + (size_t)cap * (SEG / 2);    // [32][4]
-    const size_t n_in = it.n_in;
-    for (int e = threadIdx.x; e < ntab * SEG; e += blockDim.x) {
-        const int slot = e / SEG, k = e % SEG;
-        const size_t tab = slot ? (size_t)(2 * i0 + slot - 1) : 0;
-        A[e] = it.in[tab * n_in + (size_t)seg * SEG + k];
-    }
-    __syncthreads();
-    X* cur = A;
-    X* nxt = Bf;
-    int len = SEG;
-    const int ncta = it.nseg * it.groups;
-    for (int q = 0; q < it.K; q++) {
-        const X r = it.chal[q];
-        const typename FP::FoldAux aux = FP::fold_aux(r);
-        const int npairs = len / 4, half = len / 2;
-        X acc[3] = {FP::x_zero(), FP::x_zero(), FP::x_zero()};
-        for (int b = threadIdx.x; b < npairs; b += blockDim.x) {  // this CTA's copy of t_0
-            const X* t = cur + 4 * b;
-            nxt[2 * b] = FP::fold(t[0], t[1], r, aux);
-            nxt[2 * b + 1] = FP::fold(t[2], t[3], r, aux);
-        }
-        for (int e = threadIdx.x; e < nt * npairs; e += blockDim.x) {
-            const int k = e / npairs, b = e % npairs;
-            const X* t = cur + 4 * b;
-            const X* l = cur + (1 + 2 * k) * len + 4 * b;
-            const X* g = cur + (2 + 2 * k) * len + 4 * b;
-            const X t_lo = FP::fold(t[0], t[1], r, aux), t_hi = FP::fold(t[2], t[3], r, aux);
-            const X l_lo = FP::fold(l[0], l[1], r, aux), l_hi = FP::fold(l[2], l[3], r, aux);
-            const X r_lo = FP::fold(g[0], g[1], r, aux), r_hi = FP::fold(g[2], g[3], r, aux);
-            nxt[(1 + 2 * k) * half + 2 * b] = l_lo;
-            nxt[(1 + 2 * k) * half + 2 * b + 1] = l_hi;
-            nxt[(2 + 2 * k) * half + 2 * b] = r_lo;
-            nxt[(2 + 2 * k) * half + 2 * b + 1] = r_hi;
-            const X p0 = FP::fmul(l_lo, r_lo), p1 = FP::fmul(FP::slope(l_lo, l_hi), FP::slope(r_lo, r_hi)),
-                    p2 = FP::fmul(FP::at_m1(l_lo, l_hi), FP::at_m1(r_lo, r_hi));
-            acc[0] = FP::x_add(acc[0], FP::fmul(t_lo, p0));
-            acc[1] = FP::x_add(acc[1], FP::fmul(FP::slope(t_lo, t_hi), p1));
-            acc[2] = FP::x_add(acc[2], FP::fmul(FP::at_m1(t_lo, t_hi), p2));
-        }
-        tail_block_sum<FP, 3>(acc, red, it.part + ((size_t)q * ncta + lb) * 3);  // ends with __syncthreads: nxt is complete
-        X* tmp = cur; cur = nxt; nxt = tmp;
-        len = half;
-    }
-    // len = SEG >> K entries per table go back to memory
-    const size_t n_out = n_in >> it.K;
-    for (int e = threadIdx.x; e < ntab * len; e += blockDim.x) {
-        const int slot = e / len, k = e % len;
-        if (slot == 0 && !(it.write_t0 && grp == 0)) continue;  // t_0 is table 0 = l_0: written by the CTA that owns term 0, or by group 0 when no term 0 here
-        const size_t tab = slot ? (size_t)(2 * i0 + slot - 1) : 0;
-        it.out[tab * n_out + (size_t)seg * len + k] = cur[slot * len + k];
-    }
 }
 
 }  // namespace hg

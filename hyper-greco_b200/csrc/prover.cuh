@@ -427,15 +427,14 @@ struct ScScratch {
     void* partials = nullptr;  // X [max_blocks * max_batch * 4]
     unsigned* counters = nullptr;
     int max_blocks = 0;
-    void* midpart = nullptr;   // X [HG_PROD_MID_K][midpart_segs][4]: CTA partial sums of the mid stage (k_prod_mid); nullptr: no mid stage
+    void* midpart = nullptr;   // X [HG_PROD_MID_K][midpart_segs][4]: CTA partial sums of the mid stage (k_prod_mid_one); nullptr: no mid stage
     size_t midpart_segs = 0;
 };
-// shared memory of k_prod_mid for up to two input tables next to the weights (set once, for the largest user)
+// shared memory of k_prod_mid_one for up to two input tables next to the weights (set once, for the largest user)
 template <class FP> inline size_t prod_mid_smem(int nt) { return ((size_t)(nt + 1) * (HG_PROD_MID_SEG + HG_PROD_MID_SEG / 2) + (size_t)HG_PROD_MID_K * 8 * 3) * sizeof(typename FP::X); }
 template <class FP> inline void prod_mid_set_smem() {
     static bool done = false;  // (per device in a multi-device process: the attribute is per function and device; one device per process here)
     if (!done) {
-        HG_CUDA(cudaFuncSetAttribute(k_prod_mid<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prod_mid_smem<FP>(2)));
         HG_CUDA(cudaFuncSetAttribute(k_prod_mid_one<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prod_mid_smem<FP>(2)));
         done = true;
     }
@@ -566,10 +565,9 @@ void sumcheck_dev(DeviceCtx* ctx, int kclass, Channel<FP>& ch, const WireOptions
     // g = t_0 * t_1 (the collation sumcheck: coefficients {0, 1}) with all challenges known: the last rounds run in one
     // shared-memory launch (k_prod_tail_one), the streamed rounds stop at jt
     const bool tail = product_of_two && ARITY == 1 && nterm == 2 && ch.prefetching() && nv >= 3;
-    // with nv >= 12 the HG_PROD_MID_K rounds before the tail run in ONE launch on 1024-entry segments (k_prod_mid): streamed rounds
+    // with nv >= 12 the HG_PROD_MID_K rounds before the tail run in ONE launch on 1024-entry segments (k_prod_mid_one): streamed rounds
     // [0, js), mid rounds [js, jt), tail rounds [jt, nv)
-    static const bool env_mid = getenv("HG_PROD_MID") ? atoi(getenv("HG_PROD_MID")) != 0 : true;
-    const bool mid = tail && env_mid && nv >= 12 && sc.midpart != nullptr;
+    const bool mid = tail && nv >= 12 && sc.midpart != nullptr;
     const int js = !tail ? nv : (mid ? std::max(2, nv - 2 * HG_PROD_MID_K) : std::max(2, nv - HG_PROD_TAIL_LOG));
     const int jt = !tail ? nv : (mid ? js + HG_PROD_MID_K : js);
     const void* cur_in = d_tables;
@@ -612,7 +610,7 @@ void sumcheck_dev(DeviceCtx* ctx, int kclass, Channel<FP>& ch, const WireOptions
         t.mid_part = nullptr; t.mid_msg = nullptr; t.mid_nseg = 0; t.mid_rounds = 0;
         if (mid) {
             ProdMidItem<FP> mi;
-            mi.n_in = n_in; mi.nt = 1; mi.nseg = (int)(n_in / HG_PROD_MID_SEG); mi.blk_start = 0;
+            mi.n_in = n_in; mi.nt = 1; mi.nseg = (int)(n_in / HG_PROD_MID_SEG);
             if (n_in < 2 * (size_t)HG_PROD_MID_SEG || (size_t)mi.nseg > sc.midpart_segs) throw std::runtime_error("sumcheck_dev: mid stage does not fit its scratch");
             X* obuf = (cur_in == (const void*)bufA) ? bufB : bufA;
             const size_t n_out = n_in >> HG_PROD_MID_K;
@@ -645,7 +643,6 @@ void sumcheck_dev(DeviceCtx* ctx, int kclass, Channel<FP>& ch, const WireOptions
 // one layer sumcheck recorded for batched execution (prefetch mode): everything the device needs is static
 template <class FP> struct GpLayerJob {
     const typename FP::B* tables;  // [nvec][2n]
-    const typename FP::B* parent;  // [nvec][n]: the tree layer above (entries l_i * r_i), read by round 0
     size_t n;
     int nvec, nv;
     size_t gamma_idx, r0_idx, msg_off, evals_off;
@@ -661,7 +658,7 @@ template <class FP>
 void gp_sumcheck_dev(DeviceCtx* ctx, Channel<FP>& ch, const WireOptions& wo, const typename FP::B* d_tables, size_t n, int nvec,
                      const typename FP::X* d_gamma, typename FP::X* d_coeffs, typename FP::X* bufA, typename FP::X* bufB, const ScScratch& sc,
                      std::shared_ptr<ScHostState<FP>> st, size_t* first_chal, size_t* evals_off, bool* scaled,
-                     std::vector<GpLayerJob<FP>>* batch = nullptr, size_t gamma_idx = 0, const typename FP::B* d_parent = nullptr) {
+                     std::vector<GpLayerJob<FP>>* batch = nullptr, size_t gamma_idx = 0) {
     typedef typename FP::B B;
     typedef typename FP::X X;
     constexpr int D = 3;
@@ -671,8 +668,7 @@ void gp_sumcheck_dev(DeviceCtx* ctx, Channel<FP>& ch, const WireOptions& wo, con
     if (batch) {
         // prefetch mode: only the protocol bookkeeping happens here; LassoNodeDev::run_gp_batch launches the work
         GpLayerJob<FP> job;
-        job.tables = d_tables; job.parent = d_parent; job.n = n; job.nvec = nvec; job.nv = nv; job.gamma_idx = gamma_idx;
-        if (!d_parent) throw std::runtime_error("gp_sumcheck_dev: batched mode needs the parent layer");
+        job.tables = d_tables; job.n = n; job.nvec = nvec; job.nv = nv; job.gamma_idx = gamma_idx;
         for (int j = 0; j < nv; j++) {
             size_t off = ch.alloc_msg(j == 0 ? D + 1 : D);
             if (j == 0) job.msg_off = off;
@@ -847,24 +843,22 @@ template <class FP> class LassoNodeDev {
         // prefetch mode runs all layers concurrently: every layer needs its own fold buffers, sum < 3/4 * 4m * (R + M) elements
         d_pool_.alloc(3 * (size_t)m_ * (R_ + M_) + 64);
         d_gp_partials_.alloc((size_t)ctx->sm_count * 64 * 4 + 4096);
-        d_gp_counters_.alloc(128);
+        d_gp_counters_.alloc(64);  // one per layer of a batched round
         // CTA partial sums of the fused round 0 (gp_fused.cuh): <= sm_count*64 + 2m blocks per launch and layer, two layers per tree launch
         d_r0part_.alloc(4 * ((size_t)ctx->sm_count * 64 + 4 * (size_t)m_) * (size_t)(num_vars_ + log2M_ + 2));
         HG_CUDA(cudaMemset(d_gp_counters_.p, 0, d_gp_counters_.bytes()));
         h_desc_.alloc(1 << 16);
         d_desc_.alloc(1 << 16);
         {
-            // grand-product tail kernel: tables of at most 2^tail_log_ entries, every layer split over tail_groups_ CTAs by terms
-            tail_log_ = getenv("HG_GP_TAIL_LOG") ? atoi(getenv("HG_GP_TAIL_LOG")) : FP::GP_TAIL_LOG;
-            tail_groups_ = getenv("HG_GP_TAIL_GROUPS") ? atoi(getenv("HG_GP_TAIL_GROUPS")) : FP::GP_TAIL_GROUPS;
-            if (tail_log_ < 2 || tail_log_ > HG_GP_TAIL_MAXR + 1) throw std::runtime_error("LassoNode: HG_GP_TAIL_LOG out of range");
-            tail_groups_ = std::max(1, std::min(tail_groups_, 2 * m_));
+            // grand-product tail kernel: tables of at most 2^GP_TAIL_LOG entries, every layer split over tail_groups_ CTAs by terms
+            static_assert(FP::GP_TAIL_LOG >= 2 && FP::GP_TAIL_LOG <= HG_GP_TAIL_MAXR + 1, "GP_TAIL_LOG is out of the tail kernel's range");
+            tail_groups_ = std::max(1, std::min((int)FP::GP_TAIL_GROUPS, 2 * m_));
             int smem_max = 0;
             HG_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
             while (gp_tail_smem(tail_groups_) > (size_t)smem_max && tail_groups_ < 2 * m_) tail_groups_++;  // more groups = fewer tables per CTA
             if (gp_tail_smem(tail_groups_) > (size_t)smem_max)
                 throw std::runtime_error("LassoNode: the grand-product tail kernel needs " + std::to_string(gp_tail_smem(tail_groups_)) + " bytes of shared memory, the device offers " +
-                                         std::to_string(smem_max) + " (lower HG_GP_TAIL_LOG)");
+                                         std::to_string(smem_max));
             HG_CUDA(cudaFuncSetAttribute(k_gp_tail<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gp_tail_smem(tail_groups_)));
             d_gp_tailpart_.alloc((size_t)(num_vars_ + log2M_ + 2) * tail_groups_ * (HG_GP_TAIL_MAXR + 1) * 4);
             d_gp_tailcnt_.alloc((size_t)(num_vars_ + log2M_ + 2));
@@ -1074,10 +1068,9 @@ template <class FP> class LassoNodeDev {
         // With every challenge known up front nothing below waits for the claim or the collation sumcheck (gamma, tau are challenges), so
         // they run on the side stream behind the access counters, next to the hash / tree / grand-product kernels, and are joined before
         // the openings (which reuse the eq tables and the partial-sum scratch). Measured: no change of the single-proof latency (5.07 vs
-        // 5.08 ms, profiles/r2_experiments.md) because the three streams already keep the SMs busy; off by default.
-        static const bool env_coll_side = getenv("HG_COLL_SIDE") ? atoi(getenv("HG_COLL_SIDE")) != 0 : false;
-        // (a sharded proof is latency-bound on every rank and rank 0 alone runs these two: there the side stream is always used)
-        const bool coll_side = (env_coll_side || shard_world_ > 1) && lead && mode == kModePrefetch && ctx_->two_streams && !ctx_->profile && ctx_->stream3 != nullptr && ctx_->ev_coll != nullptr;
+        // 5.08 ms, profiles/r2_experiments.md) because the three streams already keep the SMs busy, so a single-device proof keeps them
+        // on the main stream. A sharded proof is latency-bound on every rank and rank 0 alone runs these two: there the side stream is used.
+        const bool coll_side = shard_world_ > 1 && lead && mode == kModePrefetch && ctx_->two_streams && !ctx_->profile && ctx_->stream3 != nullptr && ctx_->ev_coll != nullptr;
         struct CollStream {  // launches go to stream3 while this lives (RAII: an exception must not leave the context there)
             DeviceCtx* c; cudaStream_t main; bool on;
             CollStream(DeviceCtx* ctx, bool enable) : c(ctx), main(ctx->stream), on(enable) {
@@ -1117,57 +1110,46 @@ template <class FP> class LassoNodeDev {
         const bool fused_up = R >= 4;  // hash build fused with the first tree level
         size_t x_idx = 0, y_idx = 0;
         std::vector<GpLayerJob<FP>> jobs;
+        GpPlan plan1, plan2;
+        bool fuse_hash = false;
         if (mode == kModePrefetch) {
             // all challenges are on the device already: do the protocol bookkeeping of both grand products first (message
             // slots, challenge indices), then launch coefficients -> hashes -> trees (+ round 0) -> rounds >= 1
-            GpPlan plan1, plan2;
             grand_product(ch, wo, d_tree1_.p, R, &x_idx, &jobs, fused_up, &plan1);
             grand_product(ch, wo, d_tree2_.p, M, &y_idx, &jobs, false, &plan2);
             prepare_gp_coeffs(ch, wo, jobs);
-            static const bool env_fuse = getenv("HG_GP_FUSE_R0") ? atoi(getenv("HG_GP_FUSE_R0")) != 0 : true;
-            const bool fuse = env_fuse;
-            const bool fuse_hash = fuse && fused_up && gp_needs_r0(R, 0, plan1.nvars);
-            if (fuse_hash) {
-                GpLayerJob<FP>& j0 = jobs[plan1.job_begin + plan1.nvars - 2];  // the sumcheck on layer 0
-                const size_t work = R / 4;                                      // row pairs per memory
-                const int nxb = fused_nxb(work, m);
-                X* part = r0_alloc((size_t)nxb * m);
-                j0.r0part = part; j0.r0n = nxb * m;
-                HG_K(ctx_, KC_HASH, 0, k_hash_t0<FP><<<(unsigned)((R / 4 + HG_BLOCK - 1) / HG_BLOCK), HG_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p,
-                                                                                                                    d_pos_slot_.p, ch.d_chal(gt_idx), R, d_tree1_.p));
-                HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 4 * sizeof(B)),
-                     k_hash_rw_up_r0<FP><<<nxb * m, HG_FUSED_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p, d_pos_slot_.p, ch.d_chal(gt_idx), R, m,
-                                                                          d_tree1_.p, d_tree1_.p + (size_t)2 * m * R, own_range(2 * m), j0.coef, part, nxb));
-            } else if (fused_up) {
-                HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 4 * sizeof(B)),
-                     k_hash_rw_up<FP><<<dim3((unsigned)((R / 4 + HG_BLOCK - 1) / HG_BLOCK + (R < 4 ? 1 : 0)), m), HG_BLOCK, 0, s>>>(
-                         d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p, d_pos_slot_.p, ch.d_chal(gt_idx), R, m, d_tree1_.p,
-                         d_tree1_.p + (size_t)2 * m * R, own_range(2 * m)));
-            } else {
-                HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 3 * sizeof(B)),
-                     k_hash_rw<FP><<<dim3((unsigned)((R + HG_BLOCK - 1) / HG_BLOCK), m), HG_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p,
-                                                                                                           d_pos_slot_.p, ch.d_chal(gt_idx), R, m, d_tree1_.p));
-            }
-            HG_K(ctx_, KC_HASH, (size_t)m * M * (4 + 3 * sizeof(B)),
-                 k_hash_if<FP><<<dim3((unsigned)((M + HG_BLOCK - 1) / HG_BLOCK), m), HG_BLOCK, 0, s>>>(d_subtables_.p, d_final_cts_.p, d_pos_sub_.p, d_pos_slot_.p,
-                                                                                                       ch.d_chal(gt_idx), M, m, d_tree2_.p, own_range(2 * m)));
-            build_trees(ch, plan1, plan2, jobs, fuse);
-            run_gp_batch(ch, wo, jobs);
-        } else {
-        if (fused_up)
+            fuse_hash = fused_up && gp_needs_r0(R, 0, plan1.nvars);
+        }
+        if (fuse_hash) {
+            GpLayerJob<FP>& j0 = jobs[plan1.job_begin + plan1.nvars - 2];  // the sumcheck on layer 0
+            const size_t work = R / 4;                                      // row pairs per memory
+            const int nxb = fused_nxb(work, m);
+            X* part = r0_alloc((size_t)nxb * m);
+            j0.r0part = part; j0.r0n = nxb * m;
+            HG_K(ctx_, KC_HASH, 0, k_hash_t0<FP><<<(unsigned)((R / 4 + HG_BLOCK - 1) / HG_BLOCK), HG_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p,
+                                                                                                                d_pos_slot_.p, ch.d_chal(gt_idx), R, d_tree1_.p));
+            HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 4 * sizeof(B)),
+                 k_hash_rw_up_r0<FP><<<nxb * m, HG_FUSED_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p, d_pos_slot_.p, ch.d_chal(gt_idx), R, m,
+                                                                      d_tree1_.p, d_tree1_.p + (size_t)2 * m * R, own_range(2 * m), j0.coef, part, nxb));
+        } else if (fused_up) {
             HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 4 * sizeof(B)),
                  k_hash_rw_up<FP><<<dim3((unsigned)((R / 4 + HG_BLOCK - 1) / HG_BLOCK + (R < 4 ? 1 : 0)), m), HG_BLOCK, 0, s>>>(
                      d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p, d_pos_slot_.p, ch.d_chal(gt_idx), R, m, d_tree1_.p,
                      d_tree1_.p + (size_t)2 * m * R, own_range(2 * m)));
-        else
+        } else {
             HG_K(ctx_, KC_HASH, (size_t)m * R * (2 + 4 + 3 * sizeof(B)),
                  k_hash_rw<FP><<<dim3((unsigned)((R + HG_BLOCK - 1) / HG_BLOCK), m), HG_BLOCK, 0, s>>>(d_dims_.p, d_read_cts_.p, d_E_.p, d_pos_mem_.p, d_pos_dim_.p,
                                                                                                        d_pos_slot_.p, ch.d_chal(gt_idx), R, m, d_tree1_.p));
+        }
         HG_K(ctx_, KC_HASH, (size_t)m * M * (4 + 3 * sizeof(B)),
              k_hash_if<FP><<<dim3((unsigned)((M + HG_BLOCK - 1) / HG_BLOCK), m), HG_BLOCK, 0, s>>>(d_subtables_.p, d_final_cts_.p, d_pos_sub_.p, d_pos_slot_.p,
                                                                                                    ch.d_chal(gt_idx), M, m, d_tree2_.p, own_range(2 * m)));
-        grand_product(ch, wo, d_tree1_.p, R, &x_idx, nullptr, fused_up);
-        grand_product(ch, wo, d_tree2_.p, M, &y_idx, nullptr, false);
+        if (mode == kModePrefetch) {
+            build_trees(ch, plan1, plan2, jobs);
+            run_gp_batch(ch, wo, jobs);
+        } else {
+            grand_product(ch, wo, d_tree1_.p, R, &x_idx, nullptr, fused_up);
+            grand_product(ch, wo, d_tree2_.p, M, &y_idx, nullptr, false);
         }
         // ---- openings (prover.rs:173-178, mod.rs:80-93)
         const size_t o_dims = ch.alloc_msg(pp_.C), o_rts = ch.alloc_msg(nslots_), o_fcs = ch.alloc_msg(nslots_), o_e = ch.alloc_msg(m);
@@ -1258,21 +1240,21 @@ template <class FP> class LassoNodeDev {
     }
 
     // prove_grand_product (prover.rs:183-266) over nvec = 2m vectors of length N stored at tree (layer 0), upper layers appended
-    // a grand product whose launches were deferred (prefetch mode): what build_tree needs
+    // one grand product's tree and message slots: what build_tree_rest needs, and build_trees when the launches were deferred (prefetch mode)
     struct GpPlan { B* tree = nullptr; size_t N = 0; int nvars = 0; size_t roots_off = 0, ev0_off = 0, job_begin = 0; bool level1_done = false; };
     // does layer k of a tree over vectors of length N get its round 0 from a streaming kernel (tables longer than the tail kernel takes)?
-    bool gp_needs_r0(size_t N, int k, int nvars) const { return k <= nvars - 2 && ((N >> k) / 2) > ((size_t)1 << tail_log_); }
-    // shared memory of k_gp_tail when a layer's 2m terms are split over `groups` CTAs: (1 + 2 tpg) tables of 2^tail_log_ entries + half as many folded
+    bool gp_needs_r0(size_t N, int k, int nvars) const { return k <= nvars - 2 && ((N >> k) / 2) > ((size_t)1 << FP::GP_TAIL_LOG); }
+    // shared memory of k_gp_tail when a layer's 2m terms are split over `groups` CTAs: (1 + 2 tpg) tables of 2^GP_TAIL_LOG entries + half as many folded
     size_t gp_tail_smem(int groups) const {
         const int tpg = (2 * m_ + groups - 1) / groups;
-        return ((size_t)(1 + 2 * tpg) * (((size_t)1 << tail_log_) + ((size_t)1 << tail_log_) / 2) + 32 * 4) * sizeof(X);
+        return ((size_t)(1 + 2 * tpg) * (((size_t)1 << FP::GP_TAIL_LOG) + ((size_t)1 << FP::GP_TAIL_LOG) / 2) + 32 * 4) * sizeof(X);
     }
     // position blocks per vector of the fused builders: every CTA ends with a block-level reduction that costs about as much as
     // one pass over its data, so CTAs are long (~16 per SM over the whole launch, at least 8 positions per thread)
     int fused_nxb(size_t work, int nvec) const {
-        static const int env_cps = getenv("HG_FUSED_CPS") ? atoi(getenv("HG_FUSED_CPS")) : 16;
+        constexpr int ctas_per_sm = 16;
         const size_t by_work = (work + (size_t)HG_FUSED_BLOCK * 8 - 1) / ((size_t)HG_FUSED_BLOCK * 8);
-        const size_t by_grid = std::max<size_t>(1, (size_t)ctx_->sm_count * env_cps / nvec);
+        const size_t by_grid = std::max<size_t>(1, (size_t)ctx_->sm_count * ctas_per_sm / nvec);
         return (int)std::max<size_t>(1, std::min(by_work, by_grid));
     }
     X* r0_alloc(size_t nblk) {
@@ -1282,12 +1264,10 @@ template <class FP> class LassoNodeDev {
         r0_used_ += need;
         return p;
     }
-    // product tree of one grand product (prover.rs:191-195, Layer::up :332-354); with `fuse` the builders also sample round 0 of
-    // every layer that is streamed (gp_fused.cuh) and the layer jobs get the partial-sum regions
     // one fused builder step of a tree (k_tree_up_r0): its arguments, whether it builds two levels, its grid and algorithmic bytes
     struct TreeStep { TreeR0Args<FP> a; bool two; unsigned nblk; size_t bytes; };
     // the fused steps of one tree (layers whose round 0 is streamed); *cur_out = last complete layer afterwards
-    std::vector<TreeStep> plan_tree_fused(const GpPlan& pl, std::vector<GpLayerJob<FP>>& jobs, bool fuse, int* cur_out) {
+    std::vector<TreeStep> plan_tree_fused(const GpPlan& pl, std::vector<GpLayerJob<FP>>& jobs, int* cur_out) {
         const int nvec = 2 * m_, nvars = pl.nvars;
         const size_t N = pl.N;
         std::vector<B*> layer(nvars);
@@ -1296,7 +1276,7 @@ template <class FP> class LassoNodeDev {
         auto job_of = [&](int k) -> GpLayerJob<FP>& { return jobs[pl.job_begin + (size_t)(nvars - 2 - k)]; };  // sumcheck nv = nvars-1-k is job nv-1
         int cur = pl.level1_done ? 1 : 0;  // last layer that is complete
         std::vector<TreeStep> steps;
-        while (fuse && cur < nvars - 1 && gp_needs_r0(N, cur, nvars)) {
+        while (cur < nvars - 1 && gp_needs_r0(N, cur, nvars)) {
             const bool two = cur + 2 <= nvars - 1 && gp_needs_r0(N, cur + 1, nvars);
             const size_t len = N >> cur, q = two ? len / 4 : len / 2;
             TreeStep st;
@@ -1330,15 +1310,14 @@ template <class FP> class LassoNodeDev {
         else k_tree_up_r0<FP, false><<<grid, HG_FUSED_BLOCK, 0, s>>>(x.a, y ? y->a : x.a, x.nblk);
         HG_LAUNCH_CHECK();
     }
-    // both product trees of the node (prover.rs:191-195, Layer::up :332-354). With `fuse` the builders also sample round 0 of every
-    // layer that is streamed (gp_fused.cuh) and the layer jobs get the partial-sum regions; step k of both trees shares a launch.
-    void build_trees(Channel<FP>& ch, const GpPlan& pl1, const GpPlan& pl2, std::vector<GpLayerJob<FP>>& jobs, bool fuse) {
-        static const bool env_pair = getenv("HG_TREE_PAIR") ? atoi(getenv("HG_TREE_PAIR")) != 0 : true;
+    // both product trees of the node (prover.rs:191-195, Layer::up :332-354). The builders also sample round 0 of every layer that
+    // is streamed (gp_fused.cuh) and the layer jobs get the partial-sum regions; step k of both trees shares a launch.
+    void build_trees(Channel<FP>& ch, const GpPlan& pl1, const GpPlan& pl2, std::vector<GpLayerJob<FP>>& jobs) {
         int cur1 = 0, cur2 = 0;
-        const std::vector<TreeStep> s1 = plan_tree_fused(pl1, jobs, fuse, &cur1), s2 = plan_tree_fused(pl2, jobs, fuse, &cur2);
+        const std::vector<TreeStep> s1 = plan_tree_fused(pl1, jobs, &cur1), s2 = plan_tree_fused(pl2, jobs, &cur2);
         size_t k2 = 0;
         for (size_t k1 = 0; k1 < s1.size(); k1++) {
-            const TreeStep* mate = (env_pair && k2 < s2.size() && s2[k2].two == s1[k1].two) ? &s2[k2] : nullptr;
+            const TreeStep* mate = (k2 < s2.size() && s2[k2].two == s1[k1].two) ? &s2[k2] : nullptr;
             launch_tree_step(s1[k1], mate);
             if (mate) k2++;
         }
@@ -1377,7 +1356,6 @@ template <class FP> class LassoNodeDev {
 
     void grand_product(Channel<FP>& ch, const WireOptions& wo, B* tree, size_t N, size_t* point_idx, std::vector<GpLayerJob<FP>>* batch,
                        bool level1_done, GpPlan* defer = nullptr) {
-        cudaStream_t s = ctx_->stream;
         const int nvec = 2 * m_;
         int nvars = 0;
         while (((size_t)1 << nvars) < N) nvars++;
@@ -1385,28 +1363,12 @@ template <class FP> class LassoNodeDev {
         std::vector<B*> layer(nvars);
         layer[0] = tree;
         for (int k = 1; k < nvars; k++) layer[k] = layer[k - 1] + (size_t)nvec * (N >> (k - 1));
-        if (defer) { defer->tree = tree; defer->N = N; defer->nvars = nvars; defer->level1_done = level1_done; defer->job_begin = batch ? batch->size() : 0; }
-        for (int k = (level1_done ? 2 : 1); k < nvars && !defer;) {
-            const size_t len_prev = N >> (k - 1);  // vector length of the layer this step reads
-            if (len_prev <= (size_t)HG_TREE_TAIL && len_prev > 2) {  // the rest of the tree in one launch (shared memory)
-                HG_K(ctx_, KC_TREE, (size_t)nvec * len_prev * 2 * sizeof(B),
-                     k_tree_tail<FP><<<nvec, 256, len_prev * sizeof(B), s>>>(layer[k - 1], nvec, (int)len_prev, own_range(nvec)));
-                break;
-            }
-            if (k + 1 < nvars) {  // two levels per launch: layer k is written and never re-read by the build
-                const size_t q = N >> (k + 1);
-                HG_K(ctx_, KC_TREE, (size_t)nvec * q * 7 * sizeof(B),
-                     k_tree_up2<FP><<<dim3((unsigned)(((q >= 2 ? q / 2 : q) + HG_BLOCK - 1) / HG_BLOCK), nvec), HG_BLOCK, 0, s>>>(layer[k - 1], layer[k], layer[k + 1], q, own_range(nvec)));
-                k += 2;
-            } else {
-                const size_t h = N >> k;
-                HG_K(ctx_, KC_TREE, (size_t)nvec * h * 3 * sizeof(B), k_tree_up<FP><<<dim3((unsigned)((h + HG_BLOCK - 1) / HG_BLOCK), nvec), HG_BLOCK, 0, s>>>(layer[k - 1], layer[k], h, own_range(nvec)));
-                k += 1;
-            }
-        }
         const size_t roots_off = ch.alloc_msg(nvec), ev0_off = ch.alloc_msg(2 * nvec);
-        if (defer) { defer->roots_off = roots_off; defer->ev0_off = ev0_off; }
-        else HG_K(ctx_, KC_TREE, (size_t)nvec * 2 * sizeof(B), k_tree_top<FP><<<(nvec + HG_BLOCK - 1) / HG_BLOCK, HG_BLOCK, 0, s>>>(layer[nvars - 1], own_begin(nvec), own_end(nvec), ch.d_msg(roots_off), ch.d_msg(ev0_off)));
+        GpPlan pl;
+        pl.tree = tree; pl.N = N; pl.nvars = nvars; pl.level1_done = level1_done; pl.job_begin = batch ? batch->size() : 0;
+        pl.roots_off = roots_off; pl.ev0_off = ev0_off;
+        if (defer) *defer = pl;
+        else build_tree_rest(ch, pl, level1_done ? 1 : 0);
         struct GpHost { std::vector<X> claimed; std::vector<X> evals; size_t mu_idx = 0; bool pending = false; };
         auto gp = std::make_shared<GpHost>();
         Channel<FP>* chp = &ch;
@@ -1440,8 +1402,7 @@ template <class FP> class LassoNodeDev {
             size_t sc_first = 0, ev_off = 0;
             bool scaled = false;
             const B* tables = layer[nvars - 1 - nv];
-            gp_sumcheck_dev<FP>(ctx_, ch, wo, tables, (size_t)1 << nv, nvec, ch.d_chal(gamma_idx), d_gp_coeffs_.p, d_bufA_.p, d_bufB_.p, sc_, st, &sc_first, &ev_off, &scaled, batch, gamma_idx,
-                                layer[nvars - nv]);
+            gp_sumcheck_dev<FP>(ctx_, ch, wo, tables, (size_t)1 << nv, nvec, ch.d_chal(gamma_idx), d_gp_coeffs_.p, d_bufA_.p, d_bufB_.p, sc_, st, &sc_first, &ev_off, &scaled, batch, gamma_idx);
             ch.emit([chp, gp, ev_off, nvec, scaled, gamma_idx, asc]() {
                 auto& t = chp->transcript();
                 // the device keeps l_i (i > 0) and r_0 pre-multiplied by c_i (gp_kernels.cuh); undo it exactly with c_i^{-1}
@@ -1493,63 +1454,49 @@ template <class FP> class LassoNodeDev {
         const int nl = (int)jobs.size();
         if (!nl) return;
         (void)wo;
+        constexpr size_t tail_n = (size_t)1 << FP::GP_TAIL_LOG;
         // carve per-layer regions out of the pools
         std::vector<X*> bufA(nl, nullptr), bufB(nl, nullptr), coef(nl, nullptr);
         size_t pool_off = 0;
         for (int k = 0; k < nl; k++) {
             const auto& j = jobs[k];
             coef[k] = j.coef;
-            if (j.n > ((size_t)1 << tail_log_)) {
+            if (j.n > tail_n) {
                 size_t a = 2 * (size_t)j.nvec * (j.n / 2), b = 2 * (size_t)j.nvec * (j.n / 4);
                 bufA[k] = d_pool_.p + pool_off; pool_off += a;
                 bufB[k] = d_pool_.p + pool_off; pool_off += b;
             }
         }
         if (pool_off > d_pool_.n) throw std::runtime_error("run_gp_batch: pool too small");
-        // Rounds of layer k: streamed launches r = 1..S_k (r = 0 only without the fused tree builders), then up to HG_GP_MID_STAGES mid
-        // stages of <= 5 rounds each in shared-memory segments (k_gp_mid) once the tables are at most 2^HG_GP_MID_LOG long, then the tail
-        // kernel from 2^GP_TAIL_LOG entries on. Round 1 is always streamed: it scales the tables by c_i.
-        static const int env_mid_log = getenv("HG_GP_MID_LOG") ? atoi(getenv("HG_GP_MID_LOG")) : FP::GP_MID_LOG;
-        static const int env_mid_tpg = getenv("HG_GP_MID_TPG") ? std::max(1, atoi(getenv("HG_GP_MID_TPG"))) : 7;
+        // Rounds of layer k: round 0 sampled by the fused tree builders, streamed launches r = 1..S_k, then the tail kernel from
+        // 2^GP_TAIL_LOG entries on. Round 1 is always streamed: it scales the tables by c_i. S_k = 0: the whole layer runs in the tail.
         std::vector<int> S(nl, 0);
-        std::vector<std::vector<int>> midK(nl);
-        int maxJ = -1;
+        int maxJ = 0;
         for (int k = 0; k < nl; k++) {
             const auto& j = jobs[k];
-            if (j.n <= ((size_t)1 << tail_log_)) continue;
-            const int J = j.nv - tail_log_;  // rounds before the tail
-            S[k] = J;
-            if (env_mid_log > tail_log_ && J >= 2) {
-                S[k] = std::max(1, j.nv - env_mid_log);
-                int left = J - S[k];
-                if (left > HG_GP_MID_STAGES * HG_GP_MID_MAXK) { S[k] += left - HG_GP_MID_STAGES * HG_GP_MID_MAXK; left = HG_GP_MID_STAGES * HG_GP_MID_MAXK; }
-                while (left > 0) { const int K = std::min(left, HG_GP_MID_MAXK); midK[k].push_back(K); left -= K; }
-            }
+            if (j.n <= tail_n) continue;
+            if (j.r0n == 0) throw std::runtime_error("run_gp_batch: a streamed layer has no round 0 from the tree builders");
+            S[k] = j.nv - FP::GP_TAIL_LOG;
             maxJ = std::max(maxJ, S[k]);
         }
-        std::vector<std::vector<GpItem<FP>>> rounds(maxJ + 1);
-        std::vector<GpItem<FP>> round0a;  // first half of round 0 (k_gp_r0a_multi): own geometry, partials and counters
-        size_t round0a_bytes = 0, part0a_off = 0;
-        int blk0a = 0;
+        std::vector<std::vector<GpItem<FP>>> rounds(maxJ + 1);  // indexed by round; rounds[0] stays empty
         std::vector<size_t> round_bytes(maxJ + 1, 0);
         size_t part_need = 0;
-        // grid shape of the streaming launches: at most gp_max_bx blocks along a table, term groups added until an item has
-        // about gp_target blocks (tunable for experiments through HG_GP_MAXBX / HG_GP_TARGET, in units of the SM count)
-        static const int env_maxbx = getenv("HG_GP_MAXBX") ? atoi(getenv("HG_GP_MAXBX")) : 4;
+        // grid shape of the streaming launches: at most max_bx_per_sm blocks per SM along a table, term groups added until an item
+        // has about FP::GP_TARGET blocks (in units of the SM count)
+        constexpr int max_bx_per_sm = 4;
         // measured optimum: one term group (every thread loops over all terms of its pairs and reuses t_0) as soon as a table gives
         // ~37 CTAs; smaller layers get term groups so that no layer runs on fewer CTAs than that
-        static const double env_target = getenv("HG_GP_TARGET") ? atof(getenv("HG_GP_TARGET")) : FP::GP_TARGET;
-        const int target_blocks = std::max(1, (int)(ctx_->sm_count * env_target * (HG_BLOCK / FP::GP_BLOCK)));
-        const size_t gp_max_bx = (size_t)ctx_->sm_count * env_maxbx * (HG_BLOCK / FP::GP_BLOCK);
-        // Work-balanced shape (HG_GP_BALANCE, default on for fields with GP_BALANCE): a round finishes with its slowest CTA, and a
-        // CTA's time is (terms it loops over) x (positions per thread). With one term group per large layer the late rounds ran
-        // ~1000 CTAs of which the largest layer's looped over all 2m terms while the SMs were half empty (profiles/r2_launch_list.md:
-        // round 5 93 us for 0.3 GB). Here every item gets term groups of about total thread-terms / resident threads, so that the
-        // whole round is one wave of equal CTAs, and the items are placed in the grid heaviest CTA first.
-        static const int env_balance = getenv("HG_GP_BALANCE") ? atoi(getenv("HG_GP_BALANCE")) : FP::GP_BALANCE;
-        static const int env_min_tpg = getenv("HG_GP_MIN_TPG") ? std::max(1, atoi(getenv("HG_GP_MIN_TPG"))) : 4;
+        const int target_blocks = std::max(1, (int)(ctx_->sm_count * FP::GP_TARGET * (HG_BLOCK / FP::GP_BLOCK)));
+        const size_t gp_max_bx = (size_t)ctx_->sm_count * max_bx_per_sm * (HG_BLOCK / FP::GP_BLOCK);
+        // Work-balanced shape (fields with FP::GP_BALANCE): a round finishes with its slowest CTA, and a CTA's time is (terms it
+        // loops over) x (positions per thread). With one term group per large layer the late rounds ran ~1000 CTAs of which the
+        // largest layer's looped over all 2m terms while the SMs were half empty (profiles/r2_launch_list.md: round 5 93 us for
+        // 0.3 GB). Here every item gets term groups of about total thread-terms / resident threads, so that the whole round is one
+        // wave of equal CTAs, and the items are placed in the grid heaviest CTA first.
+        constexpr int min_tpg = 4;
         const size_t resident_threads = (size_t)ctx_->sm_count * FP::GP_MIN_BLOCKS * HG_BLOCK;
-        for (int r = 0; r <= maxJ; r++) {
+        for (int r = 1; r <= maxJ; r++) {
             int blk = 0;
             size_t part_off = 0;
             // layers that take part in this round, their thread count along the table, and the round's total thread-terms
@@ -1558,45 +1505,32 @@ template <class FP> class LassoNodeDev {
             size_t total_tt = 0;
             for (int k = 0; k < nl; k++) {
                 const auto& j = jobs[k];
-                if (j.n <= ((size_t)1 << tail_log_) || r > S[k]) continue;
-                if (r == 0 && j.r0n > 0) continue;  // sampled by the fused tree builders
-                tx[k] = r == 0 ? (j.n / 2 + FP::GP_R0_U - 1) / FP::GP_R0_U : (j.n >> (r - 1)) / 4;
+                if (r > S[k]) continue;
+                tx[k] = (j.n >> (r - 1)) / 4;
                 total_tt += std::min(tx[k], gp_max_bx * FP::GP_BLOCK) * (size_t)(own_end(j.nvec) - own_begin(j.nvec));
                 order.push_back(k);
             }
-            const size_t tpg_bal = std::max<size_t>((size_t)env_min_tpg, (total_tt + resident_threads - 1) / resident_threads);
-            if (env_balance && r >= 1)  // heaviest CTAs first: longer table (more positions per thread, the same term count) first
+            const size_t tpg_bal = std::max<size_t>((size_t)min_tpg, (total_tt + resident_threads - 1) / resident_threads);
+            if (FP::GP_BALANCE)  // heaviest CTAs first: longer table (more positions per thread, the same term count) first
                 std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return tx[a] > tx[b]; });
             for (int k : order) {
                 const auto& j = jobs[k];
                 GpItem<FP> it;
-                const int ntab = 2 * j.nvec;
                 it.nvec = j.nvec;
-                it.parent = j.parent;
                 it.i_begin = own_begin(j.nvec); it.i_end = own_end(j.nvec); it.write_t0 = it.i_begin > 0;
                 const int nown = it.i_end - it.i_begin;
                 it.c = coef[k]; it.cr = coef[k] + j.nvec;
-                size_t threads_x;
-                if (r == 0) {
-                    it.in = j.tables; it.out = nullptr; it.n_in = j.n; it.r_prev = nullptr;
-                    it.msg = ch.d_msg(j.msg_off);
-                    threads_x = (j.n / 2 + FP::GP_R0_U - 1) / FP::GP_R0_U;
-                    round_bytes[r] += (size_t)(2 * nown + it.write_t0) * j.n * sizeof(B);
-                } else {
-                    it.n_in = j.n >> (r - 1);
-                    it.in = (r == 1) ? (const void*)j.tables : (const void*)(((r - 1) & 1) ? bufA[k] : bufB[k]);
-                    it.out = (r & 1) ? bufA[k] : bufB[k];
-                    it.r_prev = ch.d_chal(j.r0_idx + r - 1);
-                    it.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)(r - 1));
-                    threads_x = it.n_in / 4;
-                    round_bytes[r] += (size_t)(2 * nown + it.write_t0) * (it.n_in * (r == 1 ? sizeof(B) : sizeof(X)) + (it.n_in / 2) * sizeof(X));
-                    (void)ntab;
-                }
-                size_t b = (threads_x + FP::GP_BLOCK - 1) / FP::GP_BLOCK;
+                it.n_in = j.n >> (r - 1);
+                it.in = (r == 1) ? (const void*)j.tables : (const void*)(((r - 1) & 1) ? bufA[k] : bufB[k]);
+                it.out = (r & 1) ? bufA[k] : bufB[k];
+                it.r_prev = ch.d_chal(j.r0_idx + r - 1);
+                it.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)(r - 1));
+                round_bytes[r] += (size_t)(2 * nown + it.write_t0) * (it.n_in * (r == 1 ? sizeof(B) : sizeof(X)) + (it.n_in / 2) * sizeof(X));
+                size_t b = (tx[k] + FP::GP_BLOCK - 1) / FP::GP_BLOCK;
                 if (b < 1) b = 1;
                 if (b > gp_max_bx) b = gp_max_bx;
                 int g = (int)std::min<size_t>((size_t)nown, std::max<size_t>(1, ((size_t)target_blocks + b - 1) / b));
-                if (env_balance && r >= 1 && tpg_bal * 5 < (size_t)nown * 4)  // (a split that saves less than a fifth of the loop is not worth re-folding t_0)
+                if (FP::GP_BALANCE && tpg_bal * 5 < (size_t)nown * 4)  // (a split that saves less than a fifth of the loop is not worth re-folding t_0)
                     g = std::max(g, (int)std::max<size_t>(1, (size_t)nown / tpg_bal));  // rounded down: rather one wave of slightly longer CTAs than a second wave
                 it.tpg = (nown + g - 1) / g;
                 it.groups = (nown + it.tpg - 1) / it.tpg;
@@ -1608,44 +1542,17 @@ template <class FP> class LassoNodeDev {
                 part_off += (size_t)it.nblk * 4;
                 it.counter = d_gp_counters_.p + rounds[r].size();
                 rounds[r].push_back(it);
-                if (r == 0) {  // the parent-layer half: 4 pairs per thread, term groups until the item has ~target blocks
-                    GpItem<FP> a = it;
-                    size_t ba = (j.n / 4 + FP::GP_R0A_QPT * FP::GP_BLOCK - 1) / (FP::GP_R0A_QPT * FP::GP_BLOCK);  // GP_R0A_QPT quads of parent entries per thread and term
-                    if (ba < 1) ba = 1;
-                    if (ba > gp_max_bx) ba = gp_max_bx;
-                    int ga = (int)std::min<size_t>((size_t)nown, std::max<size_t>(1, ((size_t)target_blocks + ba - 1) / ba));
-                    a.tpg = (nown + ga - 1) / ga;
-                    a.groups = (nown + a.tpg - 1) / a.tpg;
-                    a.bx = (int)ba;
-                    a.nblk = a.bx * a.groups;
-                    a.blk_start = blk0a;
-                    blk0a += a.nblk;
-                    a.partials = nullptr;  // assigned below, behind the partials of the largest round
-                    part0a_off += (size_t)a.nblk * 2;
-                    a.counter = d_gp_counters_.p + 64 + round0a.size();
-                    round0a_bytes += (size_t)nown * j.n * sizeof(B);  // actual traffic of the parent-layer half (not algorithmic)
-                    round0a.push_back(a);
-                }
             }
             part_need = std::max(part_need, part_off);
-            if (rounds[r].size() > 64) throw std::runtime_error("run_gp_batch: too many layers");
+            if (rounds[r].size() > d_gp_counters_.n) throw std::runtime_error("run_gp_batch: too many layers");
         }
-        if (part_need + part0a_off > d_gp_partials_.n) { d_gp_partials_.alloc((part_need + part0a_off) * 2); /* re-point */
+        if (part_need > d_gp_partials_.n) { d_gp_partials_.alloc(part_need * 2); /* re-point */
             for (auto& rv : rounds) { size_t off = 0; for (auto& it : rv) { it.partials = d_gp_partials_.p + off; off += (size_t)it.nblk * 4; } } }
-        (void)round0a_bytes;
-        { size_t off = part_need; for (auto& a : round0a) { a.partials = d_gp_partials_.p + off; off += (size_t)a.nblk * 2; } }
-        if (round0a.size() + 64 > d_gp_counters_.n) throw std::runtime_error("run_gp_batch: too many layers");
         std::vector<GpTailItem<FP>> titems(nl);
         size_t tail_bytes = 0;
-        std::vector<GpMidItem<FP>> mitems[HG_GP_MID_STAGES];
-        std::vector<int> mitem_layer[HG_GP_MID_STAGES];
-        std::vector<std::array<size_t, HG_GP_MID_STAGES>> mid_part_off(nl);
-        int mid_blk[HG_GP_MID_STAGES] = {0, 0, 0}, mid_tpg_max = 1;
-        size_t mid_bytes[HG_GP_MID_STAGES] = {0, 0, 0}, mid_part_need = 0;
         for (int k = 0; k < nl; k++) {
             const auto& j = jobs[k];
             GpTailItem<FP>& t = titems[k];
-            for (int st = 0; st < HG_GP_MID_STAGES; st++) { t.mid_part[st] = nullptr; t.mid_msg[st] = nullptr; t.mid_n[st] = 0; t.mid_K[st] = 0; }
             {
                 const int nown = own_end(j.nvec) - own_begin(j.nvec);
                 t.tpg = std::max(1, (j.nvec + tail_groups_ - 1) / tail_groups_);  // sized for all 2m terms: the shared-memory budget was checked for that
@@ -1657,53 +1564,19 @@ template <class FP> class LassoNodeDev {
             t.c = coef[k]; t.nvec = j.nvec; t.evals = ch.d_msg(j.evals_off);
             t.i_begin = own_begin(j.nvec); t.i_end = own_end(j.nvec);
             t.r0part = j.r0part; t.r0n = j.r0n;
-            if (j.n <= ((size_t)1 << tail_log_)) {
+            if (j.n <= tail_n) {
                 t.from_base = 1; t.in = j.tables; t.n = (int)j.n; t.rounds = j.nv - 1;
                 t.chal = ch.d_chal(j.r0_idx); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4);
                 tail_bytes += 2 * (size_t)j.nvec * j.n * sizeof(B);
-            } else {
-                const int J = j.nv - tail_log_;
-                // mid stages: in = what the last streamed round (or the previous stage) wrote, out = the other buffer of the layer
-                const X* cur = (S[k] & 1) ? bufA[k] : bufB[k];
-                int rnd = S[k];  // rounds done so far
-                const int nown = t.i_end - t.i_begin;
-                for (size_t st = 0; st < midK[k].size(); st++) {
-                    GpMidItem<FP> mi;
-                    mi.in = cur; mi.out = (cur == bufA[k]) ? bufB[k] : bufA[k];
-                    mi.n_in = j.n >> rnd; mi.K = midK[k][st];
-                    mi.chal = ch.d_chal(j.r0_idx + rnd);
-                    mi.nvec = j.nvec; mi.nseg = (int)(mi.n_in / HG_GP_MID_SEG);
-                    mi.tpg = std::min(nown, env_mid_tpg); mi.groups = (nown + mi.tpg - 1) / mi.tpg;
-                    mi.i_begin = t.i_begin; mi.i_end = t.i_end; mi.write_t0 = t.i_begin > 0;
-                    const int ncta = mi.nseg * mi.groups;
-                    mi.blk_start = mid_blk[st]; mid_blk[st] += ncta;
-                    mi.part = nullptr;  // assigned below
-                    mid_part_off[k][st] = mid_part_need; mid_part_need += (size_t)mi.K * ncta * 3;
-                    t.mid_n[st] = ncta; t.mid_K[st] = mi.K; t.mid_msg[st] = ch.d_msg(j.msg_off + 4 + 3 * (size_t)rnd);
-                    mid_bytes[st] += (size_t)(2 * nown + mi.write_t0) * (mi.n_in + (mi.n_in >> mi.K)) * sizeof(X);
-                    mid_tpg_max = std::max(mid_tpg_max, mi.tpg);
-                    mitems[st].push_back(mi);
-                    mitem_layer[st].push_back(k);
-                    cur = mi.out; rnd += mi.K;
-                }
-                if (rnd != J) throw std::runtime_error("run_gp_batch: round plan does not reach the tail");
-                t.from_base = 0; t.in = cur; t.n = 1 << tail_log_; t.rounds = tail_log_ - 1;
-                t.chal = ch.d_chal(j.r0_idx + J); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)J);
-                tail_bytes += 2 * (size_t)j.nvec * ((size_t)1 << tail_log_) * sizeof(X);
+            } else {  // the tables the last streamed round wrote
+                t.from_base = 0; t.in = (S[k] & 1) ? bufA[k] : bufB[k]; t.n = (int)tail_n; t.rounds = FP::GP_TAIL_LOG - 1;
+                t.chal = ch.d_chal(j.r0_idx + S[k]); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)S[k]);
+                tail_bytes += 2 * (size_t)j.nvec * tail_n * sizeof(X);
             }
         }
-        if (mid_part_need > d_gp_midpart_.n) { HG_CUDA(cudaStreamSynchronize(s)); d_gp_midpart_.alloc(mid_part_need * 2); }
-        for (int st = 0; st < HG_GP_MID_STAGES; st++)
-            for (size_t q = 0; q < mitems[st].size(); q++) {
-                const int k = mitem_layer[st][q];
-                mitems[st][q].part = d_gp_midpart_.p + mid_part_off[k][st];
-                titems[k].mid_part[st] = mitems[st][q].part;
-            }
         // upload descriptors
-        size_t bytes = titems.size() * sizeof(GpTailItem<FP>);
+        size_t bytes = titems.size() * sizeof(GpTailItem<FP>) + 16;
         for (auto& rv : rounds) bytes += rv.size() * sizeof(GpItem<FP>) + 16;
-        for (auto& mv : mitems) bytes += mv.size() * sizeof(GpMidItem<FP>) + 16;
-        bytes += round0a.size() * sizeof(GpItem<FP>) + 64;
         if (h_desc_.n < bytes) { h_desc_.alloc(bytes * 2); d_desc_.alloc(bytes * 2); }
         unsigned char* hp = h_desc_.p;
         size_t off = 0;
@@ -1711,37 +1584,16 @@ template <class FP> class LassoNodeDev {
         std::vector<size_t> r_off(rounds.size());
         for (size_t r = 0; r < rounds.size(); r++) r_off[r] = put(rounds[r].data(), rounds[r].size() * sizeof(GpItem<FP>));
         size_t t_off = put(titems.data(), titems.size() * sizeof(GpTailItem<FP>));
-        size_t a_off = put(round0a.data(), round0a.size() * sizeof(GpItem<FP>));
-        size_t m_off[HG_GP_MID_STAGES];
-        for (int st = 0; st < HG_GP_MID_STAGES; st++) m_off[st] = put(mitems[st].data(), mitems[st].size() * sizeof(GpMidItem<FP>));
         if (off > h_desc_.n) throw std::runtime_error("run_gp_batch: descriptor staging overflow");
         HG_CUDA(cudaMemcpyAsync(d_desc_.p, h_desc_.p, off, cudaMemcpyHostToDevice, s));
         // launches
-        for (size_t r = 0; r < rounds.size(); r++) {
-            if (rounds[r].empty()) continue;
+        for (size_t r = 1; r < rounds.size(); r++) {
             const auto& last = rounds[r].back();
             const int grid = last.blk_start + last.nblk, ni = (int)rounds[r].size();
             const GpItem<FP>* di = (const GpItem<FP>*)(d_desc_.p + r_off[r]);
-            if (r == 0 && !round0a.empty()) {
-                KernelScope ka(ctx_, KC_SC_GP, 0);  // reads the parent layer: no algorithmic bytes of its own (SURVEY.md 8d counts round 0 once)
-                k_gp_r0a_multi<FP><<<blk0a, FP::GP_BLOCK, 0, s>>>((const GpItem<FP>*)(d_desc_.p + a_off), (int)round0a.size());
-                HG_LAUNCH_CHECK();
-            }
             KernelScope ks(ctx_, KC_SC_GP, round_bytes[r]);
-            if (r == 0) k_gp_r0_multi<FP, FP::GP_R0_U><<<grid, FP::GP_BLOCK, 0, s>>>(di, ni);
-            else if (r == 1) k_gp_fold_multi<FP, B, true><<<grid, FP::GP_BLOCK, 0, s>>>(di, ni);
+            if (r == 1) k_gp_fold_multi<FP, B, true><<<grid, FP::GP_BLOCK, 0, s>>>(di, ni);
             else k_gp_fold_multi<FP, X, false><<<grid, FP::GP_BLOCK, 0, s>>>(di, ni);
-            HG_LAUNCH_CHECK();
-        }
-        for (int st = 0; st < HG_GP_MID_STAGES; st++) {
-            if (mitems[st].empty()) continue;
-            const size_t smem = gp_mid_smem<FP>(mid_tpg_max);
-            if (smem > gp_mid_smem_set_) {
-                HG_CUDA(cudaFuncSetAttribute(k_gp_mid<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                gp_mid_smem_set_ = smem;
-            }
-            KernelScope ks(ctx_, KC_SC_GP, mid_bytes[st]);
-            k_gp_mid<FP><<<mid_blk[st], HG_GP_MID_THREADS, smem, s>>>((const GpMidItem<FP>*)(d_desc_.p + m_off[st]), (int)mitems[st].size());
             HG_LAUNCH_CHECK();
         }
         {
@@ -1799,10 +1651,9 @@ template <class FP> class LassoNodeDev {
     DevBuf<X> d_eq_, d_gp_coeffs_, d_bufA_, d_bufB_, d_partials_, d_coll_terms_;
     int coll_coeff_state_ = 0;  // 0 not uploaded, 1 ascending, 2 descending
     DevBuf<unsigned> d_counters_, d_gp_counters_;
-    DevBuf<X> d_pool_, d_gp_partials_, d_r0part_, d_midpart_, d_gp_midpart_, d_gp_tailpart_;
+    DevBuf<X> d_pool_, d_gp_partials_, d_r0part_, d_midpart_, d_gp_tailpart_;
     DevBuf<unsigned> d_gp_tailcnt_;
-    int tail_log_ = FP::GP_TAIL_LOG, tail_groups_ = 1;
-    size_t gp_mid_smem_set_ = 48 * 1024;  // largest dynamic shared memory k_gp_mid has been allowed so far
+    int tail_groups_ = 1;
     size_t r0_used_ = 0;
     DevBuf<unsigned char> d_desc_, d_cdesc_;
     PinnedBuf<unsigned char> h_desc_, h_cdesc_;

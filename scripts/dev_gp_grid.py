@@ -1,4 +1,4 @@
-"""Lasso-node proof time (device-resident input) for the current HG_GP_* environment."""
+"""Lasso-node proof time (device-resident input) and the hash / tree / grand-product class times."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -24,5 +24,4 @@ for _ in range(3):
     tr = api.Keccak256Transcript(); node.prove_claim_reduction(buf, tr, 0, n_inputs=inp.size)
 prof = ctx.profile_read(); ctx.profile(False)
 gp = prof["sumcheck_grand_product"]
-tag = " ".join(f"{k}={v}" for k, v in os.environ.items() if k.startswith("HG_"))
-print(f"[{tag}] {dt*1e3:.3f} ms/proof, hash {prof['hash_build'][1]/3:.3f} tree {prof['product_tree'][1]/3:.3f} GP {gp[1]/3:.3f} ms, sha={hashlib.sha256(proof).hexdigest()[:12]}")
+print(f"{dt*1e3:.3f} ms/proof, hash {prof['hash_build'][1]/3:.3f} tree {prof['product_tree'][1]/3:.3f} GP {gp[1]/3:.3f} ms, sha={hashlib.sha256(proof).hexdigest()[:12]}")

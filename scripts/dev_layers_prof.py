@@ -1,4 +1,4 @@
-"""Per-class kernel time of the full GKR proof for the current environment (single stream, profiling mode)."""
+"""Per-class kernel time of the full GKR proof (single stream, profiling mode)."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -31,5 +31,4 @@ dt = (time.perf_counter() - t0) / 20
 ctx.profile(True)
 for _ in range(3): step()
 prof = ctx.profile_read(); ctx.profile(False)
-tag = " ".join(f"{k}={v}" for k, v in os.environ.items() if k.startswith("HG_"))
-print(f"[{tag}] {dt*1e3:.3f} ms/proof sha={hashlib.sha256(pr).hexdigest()[:10]} " + " ".join(f"{k}={v[1]/3:.3f}" for k, v in sorted(prof.items(), key=lambda kv: -kv[1][1])[:12]))
+print(f"{dt*1e3:.3f} ms/proof sha={hashlib.sha256(pr).hexdigest()[:10]} " + " ".join(f"{k}={v[1]/3:.3f}" for k, v in sorted(prof.items(), key=lambda kv: -kv[1][1])[:12]))

@@ -14,10 +14,10 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CLASSES = [
-    ("sumcheck_grand_product", r"k_gp_r0a_multi|k_gp_r0_multi|k_gp_fold_multi|k_gp_tail|k_gp_mid"),
+    ("sumcheck_grand_product", r"k_gp_fold_multi|k_gp_tail"),
     ("misc", r"k_gp_coeffs_multi"),
     ("sumcheck_collation", r"k_coll_round|k_prod_tail_one|k_sc_round|k_fold_final|k_prod_mid_one"),
-    ("gkr_layer_sumcheck", r"k_prod_round_multi|k_prod_tail|k_prod_mid|k_copy_items|k_fold_items"),
+    ("gkr_layer_sumcheck", r"k_prod_round_multi|k_prod_tail|k_copy_items|k_fold_items"),
     ("gkr_layer_weights", r"k_eq_split_multi|k_eq_accumulate|k_wiring_gather|k_wiring_runs|k_concat_items|k_ext_split|k_ext_merge|k_dot_wconst"),
     ("counters", r"k_cnt_"),
     ("hash_build", r"k_hash_"),

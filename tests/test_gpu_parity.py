@@ -1094,56 +1094,3 @@ def test_plugin_lookup_types_on_the_device(api, ctx, golden_dir):
         api.lasso_node_verify(pp2, nv2, api.Keccak256Transcript(api.GOLDILOCKS, bytes(bad)))
     node2.free()
 
-
-_SWITCH_SCRIPT = r"""
-import hashlib, os, sys
-import numpy as np
-sys.path.insert(0, sys.argv[1])
-import hyper_greco_b200  # noqa
-from hyper_greco_b200 import api, params, witness
-gd = os.path.join(sys.argv[1], "tests", "golden")
-name = "4096_2x55_65537"
-P = params.PARAMS[name]
-ctx = api.Context(0)
-inp = np.load(os.path.join(gd, f"lasso_inputs_{name}.npz"))["inputs"]
-node = api.LassoNode(ctx, api.LassoPreprocessing.preprocess(witness.lasso_lookup_bounds(P)), witness.lasso_num_vars(P), witness.lasso_lookup_segments(P))
-tr = api.Keccak256Transcript(api.GOLDILOCKS)
-node.prove_claim_reduction(inp, tr)
-h1 = hashlib.sha256(tr.into_proof()).hexdigest()
-io = np.load(os.path.join(gd, f"circuit_io_{name}.npz"))
-flat = [io["s"], io["e"], io["k1"]] + list(io["ais"]) + list(io["r1is"]) + [io["r2is"]]
-prover = api.BfvSkEncryptProver(ctx, P)
-proof, _ = prover.prove_host([np.ascontiguousarray(v).reshape(-1) for v in flat], np.ascontiguousarray(io["ct0is"]).reshape(-1))
-print("HASHES", h1, hashlib.sha256(proof).hexdigest())
-"""
-
-
-@pytest.mark.timeout(600)
-def test_launch_shape_switches_do_not_change_a_byte():
-    """The launch-shape switches of DESIGN.md section 5 (term-group balance, tail groups / length, mid stages, fused round 0 of the
-    grand product and of the node sumchecks, run-compressed wiring and forward evaluation, early flush, side streams) select other
-    kernels or grids for the same arithmetic: Lasso-node and whole-proof bytes on the reference's n=4096 witness must not move.
-    The switches are read once per process, so every setting runs in its own interpreter."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    settings = [
-        {},
-        {"HG_GP_BALANCE": "0", "HG_GP_TAIL_GROUPS": "1", "HG_GP_TAIL_LOG": "6"},
-        {"HG_GP_TAIL_GROUPS": "13", "HG_GP_TAIL_LOG": "9", "HG_GP_MIN_TPG": "2"},
-        {"HG_GP_MID_LOG": "11", "HG_GP_MID_TPG": "4"},
-        {"HG_GP_FUSE_R0": "0", "HG_PROD_FUSE0": "0"},
-        {"HG_WIRE_RUNS": "0", "HG_FWD_RUNS": "0", "HG_EARLY_FLUSH": "0"},
-        {"HG_COLL_SIDE": "1", "HG_PROD_MID": "0", "HG_PROD_MID_LAYERS": "1"},
-    ]
-    seen = []
-    for extra in settings:
-        env = dict(os.environ)
-        env.update(extra)
-        r = subprocess.run([sys.executable, "-c", _SWITCH_SCRIPT, root], env=env, capture_output=True, text=True, timeout=300)
-        assert r.returncode == 0, (extra, r.stderr[-2000:])
-        line = [l for l in r.stdout.splitlines() if l.startswith("HASHES")]
-        assert line, (extra, r.stdout[-500:])
-        seen.append((extra, line[-1]))
-    assert all(h == seen[0][1] for _, h in seen), seen
