@@ -89,6 +89,27 @@ template <class FP> struct FieldState {
     PinnedBuf<X> mle_hpt;
 };
 
+// cudaFuncAttributeMaxDynamicSharedMemorySize belongs to a kernel and a device, so every context in the process shares it. It is
+// set here, at context creation, for every kernel that takes dynamic shared memory: to the device's whole opt-in budget less the
+// kernel's static shared memory. Every call writes the same values, so no object can lower a limit another object relies on, and
+// contexts may be created concurrently. The launch sites size their shared memory against the same device budget.
+template <class FP> void set_dynamic_smem_limits(int device) {
+    int optin = 0;
+    HG_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+    auto set = [optin](const void* kernel) {
+        cudaFuncAttributes a;
+        HG_CUDA(cudaFuncGetAttributes(&a, kernel));
+        HG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)a.sharedSizeBytes));
+    };
+    set((const void*)k_ntt_cols<FP>);
+    set((const void*)k_ntt_rows<FP>);
+    set((const void*)k_prod_tail<FP>);
+    set((const void*)k_prod_tail_one<FP>);
+    set((const void*)k_prod_mid_one<FP>);
+    set((const void*)k_gp_tail<FP>);
+    set((const void*)k_tree_tail<FP>);
+}
+
 struct hg_ctx {
     DeviceCtx dev;
     int field_id;
@@ -398,6 +419,8 @@ int hg_ctx_create(int device, int field_id, hg_ctx** out) {
         HG_CUDA(cudaGetDeviceCount(&n));
         if (device < 0 || device >= n) throw std::runtime_error("no such CUDA device");
         HG_CUDA(cudaSetDevice(device));
+        set_dynamic_smem_limits<GlField>(device);
+        set_dynamic_smem_limits<FrField>(device);
         struct CtxDeleter { void operator()(hg_ctx* p) const { hg_ctx_destroy(p); } };  // a failing call below must not leak the streams / events made before it
         std::unique_ptr<hg_ctx, CtxDeleter> c(new hg_ctx());
         with_field(field_id, [&](auto fp) { c->state.template emplace<FieldState<decltype(fp)>>(); });

@@ -1004,7 +1004,6 @@ template <class FP> class GkrCircuitDev {
             items.push_back(t);
         }
         if (items.empty()) return;
-        if (smem > tail_smem_) { HG_CUDA(cudaFuncSetAttribute(k_prod_tail<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); tail_smem_ = smem; }
         HG_K(ctx_, KC_GKR_SC, bytes, k_prod_tail<FP><<<(unsigned)items.size(), 256, smem, s>>>(stage(items)));
     }
 
@@ -1048,7 +1047,6 @@ template <class FP> class GkrCircuitDev {
     std::vector<std::unique_ptr<Node>> nodes_;
     std::vector<int> topo_;
     bool evaluated_ = false, planned_ = false, eval_planned_ = false, use_tail_ = false;
-    size_t tail_smem_ = 0;
     std::vector<EvalLevel> eval_levels_;
     size_t total_chal_ = 0, desc_off_ = 0, eq_off_ = 0;
     std::unique_ptr<Channel<FP>> ch_;

@@ -31,8 +31,6 @@ template <class FP> class NttEngine {
         // data tile + the n/2 twiddles of the in-tile transform
         const size_t smem_c = ((size_t)n1 * (tile_c | 1) + n1 / 2 + 1) * sizeof(B), smem_r = ((size_t)n2 * (tile_r | 1) + n2 / 2 + 1) * sizeof(B);
         if (smem_c > 200 * 1024 || smem_r > 200 * 1024) throw std::runtime_error("hg_ntt: transform too large for the shared-memory tiles");
-        HG_CUDA(cudaFuncSetAttribute(k_ntt_cols<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c));
-        HG_CUDA(cudaFuncSetAttribute(k_ntt_rows<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
         HG_K(ctx_, KC_NTT, 2 * N * batch * sizeof(B),
              k_ntt_cols<FP><<<dim3(n2 / tile_c, (unsigned)batch), HG_NTT_THREADS, smem_c, s>>>(d_data, scratch_.p, log_n1, log_n2, tile_c, tw->p));
         const B scale = inverse ? FP::b_inv(FP::b_from_u64(N)) : FP::b_one();

@@ -430,15 +430,8 @@ struct ScScratch {
     void* midpart = nullptr;   // X [HG_PROD_MID_K][midpart_segs][4]: CTA partial sums of the mid stage (k_prod_mid_one); nullptr: no mid stage
     size_t midpart_segs = 0;
 };
-// shared memory of k_prod_mid_one for up to two input tables next to the weights (set once, for the largest user)
+// shared memory of k_prod_mid_one for nt input tables next to the weights
 template <class FP> inline size_t prod_mid_smem(int nt) { return ((size_t)(nt + 1) * (HG_PROD_MID_SEG + HG_PROD_MID_SEG / 2) + (size_t)HG_PROD_MID_K * 8 * 3) * sizeof(typename FP::X); }
-template <class FP> inline void prod_mid_set_smem() {
-    static bool done = false;  // (per device in a multi-device process: the attribute is per function and device; one device per process here)
-    if (!done) {
-        HG_CUDA(cudaFuncSetAttribute(k_prod_mid_one<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prod_mid_smem<FP>(2)));
-        done = true;
-    }
-}
 
 // serialisation of one round message + claim bookkeeping (runs on the host when the message has been downloaded).
 // The device sends samples of the TRUE round polynomial h: h(0), h(inf), [h(-1)], and h(1) in round 0. With the running
@@ -616,7 +609,6 @@ void sumcheck_dev(DeviceCtx* ctx, int kclass, Channel<FP>& ch, const WireOptions
             const size_t n_out = n_in >> HG_PROD_MID_K;
             mi.w_in = (const X*)cur_in; mi.tab_in = (const X*)cur_in + n_in; mi.w_out = obuf; mi.tab_out = obuf + n_out;
             mi.chal = ch.d_chal(mid_chal); mi.part = (X*)sc.midpart; mi.capture = nullptr; mi.cap_round = -1; mi.arity = 1;
-            prod_mid_set_smem<FP>();
             {
                 KernelScope ks(ctx, kclass, 2 * n_in * sizeof(X));
                 k_prod_mid_one<FP><<<mi.nseg, 256, prod_mid_smem<FP>(1), ctx->stream>>>(mi);
@@ -853,13 +845,13 @@ template <class FP> class LassoNodeDev {
             // grand-product tail kernel: tables of at most 2^GP_TAIL_LOG entries, every layer split over tail_groups_ CTAs by terms
             static_assert(FP::GP_TAIL_LOG >= 2 && FP::GP_TAIL_LOG <= HG_GP_TAIL_MAXR + 1, "GP_TAIL_LOG is out of the tail kernel's range");
             tail_groups_ = std::max(1, std::min((int)FP::GP_TAIL_GROUPS, 2 * m_));
-            int smem_max = 0;
-            HG_CUDA(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+            cudaFuncAttributes fa;  // the device's opt-in budget less the kernel's static shared memory (set_dynamic_smem_limits, abi.cu)
+            HG_CUDA(cudaFuncGetAttributes(&fa, (const void*)k_gp_tail<FP>));
+            const int smem_max = fa.maxDynamicSharedSizeBytes;
             while (gp_tail_smem(tail_groups_) > (size_t)smem_max && tail_groups_ < 2 * m_) tail_groups_++;  // more groups = fewer tables per CTA
             if (gp_tail_smem(tail_groups_) > (size_t)smem_max)
                 throw std::runtime_error("LassoNode: the grand-product tail kernel needs " + std::to_string(gp_tail_smem(tail_groups_)) + " bytes of shared memory, the device offers " +
                                          std::to_string(smem_max));
-            HG_CUDA(cudaFuncSetAttribute(k_gp_tail<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gp_tail_smem(tail_groups_)));
             d_gp_tailpart_.alloc((size_t)(num_vars_ + log2M_ + 2) * tail_groups_ * (HG_GP_TAIL_MAXR + 1) * 4);
             d_gp_tailcnt_.alloc((size_t)(num_vars_ + log2M_ + 2));
             HG_CUDA(cudaMemset(d_gp_tailcnt_.p, 0, d_gp_tailcnt_.bytes()));
@@ -895,12 +887,9 @@ template <class FP> class LassoNodeDev {
             }
             HG_CUDA(cudaMemcpy(d_wpow_.p, wp.data(), wp.size() * sizeof(B), cudaMemcpyHostToDevice));
         }
-        HG_CUDA(cudaFuncSetAttribute(k_tree_tail<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(HG_TREE_TAIL * sizeof(B))));
         // the uploads above are blocking cudaMemcpy calls from pageable memory (legacy stream); the proof kernels run on non-blocking
         // streams that do not wait for it, so make everything land now
         HG_CUDA(cudaDeviceSynchronize());
-        HG_CUDA(cudaFuncSetAttribute(k_prod_tail_one<FP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)(((size_t)2 * 3 * ((size_t)1 << HG_PROD_TAIL_LOG) + 96) * sizeof(X))));
     }
 
     size_t device_bytes() const {

@@ -11,7 +11,11 @@
  *                    extension element = degree(field) base elements in `as_bases()` order.
  *   return value     0 = ok, non-zero = error; hg_last_error() returns the message (thread-local). No C++ exception
  *                    and no sticky CUDA error crosses this boundary.
- *   threading        one hg_ctx = one device + one stream, driven by one host thread at a time.
+ *   threading        one hg_ctx = one device + one stream, driven by one host thread at a time. Distinct contexts may be
+ *                    driven concurrently from different threads, objects of any shapes may be alive together, and one
+ *                    process may hold contexts on several devices. The per-kernel dynamic shared-memory limits are
+ *                    shared by the whole process; hg_ctx_create sets them for its device to the device's maximum, the
+ *                    same value on every call, so no object can lower a limit another one needs.
  *   ownership        handles are created/destroyed only through this API; the library never frees caller memory and
  *                    never keeps a host pointer after a call returns.
  */
