@@ -38,6 +38,9 @@ __device__ __forceinline__ void load4(const gl2* p, gl2 (&v)[4]) {
 __device__ __forceinline__ void load2(const u64* p, u64 (&v)[2]) { ldg128(p, v[0], v[1]); }
 __device__ __forceinline__ void load2(const gl2* p, gl2 (&v)[2]) { ldg256(p, v[0].c0, v[0].c1, v[1].c0, v[1].c1); }
 __device__ __forceinline__ void store2(gl2* p, gl2 a, gl2 b) { stg256(p, a.c0, a.c1, b.c0, b.c1); }
+__device__ __forceinline__ void store1(gl2* p, gl2 a) {
+    asm volatile("st.global.L1::no_allocate.v2.u64 [%0], {%1,%2};" ::"l"(p), "l"(a.c0), "l"(a.c1) : "memory");
+}
 // BN254: one element = one 256-bit access
 __device__ __forceinline__ void load4(const fr* p, fr (&v)[4]) {
 #pragma unroll
@@ -51,6 +54,7 @@ __device__ __forceinline__ void store2(fr* p, fr a, fr b) {
     stg256(p, a.l[0], a.l[1], a.l[2], a.l[3]);
     stg256(p + 1, b.l[0], b.l[1], b.l[2], b.l[3]);
 }
+__device__ __forceinline__ void store1(fr* p, fr a) { stg256(p, a.l[0], a.l[1], a.l[2], a.l[3]); }
 // pull the bytes a later iteration will load into L2 (costs no registers; the loop is otherwise latency-bound, profiles/)
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
 
@@ -204,11 +208,12 @@ constexpr int HG_GP_TAIL_MAXR = 10;  // most rounds the tail kernel runs (tables
 
 template <class FP> struct GpItem {
     const void* in;                  // tables read this round (base in round 1, extension later): [2*nvec][n_in]
-    typename FP::X* out;             // folded tables written this round: [2*nvec][n_in/2]
+    typename FP::X* out;             // tables written this round (see k_gp_fold_multi)
     unsigned long long n_in;
     const typename FP::X* c;         // c_i
     const typename FP::X* cr;        // c_i * r_0 (round 1)
-    const typename FP::X* r_prev;    // challenge folded in this round
+    const typename FP::X* r_prev;    // challenge of the previous round, folded on read (round 1)
+    const typename FP::X* r_cur;     // challenge of this round, folded on write
     typename FP::X* msg;
     typename FP::X* partials;
     unsigned* counter;
@@ -288,41 +293,61 @@ template <class ITEM> __device__ __forceinline__ int find_item(const ITEM* items
 }
 template <class FP> __device__ __forceinline__ int gp_find_item(const GpItem<FP>* items, int nitems) { return find_item(items, nitems); }
 
+// Round r (>= 1) of a layer sumcheck samples h_r on the pairs (2b, 2b+1) of the level-r tables L_r and writes every pair folded
+// by its own challenge r_cur, i.e. L_{r+1}: all challenges are on the device before the launch, so the next round reads half as
+// much and folds nothing on read.
+//   SCALE (round 1, TIN = B): reads quads of the base tables L_0 and folds them by r_prev = r_0 into the pairs of L_1, scaling
+//     them as it goes; l_i (i > 0) is written as c_i * l_i and r_0 as c_0 * r_0 (l_0 stays: it is also t_0).
+//   otherwise (TIN = X): reads the pairs of L_r as the previous round wrote them.
+//   in: [2*nvec][n_in] (n_in = |L_0| or |L_r|);  out: [2*nvec][n_in / 4 or n_in / 2] (|L_{r+1}|)
 template <class FP, class TIN, bool SCALE>
 __global__ void __launch_bounds__(FP::GP_BLOCK, FP::GP_FOLD_CTAS) k_gp_fold_multi(const GpItem<FP>* __restrict__ items, int nitems) {
     typedef typename FP::X X;
-    constexpr int NP = 3;
+    constexpr bool QUAD = SCALE;
+    constexpr int NP = 3, W = QUAD ? 4 : 2;  // W: entries of a table read per position
     const GpItem<FP> it = items[gp_find_item<FP>(items, nitems)];
     const unsigned lb = blockIdx.x - it.blk_start;
     const unsigned bxi = lb % it.bx, grp = lb / it.bx;
     const TIN* in = (const TIN*)it.in;
     X* out = it.out;
-    const size_t n_in = it.n_in, npairs = n_in / 4, n_out = n_in / 2;
+    const size_t n_in = it.n_in, npairs = n_in / W, n_out = npairs;
     const int i0 = it.i_begin + grp * it.tpg, i1 = min(it.i_end, i0 + it.tpg);
-    const X r = *it.r_prev;
-    const typename FP::FoldAux aux = FP::fold_aux(r);
+    X r = FP::x_zero();
+    if constexpr (QUAD) r = *it.r_prev;
+    const X rc = *it.r_cur;
+    const typename FP::FoldAux aux = FP::fold_aux(r), auxc = FP::fold_aux(rc);
+    // one pair of L_r: folded from its quad of L_{r-1}, or as read
+    auto pair = [&](const TIN (&a)[W], X& lo, X& hi) {
+        if constexpr (QUAD) { lo = FP::fold(a[0], a[1], r, aux); hi = FP::fold(a[2], a[3], r, aux); }
+        else { lo = a[0]; hi = a[1]; }
+    };
+    auto load = [&](const TIN* p, TIN (&a)[W]) {
+        if constexpr (QUAD) load4(p, a); else load2(p, a);
+    };
+    auto store = [&](X* tab, size_t b, X lo, X hi) { store1(tab + b, FP::fold(lo, hi, rc, auxc)); };
     X acc[NP];
 #pragma unroll
     for (int p = 0; p < NP; p++) acc[p] = FP::x_zero();
     for (size_t b = (size_t)bxi * blockDim.x + threadIdx.x; b < npairs; b += (size_t)it.bx * blockDim.x) {
         X t0[NP];
         {
-            TIN a[4];
-            load4(in + 4 * b, a);
-            X lo = FP::fold(a[0], a[1], r, aux), hi = FP::fold(a[2], a[3], r, aux);
+            TIN a[W];
+            load(in + W * b, a);
+            X lo, hi;
+            pair(a, lo, hi);
             t0[0] = lo; t0[1] = FP::slope(lo, hi); t0[2] = FP::at_m1(lo, hi);
-            if (it.write_t0 && grp == 0) store2(out + 2 * b, lo, hi);
+            if (it.write_t0 && grp == 0) store(out, b, lo, hi);
         }
         typename FP::XAcc P[NP];
 #pragma unroll
         for (int p = 0; p < NP; p++) P[p] = FP::xacc_zero_();
         for (int i = i0; i < i1; i++) {
-            TIN a[4], c[4];
-            load4(in + (size_t)(2 * i) * n_in + 4 * b, a);
-            load4(in + (size_t)(2 * i + 1) * n_in + 4 * b, c);
+            TIN a[W], c[W];
+            load(in + (size_t)(2 * i) * n_in + W * b, a);
+            load(in + (size_t)(2 * i + 1) * n_in + W * b, c);
             if (i + HG_GP_PREFETCH < i1) {
-                prefetch_l2(in + (size_t)(2 * (i + HG_GP_PREFETCH)) * n_in + 4 * b);
-                prefetch_l2(in + (size_t)(2 * (i + HG_GP_PREFETCH) + 1) * n_in + 4 * b);
+                prefetch_l2(in + (size_t)(2 * (i + HG_GP_PREFETCH)) * n_in + W * b);
+                prefetch_l2(in + (size_t)(2 * (i + HG_GP_PREFETCH) + 1) * n_in + W * b);
             }
             X l_lo, l_hi, r_lo, r_hi;
             if constexpr (SCALE) {
@@ -330,17 +355,17 @@ __global__ void __launch_bounds__(FP::GP_BLOCK, FP::GP_FOLD_CTAS) k_gp_fold_mult
                 const X ci = it.c[i], cri = it.cr[i];
                 if (i > 0) {
                     l_lo = FP::fold_scaled(a[0], a[1], ci, cri); l_hi = FP::fold_scaled(a[2], a[3], ci, cri);
-                    r_lo = FP::fold(c[0], c[1], r, aux); r_hi = FP::fold(c[2], c[3], r, aux);
+                    pair(c, r_lo, r_hi);
                 } else {
-                    l_lo = FP::fold(a[0], a[1], r, aux); l_hi = FP::fold(a[2], a[3], r, aux);
+                    pair(a, l_lo, l_hi);
                     r_lo = FP::fold_scaled(c[0], c[1], ci, cri); r_hi = FP::fold_scaled(c[2], c[3], ci, cri);
                 }
             } else {
-                l_lo = FP::fold(a[0], a[1], r, aux); l_hi = FP::fold(a[2], a[3], r, aux);
-                r_lo = FP::fold(c[0], c[1], r, aux); r_hi = FP::fold(c[2], c[3], r, aux);
+                pair(a, l_lo, l_hi);
+                pair(c, r_lo, r_hi);
             }
-            store2(out + (size_t)(2 * i) * n_out + 2 * b, l_lo, l_hi);
-            store2(out + (size_t)(2 * i + 1) * n_out + 2 * b, r_lo, r_hi);
+            store(out + (size_t)(2 * i) * n_out, b, l_lo, l_hi);
+            store(out + (size_t)(2 * i + 1) * n_out, b, r_lo, r_hi);
             // q_i(X) = l_i(X) r_i(X) is quadratic: sampled at X = 0, 1, inf (no value at -1 inside the term loop)
             FP::xacc_mad_(P[0], l_lo, r_lo);
             FP::xacc_mad_(P[1], FP::slope(l_lo, l_hi), FP::slope(r_lo, r_hi));
@@ -381,9 +406,9 @@ template <class FP> __global__ void k_gp_coeffs_multi(const GpCoeffItem<FP>* __r
 template <class FP> struct GpTailItem {
     const void* in;                 // from_base: base tables [nvec][2n]; else extension tables [2*nvec][n] (already scaled)
     const typename FP::X* c;
-    const typename FP::X* chal;     // chal[k] = challenge folded in the k-th tail round; chal[rounds] = last challenge (final fold)
+    const typename FP::X* chal;     // chal[k] = challenge folded in the k-th folding tail round; chal[rounds] = last challenge (final fold)
     typename FP::X* msg0;           // from_base: 4 slots for round 0
-    typename FP::X* msg;            // 3 slots per tail round
+    typename FP::X* msg;            // 3 slots per sampled tail round (!from_base: `rounds` + 1 of them, see k_gp_tail)
     typename FP::X* evals;          // 2*nvec final evaluations (l_i for i > 0 scaled by c_i, r_0 by c_0)
     int from_base, n, nvec, rounds;
     int i_begin, i_end;             // owned terms (see GpItem)
@@ -437,7 +462,7 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
     X* A = reinterpret_cast<X*>(smem_raw);        // [cap][n]
     X* Bf = A + (size_t)cap * len;                 // [cap][n / 2]
     X* red = Bf + (size_t)cap * (len / 2);         // [32][4]
-    X* gpart = it.gpart + (size_t)g * (HG_GP_TAIL_MAXR + 1) * 4;  // [1 + rounds][4]: slot 0 = round 0 (from_base), slot 1 + rd = tail round rd
+    X* gpart = it.gpart + (size_t)g * (HG_GP_TAIL_MAXR + 1) * 4;  // slot 0 = round 0 (from_base), slot 1 + k = k-th sampled tail round
     if (it.from_base) {
         const B* base = (const B*)it.in;  // vector i = [l_i (n) | r_i (n)] -> tables 2i, 2i+1 are consecutive runs of n
         for (int e = threadIdx.x; e < ntab * len; e += blockDim.x) {
@@ -485,6 +510,23 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
     }
     X* cur = A;
     X* nxt = Bf;
+    const int pre = it.from_base ? 0 : 1;
+    if (pre) {  // the last streamed round wrote its tables folded by its own challenge: sample the first tail round on them as they are
+        const int npairs = len / 2;
+        X acc[3] = {FP::x_zero(), FP::x_zero(), FP::x_zero()};
+        for (int e = threadIdx.x; e < nt * npairs; e += blockDim.x) {
+            const int k = e / npairs, b = e % npairs;
+            const X* t = cur + 2 * b;
+            const X* l = cur + (1 + 2 * k) * len + 2 * b;
+            const X* q = cur + (2 + 2 * k) * len + 2 * b;
+            const X p0 = FP::fmul(l[0], q[0]), p1 = FP::fmul(FP::slope(l[0], l[1]), FP::slope(q[0], q[1])),
+                    p2 = FP::fmul(FP::at_m1(l[0], l[1]), FP::at_m1(q[0], q[1]));
+            acc[0] = FP::x_add(acc[0], FP::fmul(t[0], p0));
+            acc[1] = FP::x_add(acc[1], FP::fmul(FP::slope(t[0], t[1]), p1));
+            acc[2] = FP::x_add(acc[2], FP::fmul(FP::at_m1(t[0], t[1]), p2));
+        }
+        tail_block_sum<FP, 3>(acc, red, gpart + 4);
+    }
     for (int rd = 0; rd < it.rounds; rd++) {
         const X r = it.chal[rd];
         const typename FP::FoldAux aux = FP::fold_aux(r);
@@ -513,7 +555,7 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
             acc[1] = FP::x_add(acc[1], FP::fmul(FP::slope(t_lo, t_hi), p1));
             acc[2] = FP::x_add(acc[2], FP::fmul(FP::at_m1(t_lo, t_hi), p2));
         }
-        tail_block_sum<FP, 3>(acc, red, gpart + (size_t)(1 + rd) * 4);  // ends with __syncthreads: nxt is complete
+        tail_block_sum<FP, 3>(acc, red, gpart + (size_t)(1 + pre + rd) * 4);  // ends with __syncthreads: nxt is complete
         X* tmp = cur; cur = nxt; nxt = tmp;
         len = half;
     }
@@ -532,7 +574,7 @@ template <class FP> __global__ void __launch_bounds__(HG_TAIL_THREADS) k_gp_tail
     __syncthreads();
     if (!is_last) return;
     __threadfence();
-    for (int e = threadIdx.x; e < (1 + it.rounds) * 4; e += blockDim.x) {
+    for (int e = threadIdx.x; e < (1 + pre + it.rounds) * 4; e += blockDim.x) {
         const int slot = e / 4, p = e % 4;
         if (slot == 0 ? !it.from_base : p == 3) continue;
         X v = FP::x_zero();

@@ -832,8 +832,9 @@ template <class FP> class LassoNodeDev {
         size_t nmax = std::max(R_, M_) / 2;  // longest sumcheck table
         d_bufA_.alloc(std::max<size_t>(4 * (size_t)m_ * (nmax / 2), 4 * (size_t)m_));
         d_bufB_.alloc(std::max<size_t>(4 * (size_t)m_ * (nmax / 4), 4 * (size_t)m_));
-        // prefetch mode runs all layers concurrently: every layer needs its own fold buffers, sum < 3/4 * 4m * (R + M) elements
-        d_pool_.alloc(3 * (size_t)m_ * (R_ + M_) + 64);
+        // prefetch mode runs all layers concurrently: every layer needs its own fold buffers (L_2 and L_3 of its tables),
+        // sum < 3/8 * 4m * (R + M) elements
+        d_pool_.alloc(3 * (size_t)m_ * (R_ + M_) / 2 + 64);
         d_gp_partials_.alloc((size_t)ctx->sm_count * 64 * 4 + 4096);
         d_gp_counters_.alloc(64);  // one per layer of a batched round
         // CTA partial sums of the fused round 0 (gp_fused.cuh): <= sm_count*64 + 2m blocks per launch and layer, two layers per tree launch
@@ -1444,14 +1445,17 @@ template <class FP> class LassoNodeDev {
         if (!nl) return;
         (void)wo;
         constexpr size_t tail_n = (size_t)1 << FP::GP_TAIL_LOG;
-        // carve per-layer regions out of the pools
+        // Round r of a streamed layer samples h_r on the level-r tables L_r (|L_r| = n >> r). All challenges are on the device, so
+        // every round writes its tables folded by its own challenge, L_{r+1}, and the next round reads those pairs: round 1 reads
+        // the base tables L_0 (folding by r_0 on read, scaling by c_i) and writes L_2, round r >= 2 reads L_r and writes L_{r+1}.
+        // carve per-layer regions out of the pools: odd rounds write bufA, even rounds bufB
         std::vector<X*> bufA(nl, nullptr), bufB(nl, nullptr), coef(nl, nullptr);
         size_t pool_off = 0;
         for (int k = 0; k < nl; k++) {
             const auto& j = jobs[k];
             coef[k] = j.coef;
             if (j.n > tail_n) {
-                size_t a = 2 * (size_t)j.nvec * (j.n / 2), b = 2 * (size_t)j.nvec * (j.n / 4);
+                size_t a = 2 * (size_t)j.nvec * (j.n / 4), b = 2 * (size_t)j.nvec * (j.n / 8);
                 bufA[k] = d_pool_.p + pool_off; pool_off += a;
                 bufB[k] = d_pool_.p + pool_off; pool_off += b;
             }
@@ -1495,7 +1499,7 @@ template <class FP> class LassoNodeDev {
             for (int k = 0; k < nl; k++) {
                 const auto& j = jobs[k];
                 if (r > S[k]) continue;
-                tx[k] = (j.n >> (r - 1)) / 4;
+                tx[k] = j.n >> (r + 1);  // pairs of L_r
                 total_tt += std::min(tx[k], gp_max_bx * FP::GP_BLOCK) * (size_t)(own_end(j.nvec) - own_begin(j.nvec));
                 order.push_back(k);
             }
@@ -1509,12 +1513,13 @@ template <class FP> class LassoNodeDev {
                 it.i_begin = own_begin(j.nvec); it.i_end = own_end(j.nvec); it.write_t0 = it.i_begin > 0;
                 const int nown = it.i_end - it.i_begin;
                 it.c = coef[k]; it.cr = coef[k] + j.nvec;
-                it.n_in = j.n >> (r - 1);
+                it.n_in = j.n >> (r == 1 ? 0 : r);
                 it.in = (r == 1) ? (const void*)j.tables : (const void*)(((r - 1) & 1) ? bufA[k] : bufB[k]);
                 it.out = (r & 1) ? bufA[k] : bufB[k];
                 it.r_prev = ch.d_chal(j.r0_idx + r - 1);
+                it.r_cur = ch.d_chal(j.r0_idx + r);
                 it.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)(r - 1));
-                round_bytes[r] += (size_t)(2 * nown + it.write_t0) * (it.n_in * (r == 1 ? sizeof(B) : sizeof(X)) + (it.n_in / 2) * sizeof(X));
+                round_bytes[r] += (size_t)(2 * nown + it.write_t0) * (it.n_in * (r == 1 ? sizeof(B) : sizeof(X)) + (j.n >> (r + 1)) * sizeof(X));
                 size_t b = (tx[k] + FP::GP_BLOCK - 1) / FP::GP_BLOCK;
                 if (b < 1) b = 1;
                 if (b > gp_max_bx) b = gp_max_bx;
@@ -1557,10 +1562,10 @@ template <class FP> class LassoNodeDev {
                 t.from_base = 1; t.in = j.tables; t.n = (int)j.n; t.rounds = j.nv - 1;
                 t.chal = ch.d_chal(j.r0_idx); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4);
                 tail_bytes += 2 * (size_t)j.nvec * j.n * sizeof(B);
-            } else {  // the tables the last streamed round wrote
-                t.from_base = 0; t.in = (S[k] & 1) ? bufA[k] : bufB[k]; t.n = (int)tail_n; t.rounds = FP::GP_TAIL_LOG - 1;
-                t.chal = ch.d_chal(j.r0_idx + S[k]); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)S[k]);
-                tail_bytes += 2 * (size_t)j.nvec * tail_n * sizeof(X);
+            } else {  // the tables the last streamed round wrote, L_{S+1}: the tail samples round S+1 on them, then folds by r_{S+1}, ...
+                t.from_base = 0; t.in = (S[k] & 1) ? bufA[k] : bufB[k]; t.n = (int)(tail_n / 2); t.rounds = FP::GP_TAIL_LOG - 2;
+                t.chal = ch.d_chal(j.r0_idx + S[k] + 1); t.msg0 = ch.d_msg(j.msg_off); t.msg = ch.d_msg(j.msg_off + 4 + 3 * (size_t)S[k]);
+                tail_bytes += 2 * (size_t)j.nvec * t.n * sizeof(X);
             }
         }
         // upload descriptors
