@@ -36,7 +36,8 @@ SYMBOLS = [
     "hg_circuit_new_host", "hg_circuit_insert_lasso_host", "hg_gkr_verify", "hg_mle_eval_host", "hg_bfv_witness_generate", "hg_lasso_node_verify", "hg_sumcheck_prove", "hg_mle_eval_batch", "hg_ntt", "hg_bfv_configure", "hg_field_selftest",
     "hg_circuit_new", "hg_circuit_free", "hg_circuit_insert_input", "hg_circuit_insert_fft", "hg_circuit_insert_lasso", "hg_circuit_insert_vanilla",
     "hg_circuit_connect", "hg_circuit_evaluate", "hg_circuit_evaluate_host", "hg_circuit_node_value", "hg_gkr_prove", "hg_gkr_timing", "hg_gkr_num_challenges", "hg_gkr_num_inputs", "hg_gkr_num_input_claims",
-    "hg_gkr_input_claim_num_vars", "hg_gkr_input_claim",
+    "hg_gkr_input_claim_num_vars", "hg_gkr_input_claim", "hg_verifier_new", "hg_verifier_free", "hg_gkr_verify_batch", "hg_verifier_reason", "hg_mle_eval_multi",
+    "hg_verifier_num_inputs", "hg_verifier_input_len", "hg_verifier_timing",
 ]
 
 # callback types of hg_transcript_from_callbacks (include/hg_b200.h)
@@ -100,6 +101,19 @@ def lib():
         L.hg_transcript_proof_copy.argtypes = [vp, vp, sz]
         L.hg_transcript_num_squeezed.argtypes = [vp]
         L.hg_transcript_num_squeezed.restype = sz
+        L.hg_verifier_new.argtypes = [vp, vp, sz, C.POINTER(vp)]
+        L.hg_verifier_free.argtypes = [vp]
+        L.hg_verifier_free.restype = None
+        L.hg_gkr_verify_batch.argtypes = [vp, sz, vp, sz, vp, vp, vp, vp, i32, vp, vp]
+        L.hg_verifier_reason.argtypes = [vp, sz]
+        L.hg_verifier_reason.restype = C.c_char_p
+        L.hg_verifier_num_inputs.argtypes = [vp]
+        L.hg_verifier_num_inputs.restype = sz
+        L.hg_verifier_input_len.argtypes = [vp, sz]
+        L.hg_verifier_input_len.restype = sz
+        L.hg_verifier_timing.argtypes = [vp, vp]
+        L.hg_verifier_timing.restype = None
+        L.hg_mle_eval_multi.argtypes = [vp, sz, vp, vp, vp, i32, vp]
         L.hg_lasso_preprocess.argtypes = [vp, sz, sz, sz, C.POINTER(vp)]
         L.hg_lasso_pp_free.argtypes = [vp]
         L.hg_lasso_preprocess_lookups.argtypes = [vp, sz, sz, sz, C.POINTER(vp)]
@@ -824,6 +838,22 @@ def mle_eval_batch(ctx: Context, d_tables: DeviceBuffer, n_tables, num_vars, poi
     return out
 
 
+def mle_eval_multi(ctx: Context, tables, points):
+    """MLE of each base table at its own point on the device (hg_mle_eval_multi). tables: DeviceBuffer / DeviceView (library
+    representation) or host numpy arrays of canonical limbs, all of one kind; points: one [num_vars, el] array per table."""
+    el = LIMBS[ctx.field] * DEGREE[ctx.field]
+    on_dev = len(tables) > 0 and not isinstance(tables[0], np.ndarray)
+    keep = [t if on_dev else np.ascontiguousarray(t, np.uint64).reshape(-1) for t in tables]
+    if len(points) != len(keep) or (not on_dev and any(t.size != (LIMBS[ctx.field] << len(p)) for t, p in zip(keep, points))):
+        raise HgError("mle_eval_multi: every table must have 2^num_vars elements, one point per table")
+    ptrs = (C.c_void_p * max(len(keep), 1))(*[(t.ptr if on_dev else t.ctypes.data) for t in keep])
+    nvs = np.array([len(p) for p in points], np.uint64)
+    pts = np.ascontiguousarray(np.concatenate([np.asarray(p, np.uint64).reshape(-1) for p in points] + [np.zeros(0, np.uint64)]))
+    out = np.zeros((len(keep), el), np.uint64)
+    _chk(lib().hg_mle_eval_multi(ctx.h, len(keep), ptrs, _p(nvs), _p(pts), 1 if on_dev else 0, _p(out)))
+    return out
+
+
 def field_selftest(ctx: Context, op, a_ext, b_ext):
     a = np.ascontiguousarray(a_ext, np.uint64)
     b = np.ascontiguousarray(b_ext, np.uint64)
@@ -1117,6 +1147,89 @@ class BfvSkEncryptVerifier:
         except HgError:
             return claims
         raise HgError("verify: trailing bytes in proof")
+
+    def verify_batch(self, ctx: Context, inputs_list, ct0is_list, proofs, options=None):
+        """verify() for a batch of proofs on the device of `ctx` (hg_gkr_verify_batch), with the same verdicts. inputs_list[p] are
+        proof p's inputs in get_inputs order and ct0is_list[p] its ct0is: host numpy arrays of canonical limbs, or DeviceBuffers in
+        the library's representation (as hg_bfv_witness_generate writes them). proofs are bytes, or transcripts (from_proof or a
+        CallbackTranscript with a read callback) positioned at the start of the proof. Returns [(ok, reason)] per proof."""
+        n = len(proofs)
+        if n == 0:
+            return []
+        bv = getattr(self, "_batch", None)
+        if bv is None or bv.ctx is not ctx or bv.max_batch < n:
+            if bv is not None:
+                bv.free()
+            bv = self._batch = GkrBatchVerifier(ctx, self.circuit, n)
+        trs = [Keccak256Transcript.from_proof(p, self.field) if isinstance(p, (bytes, bytearray)) else p for p in proofs]
+        L = self.ct0is_log2_size
+        points = [t.squeeze_challenges(L) for t in trs]                                           # :499
+        values = mle_eval_multi(ctx, list(ct0is_list), points)                                    # :500
+        el = points[0].shape[1]
+        oc = [[(np.zeros((0, el), np.uint64), np.zeros(el, np.uint64)), (points[p], values[p])] for p in range(n)]
+        res = bv.verify_batch(trs, oc, inputs_list, options)                                      # :504-516
+        out = []
+        for t, (ok, why) in zip(trs, res):
+            if ok:
+                try:
+                    t.read_felt_ext()
+                    ok, why = False, "verify: trailing bytes in proof"
+                except HgError:
+                    pass
+            out.append((ok, why))
+        return out
+
+
+class GkrBatchVerifier:
+    """Batched device verifier of one circuit (hg_verifier_new): `desc` is a host-only Circuit description."""
+
+    def __init__(self, ctx: Context, desc: "Circuit", max_batch: int):
+        self.ctx, self.desc, self.max_batch = ctx, desc, max_batch
+        self.h = C.c_void_p()
+        _chk(lib().hg_verifier_new(ctx.h, desc.h, max_batch, C.byref(self.h)))
+        self.input_lens = [int(lib().hg_verifier_input_len(self.h, i)) for i in range(lib().hg_verifier_num_inputs(self.h))]
+
+    def verify_batch(self, transcripts, output_claims, inputs, options=None):
+        """transcripts: one per proof; output_claims: per proof a list of (point, value), the same point lengths for every proof;
+        inputs: per proof the input tables in insertion order, all DeviceBuffer / DeviceView or all host numpy arrays.
+        Returns [(ok, reason)] per proof."""
+        n = len(transcripts)
+        if n == 0:
+            return []
+        lens = np.array([len(p) for p, _ in output_claims[0]], np.uint64)
+        if len(output_claims) != n or any([len(p) for p, _ in oc] != list(lens) for oc in output_claims):
+            raise HgError("verify_batch: one list of output claims per proof, with the same point lengths for every proof")
+        pts = np.ascontiguousarray(np.concatenate([np.asarray(p, np.uint64).reshape(-1) for oc in output_claims for p, _ in oc] + [np.zeros(0, np.uint64)]))
+        vals = np.ascontiguousarray(np.concatenate([np.asarray(v, np.uint64).reshape(-1) for oc in output_claims for _, v in oc] + [np.zeros(0, np.uint64)]))
+        flat = [t for ins in inputs for t in ins]
+        on_dev = len(flat) > 0 and not isinstance(flat[0], np.ndarray)
+        keep = [t if on_dev else np.ascontiguousarray(t, np.uint64).reshape(-1) for t in flat]
+        if len(inputs) != n or any(len(ins) != len(self.input_lens) for ins in inputs) or \
+                (not on_dev and any(t.size != LIMBS[self.ctx.field] * m for ins in inputs for t, m in zip(ins, self.input_lens))):
+            raise HgError("verify_batch: one list of inputs per proof, each input of its node's size")
+        ptrs = (C.c_void_p * max(len(keep), 1))(*[(t.ptr if on_dev else t.ctypes.data) for t in keep])
+        trs = (C.c_void_p * n)(*[t.h.value if isinstance(t.h, C.c_void_p) else t.h for t in transcripts])
+        status = np.zeros(n, np.int32)
+        opt = None if options is None else np.array(options, np.int32)
+        _chk(lib().hg_gkr_verify_batch(self.h, n, trs, len(lens), _p(lens), _p(pts), _p(vals), ptrs, 1 if on_dev else 0, _p(opt), _p(status)))
+        return [(bool(status[p]), lib().hg_verifier_reason(self.h, p).decode()) for p in range(n)]
+
+    def timing(self):
+        """host microseconds of the last batch: replays of every proof, device stages (enqueue and wait), closing the records"""
+        out = np.zeros(3, np.float64)
+        lib().hg_verifier_timing(self.h, _p(out))
+        return dict(zip(("replay_us", "device_us", "close_us"), (float(x) for x in out)))
+
+    def free(self):
+        if self.h:
+            lib().hg_verifier_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
 
 
 class BfvSkEncryptProver:

@@ -16,6 +16,7 @@
 #include "prover.cuh"
 #include "lasso_verify.hpp"
 #include "gkr_verify.hpp"
+#include "verify_batch.cuh"
 #include "witness_gen.cuh"
 
 using namespace hg;
@@ -87,6 +88,9 @@ template <class FP> struct FieldState {
     DevBuf<X> mle_pt, mle_eq, mle_partials, mle_out;
     DevBuf<unsigned> mle_counters;
     PinnedBuf<X> mle_hpt;
+    // hg_mle_eval_multi
+    std::unique_ptr<VerifyScratch<FP>> multi_sc;
+    DevBuf<unsigned char> multi_stage;
 };
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize belongs to a kernel and a device, so every context in the process shares it. It is
@@ -129,6 +133,15 @@ static void circuit_use_device(hg_circuit* c) {
     if (!c->ctx) throw std::runtime_error("this circuit is a host-only description (hg_circuit_new_host): it has no device, only hg_gkr_verify runs on it");
     HG_CUDA(cudaSetDevice(c->ctx->dev.device));
 }
+struct hg_verifier {
+    template <class FP> hg_verifier(hg_ctx* c, FP, const GkrVerifierHost<FP>& desc, size_t max_batch)
+        : ctx(c), v(std::in_place_type<VerifierDev<FP>>, &c->dev, typed_state<FP>(c).eng(&c->dev), desc, max_batch) {}
+    template <class FP> static FieldState<FP>& typed_state(hg_ctx* c) { return std::get<FieldState<FP>>(c->state); }
+    hg_ctx* ctx;
+    std::variant<VerifierDev<GlField>, VerifierDev<FrField>> v;
+    DevBuf<unsigned char> staging;     // host inputs on their way to the device
+    std::vector<std::string> reasons;  // of the last batch, per proof ("" when accepted)
+};
 struct hg_buf {
     void* p = nullptr;
     size_t bytes = 0;
@@ -338,6 +351,79 @@ template <class FP> void mle_eval_batch(hg_ctx* ctx, const void* d_tables, size_
     HG_CUDA(cudaMemcpyAsync(ho, out.p, n_tables * sizeof(X), cudaMemcpyDeviceToHost, s));
     HG_CUDA(cudaStreamSynchronize(s));
     for (size_t i = 0; i < n_tables; i++) FP::x_to_limbs(ho[i], out_ext + FP::X_LIMBS * i);
+}
+
+// host vectors of canonical limbs to the device, back to back in `stage`, in the library's representation; returns the tables
+template <class FP> std::vector<const typename FP::B*> stage_tables(DeviceCtx* dev, DevBuf<unsigned char>& stage, const void* const* tables, const size_t* lens, size_t n) {
+    typedef typename FP::B B;
+    size_t total = 0;
+    for (size_t i = 0; i < n; i++) total += lens[i];
+    if (stage.n < total * sizeof(B)) { HG_CUDA(cudaStreamSynchronize(dev->stream)); stage.alloc(total * sizeof(B)); }
+    std::vector<const B*> out;
+    B* p = (B*)stage.p;
+    for (size_t i = 0; i < n; i++) {
+        if (!tables[i]) throw std::runtime_error("NULL table");
+        HG_CUDA(cudaMemcpyAsync(p, tables[i], lens[i] * sizeof(B), cudaMemcpyHostToDevice, dev->stream));
+        out.push_back(p);
+        p += lens[i];
+    }
+    if (FP::FIELD_ID == 1 && total) { k_field_encode<FP><<<(unsigned)((total + 255) / 256), 256, 0, dev->stream>>>((B*)stage.p, total, 0); HG_LAUNCH_CHECK(); }
+    return out;
+}
+
+// hg_mle_eval_multi
+template <class FP> void mle_eval_multi(hg_ctx* ctx, size_t n, const void* const* tables, const size_t* num_vars, const uint64_t* points_ext, int on_device, uint64_t* out_ext) {
+    typedef typename FP::B B;
+    typedef typename FP::X X;
+    FieldState<FP>& fs = typed<FP>(ctx);
+    if (!fs.multi_sc) fs.multi_sc.reset(new VerifyScratch<FP>(&ctx->dev));
+    std::vector<std::vector<X>> pts(n);
+    std::vector<size_t> lens(n);
+    size_t off = 0;
+    for (size_t i = 0; i < n; i++) {
+        if (num_vars[i] > 40) throw std::runtime_error("hg_mle_eval_multi: num_vars out of range");
+        lens[i] = (size_t)1 << num_vars[i];
+        for (size_t k = 0; k < num_vars[i]; k++) pts[i].push_back(FP::x_from_limbs(points_ext + FP::X_LIMBS * (off + k)));
+        off += num_vars[i];
+    }
+    std::vector<const B*> tabs;
+    if (on_device) for (size_t i = 0; i < n; i++) { if (!tables[i]) throw std::runtime_error("hg_mle_eval_multi: NULL table"); tabs.push_back((const B*)tables[i]); }
+    else tabs = stage_tables<FP>(&ctx->dev, fs.multi_stage, tables, lens.data(), n);
+    std::vector<const std::vector<X>*> pp;
+    for (auto& p : pts) pp.push_back(&p);
+    const std::vector<X> v = mle_eval_items<FP>(&ctx->dev, *fs.multi_sc, tabs, pp);
+    for (size_t i = 0; i < n; i++) FP::x_to_limbs(v[i], out_ext + FP::X_LIMBS * i);
+}
+
+// hg_gkr_verify_batch
+template <class FP> void gkr_verify_batch(hg_verifier* hv, VerifierDev<FP>& vd, size_t np, hg_transcript* const* trs, size_t n_oc, const size_t* point_lens,
+                                          const uint64_t* points_ext, const uint64_t* values_ext, const void* const* inputs, int on_device, const int* options3,
+                                          int* out_status) {
+    typedef typename FP::B B;
+    typedef typename GkrVerifierHost<FP>::Claim Claim;
+    if (np > vd.max_batch()) throw std::runtime_error("hg_gkr_verify_batch: n_proofs exceeds the verifier's max_batch");
+    if (np && (!trs || !inputs || !out_status || (n_oc && (!point_lens || !points_ext || !values_ext)))) throw std::runtime_error("hg_gkr_verify_batch: NULL argument");
+    size_t pt_elems = 0;
+    for (size_t i = 0; i < n_oc; i++) pt_elems += point_lens[i];
+    std::vector<Keccak256Transcript<FP>*> tv;
+    std::vector<std::vector<Claim>> oc;
+    for (size_t p = 0; p < np; p++) {
+        if (!trs[p]) throw std::runtime_error("hg_gkr_verify_batch: NULL transcript");
+        tv.push_back(&typed<FP>(trs[p]));
+        oc.push_back(claims_from_limbs<FP, Claim>(n_oc, point_lens, points_ext + p * pt_elems * FP::X_LIMBS, values_ext + p * n_oc * FP::X_LIMBS));
+    }
+    const size_t ni = vd.num_inputs();
+    std::vector<const B*> tabs;
+    if (on_device) {
+        for (size_t k = 0; k < np * ni; k++) { if (!inputs[k]) throw std::runtime_error("hg_gkr_verify_batch: NULL input"); tabs.push_back((const B*)inputs[k]); }
+    } else {
+        std::vector<size_t> lens;
+        for (size_t p = 0; p < np; p++) lens.insert(lens.end(), vd.input_lens().begin(), vd.input_lens().end());
+        tabs = stage_tables<FP>(&hv->ctx->dev, hv->staging, inputs, lens.data(), np * ni);
+    }
+    const auto res = vd.verify(tv, oc, tabs, wire_options(options3));
+    hv->reasons.assign(np, std::string());
+    for (size_t p = 0; p < np; p++) { out_status[p] = res[p].ok ? 1 : 0; hv->reasons[p] = res[p].reason; }
 }
 
 // hg_bfv_witness_generate: scripts/circuit_sk.py:72-140 on the device (witness_gen.cuh). Small host inputs, device outputs in
@@ -973,6 +1059,56 @@ int hg_mle_eval_host(int field_id, const uint64_t* table_limbs, size_t n, size_t
             for (size_t i = 0; i < num_vars; i++) pt[i] = FP::x_from_limbs(point_ext + i * FP::X_LIMBS);
             FP::x_to_limbs(GkrVerifierHost<FP>::mle_eval_base(t.data(), n, pt), out_ext);
         });
+    })
+}
+int hg_verifier_new(hg_ctx* ctx, const hg_circuit* desc, size_t max_batch, hg_verifier** out) {
+    HG_TRY({
+        if (!ctx || !desc || !out) throw std::runtime_error("hg_verifier_new: NULL argument");
+        if (desc->ctx) throw std::runtime_error("hg_verifier_new needs a host-only circuit description (hg_circuit_new_host)");
+        if (desc->field_id != ctx->field_id) throw std::runtime_error("hg_verifier_new: the description and the context belong to different fields");
+        HG_CUDA(cudaSetDevice(ctx->dev.device));
+        *out = with_field(ctx->field_id, [&](auto fp) {
+            typedef decltype(fp) FP;
+            return new hg_verifier(ctx, fp, std::get<GkrVerifierHost<FP>>(desc->c), max_batch);
+        });
+    })
+}
+void hg_verifier_free(hg_verifier* v) {
+    if (!v) return;
+    cudaSetDevice(v->ctx->dev.device);
+    delete v;
+}
+int hg_gkr_verify_batch(hg_verifier* v, size_t n_proofs, hg_transcript* const* transcripts, size_t n_output_claims, const size_t* point_lens,
+                        const uint64_t* points_ext, const uint64_t* values_ext, const void* const* inputs, int inputs_on_device, const int* options3,
+                        int* out_status) {
+    HG_TRY({
+        if (!v) throw std::runtime_error("hg_gkr_verify_batch: NULL verifier");
+        HG_CUDA(cudaSetDevice(v->ctx->dev.device));
+        std::visit([&](auto& vd) {
+            gkr_verify_batch<field_t<decltype(vd)>>(v, vd, n_proofs, transcripts, n_output_claims, point_lens, points_ext, values_ext, inputs, inputs_on_device,
+                                                     options3, out_status);
+        }, v->v);
+    })
+}
+size_t hg_verifier_num_inputs(const hg_verifier* v) { return v ? std::visit([](auto& vd) { return vd.num_inputs(); }, v->v) : 0; }
+size_t hg_verifier_input_len(const hg_verifier* v, size_t input) {
+    if (!v) return 0;
+    return std::visit([&](auto& vd) { return input < vd.num_inputs() ? vd.input_lens()[input] : (size_t)0; }, v->v);
+}
+void hg_verifier_timing(const hg_verifier* v, double* out_us3) {
+    const double* t = std::visit([](auto& vd) { return vd.timing(); }, v->v);
+    for (int i = 0; i < 3; i++) out_us3[i] = t[i];
+}
+const char* hg_verifier_reason(const hg_verifier* v, size_t proof) {
+    if (!v || proof >= v->reasons.size()) return "";
+    return v->reasons[proof].c_str();
+}
+int hg_mle_eval_multi(hg_ctx* ctx, size_t n_items, const void* const* tables, const size_t* num_vars, const uint64_t* points_ext, int tables_on_device,
+                      uint64_t* out_ext) {
+    HG_TRY({
+        if (!ctx || (n_items && (!tables || !num_vars || !out_ext))) throw std::runtime_error("hg_mle_eval_multi: NULL argument");
+        HG_CUDA(cudaSetDevice(ctx->dev.device));
+        with_field(ctx->field_id, [&](auto fp) { mle_eval_multi<decltype(fp)>(ctx, n_items, tables, num_vars, points_ext, tables_on_device, out_ext); });
     })
 }
 void hg_circuit_free(hg_circuit* c) {

@@ -12,6 +12,12 @@
 //       FFT forward / inverse     W = transform of sum_t alpha^t eq(z_t, .)   (the DFT matrix is symmetric)
 //       Lasso                     LassoVerifier (lasso_verify.hpp)
 // It returns the claims that reach the input nodes; the caller compares them with the MLEs of the inputs (hg_mle_eval_host).
+//
+// The same walk is the replay of the batched device verifier (verify_batch.cuh): given a DeferredChecks sink, every final
+// check whose quantity is linear in the circuit size (the FFT and linear layers' weights at the sumcheck point, the Lasso
+// subtables at y) is recorded instead of computed. That is sound because no such quantity feeds a later transcript step or
+// claim: each one only closes its own node's final equality. General layers are checked in full on the host: their A(u) must
+// be, since it enters the phase-2 claim; their M(u, v) could be deferred like the others but is not (yet).
 #pragma once
 #include <algorithm>
 #include <memory>
@@ -21,35 +27,46 @@
 
 namespace hg {
 
-// gkr::sum_check::verify_sum_check for a degree-`deg` round polynomial [UPSTREAM, assumptions A3 / A3']
+// gkr::sum_check::verify_sum_check for a degree-`deg` round polynomial [UPSTREAM, assumptions A3 / A3'].
+// The final claim is an affine function of the initial one; out_slope (optional) receives its slope, so a caller that does not
+// know a term of the initial claim yet can start from claim + d and subtract slope * d from the final claim.
 template <class FP>
 void verify_sum_check_host(int deg, int nv, typename FP::X claim, Keccak256Transcript<FP>& tr, const WireOptions& wo, typename FP::X* out_claim,
-                           std::vector<typename FP::X>* out_point) {
+                           std::vector<typename FP::X>* out_point, typename FP::X* out_slope = nullptr) {
     typedef typename FP::X X;
     typedef RoundPoly<FP> RP;
     out_point->clear();
+    X slope = FP::x_one();
     for (int j = 0; j < nv; j++) {
         std::vector<X> msg(deg);
         for (auto& v : msg) v = tr.read_felt_ext();
-        std::vector<X> co(deg + 1);
-        if (wo.a3_wire == 0) {
-            co[0] = msg[0];
-            X rest = FP::x_add(co[0], co[0]);
-            for (int k = 2; k <= deg; k++) { co[k] = msg[k - 1]; rest = FP::x_add(rest, co[k]); }
-            co[1] = FP::x_sub(claim, rest);
-        } else {
-            std::vector<X> ev(deg + 1);
-            ev[0] = msg[0];
-            ev[1] = FP::x_sub(claim, ev[0]);
-            for (int k = 2; k <= deg; k++) ev[k] = msg[k - 1];
-            co = RP::interpolate(ev);
-        }
+        auto round = [&](X c) {  // the round polynomial's coefficients given the claim c
+            std::vector<X> co(deg + 1);
+            if (wo.a3_wire == 0) {
+                co[0] = msg[0];
+                X rest = FP::x_add(co[0], co[0]);
+                for (int k = 2; k <= deg; k++) { co[k] = msg[k - 1]; rest = FP::x_add(rest, co[k]); }
+                co[1] = FP::x_sub(c, rest);
+            } else {
+                std::vector<X> ev(deg + 1);
+                ev[0] = msg[0];
+                ev[1] = FP::x_sub(c, ev[0]);
+                for (int k = 2; k <= deg; k++) ev[k] = msg[k - 1];
+                co = RP::interpolate(ev);
+            }
+            return co;
+        };
+        const std::vector<X> co = round(claim);
         const X rj = tr.squeeze_challenge();
-        claim = RP::horner(co, rj);
+        const X next = RP::horner(co, rj);
+        if (out_slope) slope = FP::x_mul(slope, FP::x_sub(RP::horner(round(FP::x_add(claim, FP::x_one())), rj), next));
+        claim = next;
         out_point->push_back(rj);
     }
     *out_claim = claim;
+    if (out_slope) *out_slope = slope;
 }
+
 
 template <class FP> class GkrVerifierHost {
   public:
@@ -108,9 +125,27 @@ template <class FP> class GkrVerifierHost {
         nodes_[from].succs.push_back(to);
     }
     size_t num_nodes() const { return nodes_.size(); }
+    // what the device verifier uploads (verify_batch.cuh)
+    int node_kind(int id) const { return nodes_.at(id).kind; }
+    bool node_is_linear(int id) const { const Node& n = nodes_.at(id); return n.kind == GKR_VANILLA && n.is_linear; }
+    bool node_fft_inverse(int id) const { return nodes_.at(id).fft_inverse; }
+    size_t node_out_len(int id) const { return nodes_.at(id).out_len; }
+    size_t node_n_in(int id) const { return nodes_.at(id).n_in; }
+    size_t node_in_len(int id) const { const Node& n = nodes_.at(id); return n.a_pad * n.n_in; }  // S: the concatenated inputs
+    int node_num_reps(int id) const { return nodes_.at(id).num_reps; }
+    size_t node_num_gates(int id) const { return nodes_.at(id).ng; }
+    const VanillaDesc* node_desc(int id) const { return nodes_.at(id).desc.get(); }
+    const LassoPreprocessing* node_lasso(int id) const { return nodes_.at(id).pp.get(); }
+    std::vector<size_t> input_lens() const {
+        std::vector<size_t> v;
+        for (auto& n : nodes_) if (n.kind == GKR_INPUT) v.push_back(n.out_len);
+        return v;
+    }
 
     // verify_gkr: one output claim per output node (insertion order); returns the claims on the input nodes (insertion order)
-    std::vector<std::vector<Claim>> verify(Keccak256Transcript<FP>& tr, const WireOptions& wo, const std::vector<Claim>& output_claims) {
+    // defer == nullptr: every check now (hg_gkr_verify); otherwise the linear-size final checks are appended to *defer
+    std::vector<std::vector<Claim>> verify(Keccak256Transcript<FP>& tr, const WireOptions& wo, const std::vector<Claim>& output_claims,
+                                           DeferredChecks<FP>* defer = nullptr) {
         std::vector<std::vector<Claim>> claims(nodes_.size());
         std::vector<int> outs;
         for (size_t i = 0; i < nodes_.size(); i++) if (nodes_[i].succs.empty() && nodes_[i].kind != GKR_INPUT) outs.push_back((int)i);
@@ -121,7 +156,7 @@ template <class FP> class GkrVerifierHost {
             const int id = ord[oi];
             const Node& n = nodes_[id];
             if (n.kind == GKR_INPUT) continue;
-            std::vector<std::vector<Claim>> sub = verify_node(n, claims[id], tr, wo);
+            std::vector<std::vector<Claim>> sub = verify_node(id, n, claims[id], tr, wo, defer);
             for (size_t k = 0; k < sub.size(); k++) for (auto& c : sub[k]) claims[n.preds.at(k)].push_back(c);
         }
         std::vector<std::vector<Claim>> res;
@@ -218,37 +253,54 @@ template <class FP> class GkrVerifierHost {
         return order;
     }
 
-    std::vector<std::vector<Claim>> verify_node(const Node& n, const std::vector<Claim>& cl, Keccak256Transcript<FP>& tr, const WireOptions& wo) {
+    std::vector<std::vector<Claim>> verify_node(int id, const Node& n, const std::vector<Claim>& cl, Keccak256Transcript<FP>& tr, const WireOptions& wo,
+                                                DeferredChecks<FP>* defer) {
         std::vector<std::vector<Claim>> out(n.preds.size());
         if (n.kind == GKR_LASSO) {
             if (n.preds.size() != 1) throw VerifyError("the Lasso node takes exactly one input (lasso.rs:64)");
             LassoVerifier<FP> lv(*n.pp, n.lasso_nv, wo);
             Claim c;
-            lv.verify(tr, &c.point, &c.value);
+            lv.verify(tr, &c.point, &c.value, defer);
             out[0].push_back(c);
             return out;
         }
         if (cl.empty()) throw VerifyError("verify_gkr: node without claims");
         X alpha = FP::x_one();
         if (cl.size() > 1) alpha = tr.squeeze_challenge();
-        // combined claim and W = sum_t alpha^t eq(z_t, .)
+        // combined claim and W = sum_t alpha^t eq(z_t, .); W only where the host checks need it
         X combined = FP::x_zero();
-        std::vector<X> w(n.out_len, FP::x_zero());
         {
             X p = FP::x_one();
             for (auto& c : cl) {
                 if (((size_t)1 << c.point.size()) != n.out_len) throw VerifyError("verify_gkr: claim point does not match the node's output size");
                 combined = FP::x_add(combined, FP::x_mul(p, c.value));
+                p = FP::x_mul(p, alpha);
+            }
+        }
+        std::vector<X> w;
+        const bool on_host = !defer || (n.kind == GKR_VANILLA && !n.is_linear && !n.is_elemmul);
+        if (on_host && !n.is_elemmul) {
+            w.assign(n.out_len, FP::x_zero());
+            X p = FP::x_one();
+            for (auto& c : cl) {
                 const std::vector<X> eq = eq_table(c.point);
                 for (size_t i = 0; i < n.out_len; i++) w[i] = FP::x_add(w[i], FP::x_mul(p, eq[i]));
                 p = FP::x_mul(p, alpha);
             }
         }
+        auto record = [&](int kind, const std::vector<X>& pt, X factor, X slope, X target, const char* what) {
+            DeferredCheck<FP> d;
+            d.kind = kind; d.index = id; d.alpha = alpha; d.pt = pt; d.factor = factor; d.slope = slope; d.target = target; d.what = what;
+            for (auto& c : cl) d.z.push_back(c.point);
+            defer->push_back(std::move(d));
+        };
         std::vector<X> pt;
         X fc;
         if (n.kind == GKR_FFT) {
             verify_sum_check_host<FP>(2, n.log2_size, combined, tr, wo, &fc, &pt);
             const X in_eval = tr.read_felt_ext();
+            out.at(0).push_back({pt, in_eval});
+            if (!on_host) { record(DC_FFT, pt, in_eval, FP::x_zero(), fc, "InvalidSumCheck: FFT layer final evaluation mismatch"); return out; }
             // A = transform(W), plane by plane
             std::vector<B> plane(n.out_len);
             std::vector<X> A(n.out_len);
@@ -264,20 +316,28 @@ template <class FP> class GkrVerifierHost {
                 A[i] = FP::from_planes(b);
             }
             if (!FP::x_eq(FP::x_mul(mle_eval_ext(std::move(A), pt), in_eval), fc)) throw VerifyError("InvalidSumCheck: FFT layer final evaluation mismatch");
-            out.at(0).push_back({pt, in_eval});
         } else if (n.is_elemmul) {
             verify_sum_check_host<FP>(3, log2sz(n.out_len), combined, tr, wo, &fc, &pt);
             const X a = tr.read_felt_ext(), b = tr.read_felt_ext();
-            if (!FP::x_eq(FP::x_mul(FP::x_mul(mle_eval_ext(std::move(w), pt), a), b), fc)) throw VerifyError("InvalidSumCheck: product layer final evaluation mismatch");
+            // MLE(W)(pt) = sum_t alpha^t eq(z_t, pt), O(nv) per claim and equal to folding the table
+            X wpt = FP::x_zero(), p = FP::x_one();
+            for (auto& c : cl) {
+                X e = FP::x_one();
+                for (size_t i = 0; i < pt.size(); i++)
+                    e = FP::x_mul(e, FP::x_add(FP::x_mul(c.point[i], pt[i]), FP::x_mul(FP::x_sub(FP::x_one(), c.point[i]), FP::x_sub(FP::x_one(), pt[i]))));
+                wpt = FP::x_add(wpt, FP::x_mul(p, e));
+                p = FP::x_mul(p, alpha);
+            }
+            if (!FP::x_eq(FP::x_mul(FP::x_mul(wpt, a), b), fc)) throw VerifyError("InvalidSumCheck: product layer final evaluation mismatch");
             out.at(0).push_back({pt, a});
             out.at(1).push_back({pt, b});
         } else if (n.is_linear) {
             if ((int)n.preds.size() != n.arity) throw VerifyError("Vanilla node arity does not match its connections");
             const VanillaDesc& d = *n.desc;
             const size_t S = n.a_pad * n.n_in, sub = (size_t)1 << n.log2_sub;
-            std::vector<X> A(S, FP::x_zero());
+            std::vector<X> A(on_host ? S : 0, FP::x_zero());
             X constant = FP::x_zero();
-            for (size_t r = 0; r < (size_t)n.num_reps; r++)
+            for (size_t r = 0; on_host && r < (size_t)n.num_reps; r++)
                 for (size_t g = 0; g < n.ng; g++) {
                     const X wg = w[r * n.ng + g];
                     if (d.has_const[g]) constant = FP::x_add(constant, FP::x_mul_b(wg, FP::b_from_limbs(&d.consts[g * FP::B_LIMBS])));
@@ -286,7 +346,9 @@ template <class FP> class GkrVerifierHost {
                         a = FP::x_add(a, FP::x_mul_b(wg, FP::b_from_limbs(&d.add_coef[e * FP::B_LIMBS])));
                     }
                 }
-            verify_sum_check_host<FP>(2, log2sz(S), FP::x_sub(combined, constant), tr, wo, &fc, &pt);
+            // deferred: the sumcheck starts from `combined`, and the constant part comes back as slope * q_const
+            X slope = FP::x_zero();
+            verify_sum_check_host<FP>(2, log2sz(S), FP::x_sub(combined, constant), tr, wo, &fc, &pt, defer ? &slope : nullptr);
             const int lo_vars = log2sz(n.n_in);
             std::vector<X> lo(pt.begin(), pt.begin() + lo_vars), hi(pt.begin() + lo_vars, pt.end());
             const std::vector<X> eqhi = eq_table(hi);
@@ -296,6 +358,7 @@ template <class FP> class GkrVerifierHost {
                 x = FP::x_add(x, FP::x_mul(eqhi[k], e));
                 out[k].push_back({lo, e});
             }
+            if (!on_host) { record(DC_LINEAR, pt, x, slope, fc, "InvalidSumCheck: linear layer final evaluation mismatch"); return out; }
             if (!FP::x_eq(FP::x_mul(mle_eval_ext(std::move(A), pt), x), fc)) throw VerifyError("InvalidSumCheck: linear layer final evaluation mismatch");
         } else {  // general layer: phase 1 over x (claim c - const), phase 2 over y (claim fc1 - A(u) X(u)), DESIGN.md section 3 (A11)
             if ((int)n.preds.size() != n.arity) throw VerifyError("Vanilla node arity does not match its connections");

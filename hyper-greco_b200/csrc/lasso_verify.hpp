@@ -18,6 +18,23 @@ struct VerifyError : std::runtime_error {
     explicit VerifyError(const std::string& m) : std::runtime_error(m) {}
 };
 
+// A final check of the replay left to the device: factor * q + slope * q_const == target, where q (and q_const) are linear-size
+// quantities of the circuit fixed by the claim points, alpha and pt.
+//   DC_FFT       q = MLE(transform(W))(pt),  W = sum_t alpha^t eq(z_t, .) over the node's outputs
+//   DC_LINEAR    q = MLE(A)(pt), A = W pushed through the additive edges; q_const = sum_g W[g] const_g (the claim's constant part)
+//   DC_SUBTABLE  q = MLE(subtable `index`)(pt)
+//   DC_INPUT     q = MLE(input node `index`)(pt)
+enum DeferredKind { DC_FFT = 0, DC_LINEAR, DC_SUBTABLE, DC_INPUT };
+template <class FP> struct DeferredCheck {
+    typedef typename FP::X X;
+    int kind = DC_FFT, index = 0;  // node id (FFT, linear), subtable index, input index
+    std::vector<std::vector<X>> z;  // claim points (FFT, linear)
+    X alpha, factor, slope, target;
+    std::vector<X> pt;
+    const char* what = "";          // the rejection reason when the equality fails
+};
+template <class FP> using DeferredChecks = std::vector<DeferredCheck<FP>>;
+
 template <class FP> class LassoVerifier {
   public:
     typedef typename FP::B B;
@@ -29,8 +46,10 @@ template <class FP> class LassoVerifier {
         for (auto& kv : by_dim) chunks_.push_back(kv.second);
     }
 
-    // reads the node's part of the proof from `tr`, squeezing the challenges the prover squeezed; returns (r, claimed_sum)
-    void verify(Keccak256Transcript<FP>& tr, std::vector<X>* out_r, X* out_claimed_sum) {
+    // reads the node's part of the proof from `tr`, squeezing the challenges the prover squeezed; returns (r, claimed_sum).
+    // With `defer`, the init_ys / final_read_ys equalities, the only use of the subtable values st_y, become records
+    // gamma * st_y == ify - id_y - t gamma^2 + tau (DC_SUBTABLE) instead of materialising the subtables here.
+    void verify(Keccak256Transcript<FP>& tr, std::vector<X>* out_r, X* out_claimed_sum, DeferredChecks<FP>* defer = nullptr) {
         std::vector<X> r(num_vars_);
         for (auto& c : r) c = tr.squeeze_challenge();                         // lasso.rs:123
         const X claimed_sum = tr.read_felt_ext();                             // lasso.rs:344
@@ -46,7 +65,7 @@ template <class FP> class LassoVerifier {
         };
         X id_y = FP::x_zero();                                                // verifier.rs:74-78: sum_i 2^i y_i
         { X p2 = FP::x_one(); for (auto& yi : y) { id_y = FP::x_add(id_y, FP::x_mul(p2, yi)); p2 = FP::x_add(p2, p2); } }
-        const std::vector<X> eq_y = eq_table(y);
+        const std::vector<X> eq_y = defer ? std::vector<X>() : eq_table(y);
         std::map<size_t, X> subtable_at_y;                                     // LassoSubtable::evaluate_mle(y), one per subtable in use
         size_t off = 0;
         for (auto& mems : chunks_) {                                           // verifier.rs:61-95
@@ -57,6 +76,17 @@ template <class FP> class LassoVerifier {
                 if (!FP::x_eq(rw[off + i], hash(dim_x, e_x[i], ts_x))) throw VerifyError("verify_memories: read_xs mismatch");
                 if (!FP::x_eq(rw[m + off + i], hash(dim_x, e_x[i], FP::x_add(ts_x, FP::x_one())))) throw VerifyError("verify_memories: write_xs mismatch");
                 const size_t st = pp_.memory_to_subtable_index[mems[i]];
+                if (defer) {
+                    for (int fin = 0; fin < 2; fin++) {
+                        DeferredCheck<FP> d;
+                        d.kind = DC_SUBTABLE; d.index = (int)st; d.pt = y; d.factor = FP::lift(gamma); d.slope = FP::x_zero();
+                        const X t = fin ? fc_y : FP::x_zero();
+                        d.target = FP::x_add(FP::x_sub(FP::x_sub(ify[(fin ? m : 0) + off + i], id_y), FP::x_mul_b(t, gamma2)), FP::lift(tau));
+                        d.what = fin ? "verify_memories: final_read_ys mismatch" : "verify_memories: init_ys mismatch";
+                        defer->push_back(std::move(d));
+                    }
+                    continue;
+                }
                 if (!subtable_at_y.count(st)) subtable_at_y[st] = table_mle(pp_.subtables_by_idx[st]->materialize(pp_.M), eq_y);
                 const X st_y = subtable_at_y[st];
                 if (!FP::x_eq(ify[off + i], hash(id_y, st_y, FP::x_zero()))) throw VerifyError("verify_memories: init_ys mismatch");

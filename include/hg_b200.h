@@ -47,6 +47,7 @@ typedef struct hg_lasso_pp hg_lasso_pp;
 typedef struct hg_lasso_node hg_lasso_node;
 typedef struct hg_buf hg_buf;
 typedef struct hg_circuit hg_circuit;
+typedef struct hg_verifier hg_verifier;
 
 const char* hg_last_error(void);
 int hg_version(void);
@@ -305,6 +306,41 @@ int hg_gkr_verify(hg_circuit* c, size_t n_output_claims, const size_t* point_len
                   const int* options3);
 /* MultilinearPoly::evaluate on the host: table of 2^num_vars base elements (canonical limbs), point of num_vars extension elements */
 int hg_mle_eval_host(int field_id, const uint64_t* table_limbs, size_t n, size_t num_vars, const uint64_t* point_ext, uint64_t* out_ext);
+/* ---- batched verifier on the device: B proofs of one circuit per call.
+ *      hg_verifier_new takes a host-only description (hg_circuit_new_host + hg_bfv_configure or the insert / connect calls) of the
+ *      context's field, uploads its wiring (edges and constants of the linear layers) and its Lasso subtables once, and serves
+ *      batches of up to max_batch proofs. At most one Lasso node per circuit.
+ *      hg_gkr_verify_batch verifies n_proofs proofs: each is replayed on the host exactly as hg_gkr_verify does (every transcript
+ *      operation and scalar check), the checks whose cost is linear in the circuit size (FFT and linear layers at the sumcheck
+ *      point, Lasso subtables, every input claim) are evaluated on the device for the whole batch, and quantities that several
+ *      proofs share (the same points, as with hg_transcript_new / hg_transcript_from_proof) are computed once. General layers
+ *      are checked on the host. It is hg_gkr_verify followed by the input-claim comparison of :512-516, with the same verdict.
+ *        transcripts[p]      proof p's transcript (hg_transcript_from_proof, or a caller-owned one with a read callback), read as
+ *                            hg_gkr_verify reads it; the caller can check for trailing bytes afterwards
+ *        output claims       n_output_claims per proof with the same point_lens for every proof; proof p's points start at
+ *                            points_ext + p * sum(point_lens) * X limbs, its values at values_ext + p * n_output_claims * X limbs
+ *        inputs[p * I + i]   input node i of proof p (I input nodes, insertion order): device tables in the library's representation
+ *                            (inputs_on_device = 1, as hg_bfv_witness_generate writes them) or host vectors of canonical limbs
+ *        out_status[p]       1 accepted, 0 rejected; hg_verifier_reason(v, p) names the failed check of a rejected proof until
+ *                            the next batch (only the reason may differ from hg_gkr_verify's, never the verdict)
+ *      A malformed, truncated or tampered proof is a rejection, not an error. Invalid arguments, n_proofs > max_batch and CUDA
+ *      failures return non-zero. */
+int hg_verifier_new(hg_ctx* ctx, const hg_circuit* desc, size_t max_batch, hg_verifier** out);
+void hg_verifier_free(hg_verifier* v);
+int hg_gkr_verify_batch(hg_verifier* v, size_t n_proofs, hg_transcript* const* transcripts, size_t n_output_claims, const size_t* point_lens,
+                        const uint64_t* points_ext, const uint64_t* values_ext, const void* const* inputs, int inputs_on_device, const int* options3,
+                        int* out_status);
+const char* hg_verifier_reason(const hg_verifier* v, size_t proof);
+/* input nodes of the verifier's circuit and the elements of input i (insertion order; 0 out of range) */
+size_t hg_verifier_num_inputs(const hg_verifier* v);
+size_t hg_verifier_input_len(const hg_verifier* v, size_t input);
+/* host microseconds of the last hg_gkr_verify_batch: [replays of every proof, device stages (enqueue and wait), closing the records] */
+void hg_verifier_timing(const hg_verifier* v, double* out_us3);
+/* MLEs of n_items base tables, each at its own point, on the device: table i has 2^num_vars[i] elements (device tables in the
+ * library's representation when tables_on_device, else host vectors of canonical limbs); the points lie back to back in
+ * points_ext (num_vars[i] extension elements each); out_ext receives one extension element per item */
+int hg_mle_eval_multi(hg_ctx* ctx, size_t n_items, const void* const* tables, const size_t* num_vars, const uint64_t* points_ext, int tables_on_device,
+                      uint64_t* out_ext);
 /* host phases of the last hg_gkr_prove in microseconds: [witness kernels enqueue, squeeze+upload challenges, protocol walk,
  * batched layer enqueue, wait for the GPU, serialise]; number of extension challenges one proof squeezes */
 void hg_gkr_timing(const hg_circuit* c, double* out_us6);
