@@ -1181,7 +1181,8 @@ class BfvSkEncryptVerifier:
 
 
 class GkrBatchVerifier:
-    """Batched device verifier of one circuit (hg_verifier_new): `desc` is a host-only Circuit description."""
+    """Batched device verifier of one circuit (hg_verifier_new): `desc` is a host-only Circuit description of any node shapes the
+    host verifier takes (general Vanilla layers included); the verdicts are those of Circuit.verify_gkr plus the input-claim check."""
 
     def __init__(self, ctx: Context, desc: "Circuit", max_batch: int):
         self.ctx, self.desc, self.max_batch = ctx, desc, max_batch

@@ -669,9 +669,9 @@ template <class FP> class GkrCircuitDev {
             const size_t S = n.kind == GKR_FFT || n.is_elemmul ? n.out_len : n.a_pad * n.n_in;
             const int nv = log2sz(S), nt = n.is_elemmul ? 2 : 1;
             size_t n_claims = std::max<size_t>(1, n.succs.size());  // one claim per successor edge (upper bound: every successor pushes one)
-            // a successor may push several claims only through distinct input slots; count edges
+            // a successor pushes one claim per input slot this node fills, a general layer two (at u_lo and at v_lo)
             size_t edges = 0;
-            for (int sx : n.succs) for (int p : nodes_[sx]->preds) if (p == id) edges++;
+            for (int sx : n.succs) for (int p : nodes_[sx]->preds) if (p == id) edges += nodes_[sx]->is_general ? 2 : 1;
             n_claims = std::max<size_t>(1, edges);
             const int phases = n.is_general ? 2 : 1;
             chal += (n_claims > 1 ? 1 : 0) + phases * nv;

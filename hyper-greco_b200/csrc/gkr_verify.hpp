@@ -14,10 +14,11 @@
 // It returns the claims that reach the input nodes; the caller compares them with the MLEs of the inputs (hg_mle_eval_host).
 //
 // The same walk is the replay of the batched device verifier (verify_batch.cuh): given a DeferredChecks sink, every final
-// check whose quantity is linear in the circuit size (the FFT and linear layers' weights at the sumcheck point, the Lasso
-// subtables at y) is recorded instead of computed. That is sound because no such quantity feeds a later transcript step or
-// claim: each one only closes its own node's final equality. General layers are checked in full on the host: their A(u) must
-// be, since it enters the phase-2 claim; their M(u, v) could be deferred like the others but is not (yet).
+// check whose quantity is linear in the circuit size (the FFT and linear layers' weights at the sumcheck point, a general
+// layer's A(u), M(u, v) and constant part, the Lasso subtables at y) is recorded instead of computed. That is sound because no
+// such quantity feeds a later transcript step or challenge: each one only closes its own node's final equality. Where one enters
+// a sumcheck's initial claim (the constant parts, a general layer's A(u) X(u) in phase 2), the replay starts without it and
+// carries the sumcheck's slope into the record, since the final claim is affine in the initial one.
 #pragma once
 #include <algorithm>
 #include <memory>
@@ -128,6 +129,7 @@ template <class FP> class GkrVerifierHost {
     // what the device verifier uploads (verify_batch.cuh)
     int node_kind(int id) const { return nodes_.at(id).kind; }
     bool node_is_linear(int id) const { const Node& n = nodes_.at(id); return n.kind == GKR_VANILLA && n.is_linear; }
+    bool node_is_general(int id) const { const Node& n = nodes_.at(id); return n.kind == GKR_VANILLA && !n.is_linear && !n.is_elemmul; }
     bool node_fft_inverse(int id) const { return nodes_.at(id).fft_inverse; }
     size_t node_out_len(int id) const { return nodes_.at(id).out_len; }
     size_t node_n_in(int id) const { return nodes_.at(id).n_in; }
@@ -278,7 +280,7 @@ template <class FP> class GkrVerifierHost {
             }
         }
         std::vector<X> w;
-        const bool on_host = !defer || (n.kind == GKR_VANILLA && !n.is_linear && !n.is_elemmul);
+        const bool on_host = !defer;
         if (on_host && !n.is_elemmul) {
             w.assign(n.out_len, FP::x_zero());
             X p = FP::x_one();
@@ -288,11 +290,12 @@ template <class FP> class GkrVerifierHost {
                 p = FP::x_mul(p, alpha);
             }
         }
-        auto record = [&](int kind, const std::vector<X>& pt, X factor, X slope, X target, const char* what) {
+        auto record = [&](int kind, const std::vector<X>& pt, X c0, X c1, X c2, X target, const char* what) {
             DeferredCheck<FP> d;
-            d.kind = kind; d.index = id; d.alpha = alpha; d.pt = pt; d.factor = factor; d.slope = slope; d.target = target; d.what = what;
+            d.kind = kind; d.index = id; d.alpha = alpha; d.pt = pt; d.coef[0] = c0; d.coef[1] = c1; d.coef[2] = c2; d.target = target; d.what = what;
             for (auto& c : cl) d.z.push_back(c.point);
             defer->push_back(std::move(d));
+            return &defer->back();
         };
         std::vector<X> pt;
         X fc;
@@ -300,7 +303,7 @@ template <class FP> class GkrVerifierHost {
             verify_sum_check_host<FP>(2, n.log2_size, combined, tr, wo, &fc, &pt);
             const X in_eval = tr.read_felt_ext();
             out.at(0).push_back({pt, in_eval});
-            if (!on_host) { record(DC_FFT, pt, in_eval, FP::x_zero(), fc, "InvalidSumCheck: FFT layer final evaluation mismatch"); return out; }
+            if (!on_host) { record(DC_FFT, pt, in_eval, FP::x_zero(), FP::x_zero(), fc, "InvalidSumCheck: FFT layer final evaluation mismatch"); return out; }
             // A = transform(W), plane by plane
             std::vector<B> plane(n.out_len);
             std::vector<X> A(n.out_len);
@@ -358,7 +361,7 @@ template <class FP> class GkrVerifierHost {
                 x = FP::x_add(x, FP::x_mul(eqhi[k], e));
                 out[k].push_back({lo, e});
             }
-            if (!on_host) { record(DC_LINEAR, pt, x, slope, fc, "InvalidSumCheck: linear layer final evaluation mismatch"); return out; }
+            if (!on_host) { record(DC_LINEAR, pt, x, slope, FP::x_zero(), fc, "InvalidSumCheck: linear layer final evaluation mismatch"); return out; }
             if (!FP::x_eq(FP::x_mul(mle_eval_ext(std::move(A), pt), x), fc)) throw VerifyError("InvalidSumCheck: linear layer final evaluation mismatch");
         } else {  // general layer: phase 1 over x (claim c - const), phase 2 over y (claim fc1 - A(u) X(u)), DESIGN.md section 3 (A11)
             if ((int)n.preds.size() != n.arity) throw VerifyError("Vanilla node arity does not match its connections");
@@ -366,7 +369,7 @@ template <class FP> class GkrVerifierHost {
             const size_t S = n.a_pad * n.n_in, sub = (size_t)1 << n.log2_sub;
             const int nv = log2sz(S), lo_vars = log2sz(n.n_in);
             X constant = FP::x_zero();
-            for (size_t r = 0; r < (size_t)n.num_reps; r++)
+            for (size_t r = 0; on_host && r < (size_t)n.num_reps; r++)
                 for (size_t g = 0; g < n.ng; g++)
                     if (d.has_const[g]) constant = FP::x_add(constant, FP::x_mul_b(w[r * n.ng + g], FP::b_from_limbs(&d.consts[g * FP::B_LIMBS])));
             auto read_evals = [&](const std::vector<X>& p) {  // X(p) = sum_k eq(p_hi, k) X_k(p_lo) from the written X_k(p_lo)
@@ -382,6 +385,18 @@ template <class FP> class GkrVerifierHost {
             };
             std::vector<X> u, v;
             X fc1, fc2;
+            if (!on_host) {
+                // phase 1 starts from `combined` (without C = constant), phase 2 from its final claim (without A(u) xu); with the slopes
+                // s1, s2 the true final claim is fc2 - s2 (s1 C + xu A(u)), so the host check xu M(u, v) xv == that becomes
+                // xu xv M(u, v) + s2 xu A(u) + s1 s2 C == fc2, which has no division and so the same verdict for every proof
+                X s1, s2;
+                verify_sum_check_host<FP>(2, nv, combined, tr, wo, &fc1, &u, &s1);
+                const X xu = read_evals(u);
+                verify_sum_check_host<FP>(2, nv, fc1, tr, wo, &fc2, &v, &s2);
+                const X xv = read_evals(v);
+                record(DC_GENERAL, u, FP::x_mul(s2, xu), FP::x_mul(s1, s2), FP::x_mul(xu, xv), fc2, "InvalidSumCheck: general layer final evaluation mismatch")->v = v;
+                return out;
+            }
             verify_sum_check_host<FP>(2, nv, FP::x_sub(combined, constant), tr, wo, &fc1, &u);
             const X xu = read_evals(u);
             const std::vector<X> equ = eq_table(u);

@@ -18,19 +18,21 @@ struct VerifyError : std::runtime_error {
     explicit VerifyError(const std::string& m) : std::runtime_error(m) {}
 };
 
-// A final check of the replay left to the device: factor * q + slope * q_const == target, where q (and q_const) are linear-size
-// quantities of the circuit fixed by the claim points, alpha and pt.
-//   DC_FFT       q = MLE(transform(W))(pt),  W = sum_t alpha^t eq(z_t, .) over the node's outputs
-//   DC_LINEAR    q = MLE(A)(pt), A = W pushed through the additive edges; q_const = sum_g W[g] const_g (the claim's constant part)
-//   DC_SUBTABLE  q = MLE(subtable `index`)(pt)
-//   DC_INPUT     q = MLE(input node `index`)(pt)
-enum DeferredKind { DC_FFT = 0, DC_LINEAR, DC_SUBTABLE, DC_INPUT };
+// A final check of the replay left to the device: coef[0] q[0] + coef[1] q[1] + coef[2] q[2] == target, where the q[j] are
+// linear-size quantities of the circuit fixed by the claim points, alpha, pt and v (a coefficient is zero where the kind has no q[j]).
+//   DC_FFT       q[0] = MLE(transform(W))(pt),  W = sum_t alpha^t eq(z_t, .) over the node's outputs
+//   DC_LINEAR    q[0] = MLE(A)(pt), A = W pushed through the additive edges; q[1] = sum_g W[g] const_g (the claim's constant part)
+//   DC_GENERAL   q[0] = A(pt) and q[1] as for DC_LINEAR, q[2] = M(pt, v) = sum over the product edges of coef W[out] eq(pt, x) eq(v, y)
+//   DC_SUBTABLE  q[0] = MLE(subtable `index`)(pt)
+//   DC_INPUT     q[0] = MLE(input node `index`)(pt)
+enum DeferredKind { DC_FFT = 0, DC_LINEAR, DC_SUBTABLE, DC_INPUT, DC_GENERAL };
 template <class FP> struct DeferredCheck {
     typedef typename FP::X X;
-    int kind = DC_FFT, index = 0;  // node id (FFT, linear), subtable index, input index
-    std::vector<std::vector<X>> z;  // claim points (FFT, linear)
-    X alpha, factor, slope, target;
-    std::vector<X> pt;
+    int kind = DC_FFT, index = 0;  // node id (FFT, linear, general), subtable index, input index
+    std::vector<std::vector<X>> z;  // claim points (FFT, linear, general)
+    X alpha, target;
+    X coef[3] = {FP::x_zero(), FP::x_zero(), FP::x_zero()};
+    std::vector<X> pt, v;           // v: the general layer's phase-2 point
     const char* what = "";          // the rejection reason when the equality fails
 };
 template <class FP> using DeferredChecks = std::vector<DeferredCheck<FP>>;
@@ -79,7 +81,7 @@ template <class FP> class LassoVerifier {
                 if (defer) {
                     for (int fin = 0; fin < 2; fin++) {
                         DeferredCheck<FP> d;
-                        d.kind = DC_SUBTABLE; d.index = (int)st; d.pt = y; d.factor = FP::lift(gamma); d.slope = FP::x_zero();
+                        d.kind = DC_SUBTABLE; d.index = (int)st; d.pt = y; d.coef[0] = FP::lift(gamma);
                         const X t = fin ? fc_y : FP::x_zero();
                         d.target = FP::x_add(FP::x_sub(FP::x_sub(ify[(fin ? m : 0) + off + i], id_y), FP::x_mul_b(t, gamma2)), FP::lift(tau));
                         d.what = fin ? "verify_memories: final_read_ys mismatch" : "verify_memories: init_ys mismatch";

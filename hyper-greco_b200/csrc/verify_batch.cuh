@@ -2,18 +2,21 @@
 //
 // A batch is B proofs of one circuit. Each proof is replayed on the host by GkrVerifierHost::verify with a DeferredChecks sink
 // (gkr_verify.hpp): every transcript operation and every scalar check runs there, and the final checks whose quantity is linear
-// in the circuit size are left as records factor * q + slope * q_const == target. This file computes the q of all records of
-// the batch on the device and closes them:
+// in the circuit size are left as records sum_j coef[j] * q[j] == target (lasso_verify.hpp). This file computes the q of all
+// records of the batch on the device and closes them:
 //   DC_FFT       W = sum_t alpha^t eq(z_t, .) (k_eq_split_multi + k_eq_accumulate), transform(W) (k_ext_split + NTT + k_ext_merge),
 //                then transform(W) . eq(pt) (k_dot_eq_items over the extension table)
 //   DC_LINEAR    W as above, then one pass over the node's additive edges and constants (k_edge_sum)
+//   DC_GENERAL   W as above, A(u) and the constant part as for DC_LINEAR at pt = u, then one pass over the node's product edges
+//                with eq(u, .) and eq(v, .) (k_mul_edge_sum)
 //   DC_SUBTABLE  subtable . eq(y), the subtables uploaded once by the verifier
 //   DC_INPUT     input table . eq(pt), for every (proof, input, claim)
 // Every stage is one launch over all items. A quantity is keyed by the bytes of what determines it (node, claim points, alpha,
-// point; for inputs also the table), so proofs that carry the same points, as every proof of the library's Keccak256Transcript
-// does, share one W, one transform and one dot. Proofs with their own points get their own (processed in groups that fit the
-// weight pool).
+// point, a general layer's v; for inputs also the table), so proofs that carry the same points, as every proof of the library's
+// Keccak256Transcript does, share one W, one transform, one dot and one edge sum. Proofs with their own points get their own
+// (processed in groups that fit the weight pool).
 #pragma once
+#include <array>
 #include <chrono>
 #include <cstring>
 #include <map>
@@ -82,6 +85,39 @@ template <class FP> __global__ void __launch_bounds__(HG_BLOCK) k_edge_sum(const
     block_reduce_finalize_ex<FP, 2>(acc, it.partials, it.counter, it.out, (unsigned)it.nblk, bid);
 }
 
+// A general layer's product part in one pass over its product edges: out[0] = sum_e coef_e W[out_e] eq(u, x_e) eq(v, y_e) = M(u, v),
+// with x_e, y_e the two factors' positions in the concatenated inputs (num_reps expanded) and eq(u, .), eq(v, .) in two factors each
+template <class FP> struct MulEdgeItem {
+    const u32* out_idx;
+    const u32* x_idx;
+    const u32* y_idx;
+    const typename FP::B* coef;
+    const typename FP::X* w;
+    const typename FP::X* equ_lo;
+    const typename FP::X* equ_hi;
+    const typename FP::X* eqv_lo;
+    const typename FP::X* eqv_hi;
+    typename FP::X* out;
+    typename FP::X* partials;
+    unsigned* counter;
+    u64 n;
+    int lo_bits, blk_start, nblk;
+};
+template <class FP> __global__ void __launch_bounds__(HG_BLOCK) k_mul_edge_sum(const MulEdgeItem<FP>* __restrict__ items, int nitems) {
+    typedef typename FP::X X;
+    const MulEdgeItem<FP> it = items[find_item(items, nitems)];
+    const unsigned bid = blockIdx.x - it.blk_start;
+    const u32 lo_mask = (1u << it.lo_bits) - 1;
+    X acc[1] = {FP::x_zero()};
+    for (size_t e = (size_t)bid * blockDim.x + threadIdx.x; e < it.n; e += (size_t)it.nblk * blockDim.x) {
+        const u32 x = it.x_idx[e], y = it.y_idx[e];
+        const X wc = FP::mul(it.w[it.out_idx[e]], it.coef[e]);
+        const X eu = FP::mul(it.equ_lo[x & lo_mask], it.equ_hi[x >> it.lo_bits]), ev = FP::mul(it.eqv_lo[y & lo_mask], it.eqv_hi[y >> it.lo_bits]);
+        acc[0] = FP::x_add(acc[0], FP::mul(wc, FP::mul(eu, ev)));
+    }
+    block_reduce_finalize_ex<FP, 1>(acc, it.partials, it.counter, it.out, (unsigned)it.nblk, bid);
+}
+
 // Device scratch shared by the stages: descriptor staging through one pinned arena, eq factor pool, partial sums and counters.
 // Everything staged is valid until finish() synchronises the stream.
 template <class FP> class VerifyScratch {
@@ -97,11 +133,11 @@ template <class FP> class VerifyScratch {
         off_ += bytes;
         return r;
     }
-    // sizes every pool for one round of at most `items` reductions, `blocks` reduction blocks (two sums each), `eq` eq-factor
-    // entries and `desc` descriptor bytes; waits for the stream before it replaces a buffer
+    // sizes every pool for one round of at most `items` reductions (three output slots each), `blocks` reduction blocks (two sums
+    // each), `eq` eq-factor entries and `desc` descriptor bytes; waits for the stream before it replaces a buffer
     void reserve(size_t items, size_t blocks, size_t eq, size_t desc) {
         auto grow = [&](auto& b, size_t need) { if (b.n < need) { HG_CUDA(cudaStreamSynchronize(ctx_->stream)); b.alloc(need + need / 2); } };
-        grow(out, 2 * items);
+        grow(out, 3 * items);
         grow(partials, 2 * blocks);
         grow(eq_pool, eq);
         if (counters.n < items) {
@@ -215,14 +251,15 @@ template <class FP> class VerifierDev {
                 pp = desc.node_lasso(id);
             }
             if (desc.node_kind(id) == GKR_FFT) w_total += desc.node_out_len(id);
-            if (!desc.node_is_linear(id)) continue;
+            const bool general = desc.node_is_general(id);
+            if (!desc.node_is_linear(id) && !general) continue;
             w_total += desc.node_out_len(id);
             // the additive edges as (output, concatenated input, coefficient), constants as (gate, HG_EDGE_CONST, const)
             const VanillaDesc& d = *desc.node_desc(id);
             const size_t ng = desc.node_num_gates(id), n_in = desc.node_n_in(id), sub = (size_t)1 << d.log2_sub;
             if (desc.node_in_len(id) > HG_EDGE_CONST || desc.node_out_len(id) > HG_EDGE_CONST) throw std::runtime_error("hg_verifier_new: layer too large");
-            std::vector<u32> out_idx, in_idx;
-            std::vector<B> coef;
+            std::vector<u32> out_idx, in_idx, mul_out, mul_x, mul_y;
+            std::vector<B> coef, mul_coef;
             for (size_t r = 0; r < (size_t)desc.node_num_reps(id); r++)
                 for (size_t g = 0; g < ng; g++) {
                     const u32 o = (u32)(r * ng + g);
@@ -232,11 +269,24 @@ template <class FP> class VerifierDev {
                         in_idx.push_back((u32)((size_t)d.add_in[e] * n_in + r * sub + d.add_wire[e]));
                         coef.push_back(FP::b_from_limbs(&d.add_coef[e * FP::B_LIMBS]));
                     }
+                    // general layers: the product edges as (output, x, y, coefficient)
+                    for (uint64_t e = d.mul_ptr[g]; general && e < d.mul_ptr[g + 1]; e++) {
+                        mul_out.push_back(o);
+                        mul_x.push_back((u32)((size_t)d.mul_in0[e] * n_in + r * sub + d.mul_w0[e]));
+                        mul_y.push_back((u32)((size_t)d.mul_in1[e] * n_in + r * sub + d.mul_w1[e]));
+                        mul_coef.push_back(FP::b_from_limbs(&d.mul_coef[e * FP::B_LIMBS]));
+                    }
                 }
             Edges& E = edges_[id];
             E.n = out_idx.size();
             E.out_idx.alloc(std::max<size_t>(E.n, 1)); E.in_idx.alloc(std::max<size_t>(E.n, 1)); E.coef.alloc(std::max<size_t>(E.n, 1));
             upload(E.out_idx.p, out_idx); upload(E.in_idx.p, in_idx); upload(E.coef.p, coef);
+            if (!general) continue;
+            MulEdges& M = mul_edges_[id];
+            M.n = mul_out.size();
+            M.out_idx.alloc(std::max<size_t>(M.n, 1)); M.x_idx.alloc(std::max<size_t>(M.n, 1)); M.y_idx.alloc(std::max<size_t>(M.n, 1));
+            M.coef.alloc(std::max<size_t>(M.n, 1));
+            upload(M.out_idx.p, mul_out); upload(M.x_idx.p, mul_x); upload(M.y_idx.p, mul_y); upload(M.coef.p, mul_coef);
         }
         if (pp) {  // every subtable, materialised once
             const size_t M = pp->M;
@@ -278,7 +328,7 @@ template <class FP> class VerifierDev {
                         if (((size_t)1 << c.point.size()) != input_lens_[i]) throw VerifyError("verify: input claim point does not match the input's size");
                         DeferredCheck<FP> d;
                         d.kind = DC_INPUT; d.index = (int)(p * input_lens_.size() + i); d.pt = c.point;
-                        d.factor = FP::x_one(); d.slope = FP::x_zero(); d.target = c.value;
+                        d.coef[0] = FP::x_one(); d.target = c.value;
                         d.what = "verify: input claim does not match the input";
                         checks[p].push_back(std::move(d));
                     }
@@ -300,16 +350,17 @@ template <class FP> class VerifierDev {
                 const int idx = d.kind == DC_INPUT ? 0 : d.index;
                 key.append((const char*)&idx, sizeof idx);
                 if (d.kind == DC_INPUT) { const B* t = inputs.at(d.index); key.append((const char*)&t, sizeof t); }
-                if (d.kind == DC_FFT || d.kind == DC_LINEAR) {
+                if (weighted(d.kind)) {
                     key.append((const char*)&d.alpha, sizeof(X));
                     for (auto& z : d.z) { const size_t k = z.size(); key.append((const char*)&k, sizeof k); key.append((const char*)z.data(), k * sizeof(X)); }
                 }
                 key.append((const char*)d.pt.data(), d.pt.size() * sizeof(X));
+                key.append((const char*)d.v.data(), d.v.size() * sizeof(X));  // a general layer's v is as long as its pt: the key stays unambiguous
                 auto it = key_to_q.find(key);
                 if (it == key_to_q.end()) { it = key_to_q.emplace(std::move(key), qs.size()).first; qs.push_back(&d); }
                 q_of[p].push_back(it->second);
             }
-        std::vector<X> q(qs.size()), q_const(qs.size(), FP::x_zero());
+        std::vector<Q> q(qs.size(), Q{FP::x_zero(), FP::x_zero(), FP::x_zero()});
         // table quantities: subtables and inputs
         {
             std::vector<const B*> tabs;
@@ -327,19 +378,19 @@ template <class FP> class VerifierDev {
                 which.push_back(k);
             }
             const std::vector<X> v = mle_eval_items<FP>(ctx_, sc_, tabs, pts);
-            for (size_t i = 0; i < which.size(); i++) q[which[i]] = v[i];
+            for (size_t i = 0; i < which.size(); i++) q[which[i]][0] = v[i];
         }
         // weighted quantities, in groups whose weight tables fit the pool
         std::vector<size_t> group;
         size_t used = 0;
         for (size_t k = 0; k < qs.size(); k++) {
-            if (qs[k]->kind != DC_FFT && qs[k]->kind != DC_LINEAR) continue;
+            if (!weighted(qs[k]->kind)) continue;
             const size_t need = desc_.node_out_len(qs[k]->index);
-            if (used + need > w_pool_.n) { run_weighted(qs, group, q, q_const); group.clear(); used = 0; }
+            if (used + need > w_pool_.n) { run_weighted(qs, group, q); group.clear(); used = 0; }
             group.push_back(k);
             used += need;
         }
-        if (!group.empty()) run_weighted(qs, group, q, q_const);
+        if (!group.empty()) run_weighted(qs, group, q);
         const Clock::time_point t2 = Clock::now();
         // close every record
         for (size_t p = 0; p < np; p++) {
@@ -347,7 +398,8 @@ template <class FP> class VerifierDev {
             for (size_t r = 0; r < checks[p].size(); r++) {
                 const DeferredCheck<FP>& d = checks[p][r];
                 const size_t k = q_of[p][r];
-                const X lhs = FP::x_add(FP::x_mul(d.factor, q[k]), FP::x_mul(d.slope, q_const[k]));
+                X lhs = FP::x_zero();
+                for (int j = 0; j < 3; j++) lhs = FP::x_add(lhs, FP::x_mul(d.coef[j], q[k][j]));
                 if (!FP::x_eq(lhs, d.target)) { res[p].ok = false; res[p].reason = d.what; break; }
             }
         }
@@ -356,7 +408,10 @@ template <class FP> class VerifierDev {
     }
 
   private:
+    typedef std::array<X, 3> Q;  // the q[j] of one quantity
     struct Edges { DevBuf<u32> out_idx, in_idx; DevBuf<B> coef; size_t n = 0; };
+    struct MulEdges { DevBuf<u32> out_idx, x_idx, y_idx; DevBuf<B> coef; size_t n = 0; };
+    static bool weighted(int kind) { return kind == DC_FFT || kind == DC_LINEAR || kind == DC_GENERAL; }
     static int eq_lo_bits(size_t nv) { return (int)std::min<size_t>(nv, 12); }
     template <class T> void upload(T* dst, const std::vector<T>& v) {
         if (v.empty()) return;
@@ -364,27 +419,29 @@ template <class FP> class VerifierDev {
         HG_CUDA(cudaStreamSynchronize(ctx_->stream));  // v is the caller's temporary
     }
 
-    // W of every quantity in `group`, the FFT transforms, then the dots (FFT) and edge sums (linear)
-    void run_weighted(const std::vector<const DeferredCheck<FP>*>& qs, const std::vector<size_t>& group, std::vector<X>& q, std::vector<X>& q_const) {
+    // W of every quantity in `group`, the FFT transforms, then the dots (FFT), edge sums (linear, general) and product-edge sums
+    // (general); quantity g's results go to output slots 3g .. 3g + 2, its q[0 .. 2]
+    void run_weighted(const std::vector<const DeferredCheck<FP>*>& qs, const std::vector<size_t>& group, std::vector<Q>& q) {
         cudaStream_t s = ctx_->stream;
-        // eq factors: per quantity, the claim factors back to back (stride nlo + nhi), then the factors of pt
-        size_t eq_need = 0, pt_elems = 0, blocks = 0, n_claims = 0;
+        // eq factors: per quantity, the claim factors back to back (stride nlo + nhi), then the factors of pt (and of v)
+        size_t eq_need = 0, pt_elems = 0, blocks = 0, n_splits = 0;
         for (size_t k : group) {
             const DeferredCheck<FP>& d = *qs[k];
-            const size_t nvw = d.z.at(0).size(), lo = eq_lo_bits(nvw), nv = d.pt.size(), lp = eq_lo_bits(nv);
-            eq_need += d.z.size() * (((size_t)1 << lo) + ((size_t)1 << (nvw - lo))) + ((size_t)1 << lp) + ((size_t)1 << (nv - lp));
-            pt_elems += d.z.size() * nvw + nv + 1;
-            n_claims += d.z.size();
-            blocks += 2 * (size_t)ctx_->sm_count;
+            const size_t nvw = d.z.at(0).size(), lo = eq_lo_bits(nvw), nv = d.pt.size(), lp = eq_lo_bits(nv), npts = d.v.empty() ? 1 : 2;
+            eq_need += d.z.size() * (((size_t)1 << lo) + ((size_t)1 << (nvw - lo))) + npts * (((size_t)1 << lp) + ((size_t)1 << (nv - lp)));
+            pt_elems += d.z.size() * nvw + npts * nv + 1;
+            n_splits += d.z.size() + npts;
+            blocks += 2 * npts * (size_t)ctx_->sm_count;
         }
         sc_.reserve(group.size(), blocks, eq_need,
-                    (n_claims + group.size()) * sizeof(EqSplitItem<FP>) + group.size() * (sizeof(EqAccItem<FP>) + sizeof(EdgeItem<FP>) + sizeof(DotItem<FP, X>) + 2 * sizeof(X*)) +
+                    n_splits * sizeof(EqSplitItem<FP>) +
+                        group.size() * (sizeof(EqAccItem<FP>) + sizeof(EdgeItem<FP>) + sizeof(MulEdgeItem<FP>) + sizeof(DotItem<FP, X>) + 2 * sizeof(X*)) +
                         pt_elems * sizeof(X) + 4096);
         std::vector<X> flat;  // alphas and points, staged once all items know their offsets
         const X* d_pts = nullptr;
         std::vector<EqSplitItem<FP>> splits;
         std::vector<EqAccItem<FP>> accs;
-        struct Ref { X* w; X* plo; X* phi; int lp; };
+        struct Ref { X* w; X* plo; X* phi; X* vlo; X* vhi; int lp; };
         std::vector<Ref> refs;
         size_t eoff = 0, woff = 0;
         int split_blk = 0, acc_blk = 0;
@@ -418,11 +475,19 @@ template <class FP> class VerifierDev {
             ai.blk_start = acc_blk;
             acc_blk += (int)((out_len + HG_BLOCK * HG_EQACC_PER_THREAD - 1) / (HG_BLOCK * HG_EQACC_PER_THREAD));
             accs.push_back(ai);
-            const size_t off = flat.size();
-            flat.insert(flat.end(), d.pt.begin(), d.pt.end());
             const int lp = eq_lo_bits(d.pt.size());
-            const EqSplitItem<FP> sp = split(off, (int)d.pt.size(), lp, std::string::npos, 0);
-            refs.push_back({w_pool_.p + woff, sp.eq_lo, sp.eq_hi, lp});
+            auto point = [&](const std::vector<X>& p) {
+                const size_t off = flat.size();
+                flat.insert(flat.end(), p.begin(), p.end());
+                return split(off, (int)p.size(), lp, std::string::npos, 0);
+            };
+            const EqSplitItem<FP> sp = point(d.pt);
+            Ref r = {w_pool_.p + woff, sp.eq_lo, sp.eq_hi, nullptr, nullptr, lp};
+            if (d.kind == DC_GENERAL) {  // u and v: both phases run over the same S entries
+                const EqSplitItem<FP> sv = point(d.v);
+                r.vlo = sv.eq_lo; r.vhi = sv.eq_hi;
+            }
+            refs.push_back(r);
             woff += out_len;
         }
         d_pts = sc_.stage(flat);
@@ -449,35 +514,47 @@ template <class FP> class VerifierDev {
         }
         std::vector<DotItem<FP, X>> dots;
         std::vector<EdgeItem<FP>> edges;
-        int dot_blk = 0, edge_blk = 0;
-        size_t dot_bytes = 0, edge_bytes = 0, pblk = 0;
+        std::vector<MulEdgeItem<FP>> muls;
+        int dot_blk = 0, edge_blk = 0, mul_blk = 0;
+        size_t dot_bytes = 0, edge_bytes = 0, mul_bytes = 0, pblk = 0;
+        auto edge_blocks = [&](size_t n) { return (int)std::max<size_t>(1, std::min<size_t>((n + HG_BLOCK * 8 - 1) / (HG_BLOCK * 8), 2 * (size_t)ctx_->sm_count)); };
         for (size_t g = 0; g < group.size(); g++) {
             const DeferredCheck<FP>& d = *qs[group[g]];
             const Ref& r = refs[g];
             if (d.kind == DC_FFT) {
                 DotItem<FP, X> it;
-                it.t = r.w; it.eq_lo = r.plo; it.eq_hi = r.phi; it.out = sc_.out.p + 2 * g; it.partials = sc_.partials.p + 2 * pblk; it.counter = sc_.counters.p + g;
+                it.t = r.w; it.eq_lo = r.plo; it.eq_hi = r.phi; it.out = sc_.out.p + 3 * g; it.partials = sc_.partials.p + 2 * pblk; it.counter = sc_.counters.p + g;
                 it.n = desc_.node_out_len(d.index); it.lo_bits = r.lp; it.blk_start = dot_blk;
                 it.nblk = (int)std::min<size_t>(it.n >> r.lp, (size_t)ctx_->sm_count);
                 dot_blk += it.nblk; pblk += it.nblk; dot_bytes += it.n * sizeof(X);
                 dots.push_back(it);
-            } else {
-                const Edges& E = edges_.at(d.index);
-                EdgeItem<FP> it;
-                it.out_idx = E.out_idx.p; it.in_idx = E.in_idx.p; it.coef = E.coef.p; it.w = r.w; it.eq_lo = r.plo; it.eq_hi = r.phi;
-                it.out = sc_.out.p + 2 * g; it.partials = sc_.partials.p + 2 * pblk; it.counter = sc_.counters.p + g;
-                it.n = E.n; it.lo_bits = r.lp; it.blk_start = edge_blk;
-                it.nblk = (int)std::max<size_t>(1, std::min<size_t>((E.n + HG_BLOCK * 8 - 1) / (HG_BLOCK * 8), 2 * (size_t)ctx_->sm_count));
-                edge_blk += it.nblk; pblk += it.nblk; edge_bytes += E.n * (2 * sizeof(u32) + sizeof(B) + sizeof(X));
-                edges.push_back(it);
+                continue;
             }
+            const Edges& E = edges_.at(d.index);
+            EdgeItem<FP> it;
+            it.out_idx = E.out_idx.p; it.in_idx = E.in_idx.p; it.coef = E.coef.p; it.w = r.w; it.eq_lo = r.plo; it.eq_hi = r.phi;
+            it.out = sc_.out.p + 3 * g; it.partials = sc_.partials.p + 2 * pblk; it.counter = sc_.counters.p + g;
+            it.n = E.n; it.lo_bits = r.lp; it.blk_start = edge_blk; it.nblk = edge_blocks(E.n);
+            edge_blk += it.nblk; pblk += it.nblk; edge_bytes += E.n * (2 * sizeof(u32) + sizeof(B) + sizeof(X));
+            edges.push_back(it);
+            if (d.kind != DC_GENERAL) continue;
+            // counter g again: k_edge_sum has returned it to 0 before k_mul_edge_sum starts on the same stream
+            const MulEdges& M = mul_edges_.at(d.index);
+            MulEdgeItem<FP> mt;
+            mt.out_idx = M.out_idx.p; mt.x_idx = M.x_idx.p; mt.y_idx = M.y_idx.p; mt.coef = M.coef.p; mt.w = r.w;
+            mt.equ_lo = r.plo; mt.equ_hi = r.phi; mt.eqv_lo = r.vlo; mt.eqv_hi = r.vhi;
+            mt.out = sc_.out.p + 3 * g + 2; mt.partials = sc_.partials.p + 2 * pblk; mt.counter = sc_.counters.p + g;
+            mt.n = M.n; mt.lo_bits = r.lp; mt.blk_start = mul_blk; mt.nblk = edge_blocks(M.n);
+            mul_blk += mt.nblk; pblk += mt.nblk; mul_bytes += M.n * (3 * sizeof(u32) + sizeof(B) + sizeof(X));
+            muls.push_back(mt);
         }
         if (!dots.empty()) HG_K(ctx_, KC_DOT, dot_bytes, k_dot_eq_items<FP, X><<<dot_blk, HG_BLOCK, 0, s>>>(sc_.stage(dots), (int)dots.size()));
         if (!edges.empty()) HG_K(ctx_, KC_GKR_PREP, edge_bytes, k_edge_sum<FP><<<edge_blk, HG_BLOCK, 0, s>>>(sc_.stage(edges), (int)edges.size()));
-        sc_.finish(2 * group.size());
+        if (!muls.empty()) HG_K(ctx_, KC_GKR_PREP, mul_bytes, k_mul_edge_sum<FP><<<mul_blk, HG_BLOCK, 0, s>>>(sc_.stage(muls), (int)muls.size()));
+        sc_.finish(3 * group.size());
         for (size_t g = 0; g < group.size(); g++) {
-            q[group[g]] = sc_.h_out.p[2 * g];
-            if (qs[group[g]]->kind == DC_LINEAR) q_const[group[g]] = sc_.h_out.p[2 * g + 1];
+            const int kind = qs[group[g]]->kind, slots = kind == DC_FFT ? 1 : kind == DC_LINEAR ? 2 : 3;
+            for (int j = 0; j < slots; j++) q[group[g]][j] = sc_.h_out.p[3 * g + j];
         }
     }
 
@@ -487,7 +564,8 @@ template <class FP> class VerifierDev {
     size_t max_batch_;
     VerifyScratch<FP> sc_;
     std::vector<size_t> input_lens_;
-    std::map<int, Edges> edges_;
+    std::map<int, Edges> edges_;          // linear and general layers
+    std::map<int, MulEdges> mul_edges_;   // general layers
     DevBuf<B> subtables_;
     size_t subtable_len_ = 0;
     double timing_us_[3] = {0, 0, 0};

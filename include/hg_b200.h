@@ -308,13 +308,13 @@ int hg_gkr_verify(hg_circuit* c, size_t n_output_claims, const size_t* point_len
 int hg_mle_eval_host(int field_id, const uint64_t* table_limbs, size_t n, size_t num_vars, const uint64_t* point_ext, uint64_t* out_ext);
 /* ---- batched verifier on the device: B proofs of one circuit per call.
  *      hg_verifier_new takes a host-only description (hg_circuit_new_host + hg_bfv_configure or the insert / connect calls) of the
- *      context's field, uploads its wiring (edges and constants of the linear layers) and its Lasso subtables once, and serves
- *      batches of up to max_batch proofs. At most one Lasso node per circuit.
+ *      context's field, uploads its wiring (edges and constants of the linear and general layers, the product edges of the general
+ *      layers) and its Lasso subtables once, and serves batches of up to max_batch proofs. At most one Lasso node per circuit.
  *      hg_gkr_verify_batch verifies n_proofs proofs: each is replayed on the host exactly as hg_gkr_verify does (every transcript
  *      operation and scalar check), the checks whose cost is linear in the circuit size (FFT and linear layers at the sumcheck
- *      point, Lasso subtables, every input claim) are evaluated on the device for the whole batch, and quantities that several
- *      proofs share (the same points, as with hg_transcript_new / hg_transcript_from_proof) are computed once. General layers
- *      are checked on the host. It is hg_gkr_verify followed by the input-claim comparison of :512-516, with the same verdict.
+ *      point, general layers at their two points, Lasso subtables, every input claim) are evaluated on the device for the whole
+ *      batch, and quantities that several proofs share (the same points, as with hg_transcript_new / hg_transcript_from_proof)
+ *      are computed once. It is hg_gkr_verify followed by the input-claim comparison of :512-516, with the same verdict.
  *        transcripts[p]      proof p's transcript (hg_transcript_from_proof, or a caller-owned one with a read callback), read as
  *                            hg_gkr_verify reads it; the caller can check for trailing bytes afterwards
  *        output claims       n_output_claims per proof with the same point_lens for every proof; proof p's points start at
