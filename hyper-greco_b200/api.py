@@ -34,6 +34,7 @@ SYMBOLS = [
     "hg_lasso_node_num_chunks", "hg_lasso_node_timing", "hg_lasso_node_shard_words", "hg_lasso_node_prove_shard", "hg_lasso_node_emit_shard",
     "hg_shard_merge", "hg_lasso_node_prove_shard_dev", "hg_lasso_node_emit_shard_dev", "hg_shard_merge_device", "hg_gkr_shard_words", "hg_gkr_prove_shard_dev", "hg_gkr_emit_shard_dev", "hg_gkr_emit_shard_part_dev", "hg_transcript_append_bytes",
     "hg_circuit_new_host", "hg_circuit_insert_lasso_host", "hg_gkr_verify", "hg_mle_eval_host", "hg_bfv_witness_generate", "hg_lasso_node_verify", "hg_sumcheck_prove", "hg_mle_eval_batch", "hg_ntt", "hg_bfv_configure", "hg_field_selftest",
+    "hg_bfv_pk_configure", "hg_bfv_pk_witness_generate",
     "hg_circuit_new", "hg_circuit_free", "hg_circuit_insert_input", "hg_circuit_insert_fft", "hg_circuit_insert_lasso", "hg_circuit_insert_vanilla",
     "hg_circuit_connect", "hg_circuit_evaluate", "hg_circuit_evaluate_host", "hg_circuit_node_value", "hg_gkr_prove", "hg_gkr_timing", "hg_gkr_num_challenges", "hg_gkr_num_inputs", "hg_gkr_num_input_claims",
     "hg_gkr_input_claim_num_vars", "hg_gkr_input_claim", "hg_verifier_new", "hg_verifier_free", "hg_gkr_verify_batch", "hg_verifier_reason", "hg_mle_eval_multi",
@@ -182,6 +183,8 @@ def lib():
         L.hg_gkr_input_claim_num_vars.restype = sz
         L.hg_gkr_input_claim.argtypes = [vp, sz, sz, vp, vp]
         L.hg_bfv_configure.argtypes = [vp, sz, sz, vp, vp, vp, vp, u64, u64, u64, vp, vp, sz, vp]
+        L.hg_bfv_pk_configure.argtypes = [vp, sz, sz, vp, vp, vp, vp, vp, vp, u64, u64, u64, vp, vp, sz, vp]
+        L.hg_bfv_pk_witness_generate.argtypes = [vp, sz, sz] + [vp] * 24
         _lib = L
     return _lib
 
@@ -1276,3 +1279,142 @@ class BfvSkEncryptProver:
         el = point.shape[1]
         claims = self.circuit.prove_gkr([(np.zeros((0, el), np.uint64), np.zeros(el, np.uint64)), (point, value)], tr, mode)   # :450-457
         return tr.into_proof(), claims                                                           # :459
+
+
+# ------------------------------------------------------------------------------------------------ BFV public-key encryption
+def build_bfv_pk_circuit(c: Circuit, P, lasso_node=None, lasso_pp=None, lasso_num_vars=0):
+    """The circuit of the BFV public-key-encryption relation (params.BfvPkEncryptConstants) through hg_bfv_pk_configure, for a device
+    circuit (prover: lasso_node) or a host-only description (verifier: lasso_pp + num_vars). Returns the ids of a few nodes."""
+    K = P.K
+    u = lambda v: np.ascontiguousarray(np.array(v[:K], dtype=np.uint64))
+    ids = np.zeros(8, np.int32)
+    _chk(lib().hg_bfv_pk_configure(c.h, P.log2_size, K, _p(u(P.QIS)), _p(u(P.K0IS)), _p(u(P.R1_BOUNDS)), _p(u(P.R2_BOUNDS)), _p(u(P.P1_BOUNDS)),
+                                   _p(u(P.P2_BOUNDS)), P.U_BOUND, P.E_BOUND, P.K1_BOUND, lasso_node.h if lasso_node is not None else None,
+                                   lasso_pp.h if lasso_pp is not None else None, lasso_num_vars, _p(ids)))
+    c._keep.extend([x for x in (lasso_node, lasso_pp) if x is not None])
+    return dict(zip(("u", "e0", "e1", "k1", "lasso_in", "lasso", "sum0", "sum1"), (int(x) for x in ids)))
+
+
+def _pk_output_claims(point0, v0, point1, v1):
+    """the Lasso node's empty claim, then sum0 = ct0is at point0 and sum1 = ct1is at point1"""
+    el = point0.shape[1]
+    return [(np.zeros((0, el), np.uint64), np.zeros(el, np.uint64)), (point0, v0), (point1, v1)]
+
+
+class BfvPkEncryptProver:
+    """Proves the BFV public-key-encryption relation with every table on the device. A proof: a fresh transcript, circuit.evaluate,
+    point0 (L + log2 K challenges) and v0 = MLE(ct0is)(point0), point1 and v1 = MLE(ct1is)(point1) the same way, prove_gkr with the
+    output claims [(), 0], [point0, v0], [point1, v1] (the Lasso node, sum0, sum1)."""
+
+    def __init__(self, ctx: Context, params):
+        from . import witness
+        P = self.P = params
+        self.ctx = ctx
+        self.pp = LassoPreprocessing.preprocess(witness.pk_lasso_lookup_bounds(P))
+        self.lasso = LassoNode(ctx, self.pp, witness.pk_lasso_num_vars(P), witness.pk_lasso_lookup_segments(P))
+        c = self.circuit = Circuit(ctx)
+        self.ids = build_bfv_pk_circuit(c, P, lasso_node=self.lasso)
+        self.ct_log2_size = P.log2_size + (P.K.bit_length() - 1)
+
+    def upload_inputs(self, ins):
+        """pk_get_inputs' dict -> device buffers in input-node order"""
+        from . import witness
+        return [DeviceBuffer.from_numpy(self.ctx, np.asarray(v, dtype=np.uint64).reshape(-1)) for v in witness.pk_input_list(ins)]
+
+    def _prove(self, d_ct0is, d_ct1is, mode, transcript):
+        tr = Keccak256Transcript(self.ctx.field) if transcript is None else transcript
+        L = self.ct_log2_size
+        point0 = tr.squeeze_challenges(L)
+        v0 = mle_eval_batch(self.ctx, d_ct0is, 1, L, point0)[0]
+        point1 = tr.squeeze_challenges(L)
+        v1 = mle_eval_batch(self.ctx, d_ct1is, 1, L, point1)[0]
+        claims = self.circuit.prove_gkr(_pk_output_claims(point0, v0, point1, v1), tr, mode)
+        return tr.into_proof(), claims
+
+    def prove(self, dev_inputs, d_ct0is, d_ct1is, mode=MODE_PREFETCH, transcript=None):
+        """dev_inputs in input-node order, d_ct0is / d_ct1is device buffers in the library's representation (as
+        hg_bfv_pk_witness_generate writes them). transcript: a fresh one by default, or a caller-owned CallbackTranscript.
+        Returns (proof bytes, input claims)."""
+        self.circuit.evaluate(dev_inputs)
+        return self._prove(d_ct0is, d_ct1is, mode, transcript)
+
+    def prove_host(self, host_inputs, host_ct0is, host_ct1is, mode=MODE_PREFETCH, transcript=None):
+        """prove() from HOST vectors of canonical limbs (input-node order; ct0is and ct1is concatenated over the moduli)."""
+        cts = [np.ascontiguousarray(c, np.uint64).reshape(-1) for c in (host_ct0is, host_ct1is)]
+        if getattr(self, "_d_ct", None) is None or self._d_ct[0].nbytes != cts[0].nbytes:
+            self._d_ct = [DeviceBuffer(self.ctx, cts[0].nbytes) for _ in range(2)]
+        self.circuit.evaluate_host(host_inputs)
+        for d, c in zip(self._d_ct, cts):
+            d.upload(c)
+            if self.ctx.field == BN254:
+                _chk(lib().hg_field_encode(self.ctx.h, d.ptr, c.size // LIMBS[BN254]))
+        return self._prove(self._d_ct[0], self._d_ct[1], mode, transcript)
+
+
+class BfvPkEncryptVerifier:
+    """Verifies proofs of BfvPkEncryptProver on the HOST (verify: no GPU, no context) or in batches on a device (verify_batch)."""
+
+    def __init__(self, params, field=GOLDILOCKS):
+        from . import witness
+        self.P, self.field = params, field
+        self.pp = LassoPreprocessing.preprocess(witness.pk_lasso_lookup_bounds(params))
+        self.circuit = Circuit(None, field)
+        self.ids = build_bfv_pk_circuit(self.circuit, params, lasso_pp=self.pp, lasso_num_vars=witness.pk_lasso_num_vars(params))
+        self.ct_log2_size = params.log2_size + (params.K.bit_length() - 1)
+        self._el_bytes = 8 * LIMBS[field] * DEGREE[field]   # a proof is whole extension elements: a shorter tail is trailing bytes
+
+    def verify(self, host_inputs, host_ct0is, host_ct1is, proof: bytes, options=None):
+        """host_inputs in input-node order as canonical limbs. Raises HgError if the proof is rejected; returns the input claims."""
+        if len(proof) % self._el_bytes:
+            raise HgError("verify: trailing bytes in proof")
+        tr = Keccak256Transcript.from_proof(proof, self.field)
+        L = self.ct_log2_size
+        point0 = tr.squeeze_challenges(L)
+        v0 = mle_eval_host(self.field, host_ct0is, L, point0)
+        point1 = tr.squeeze_challenges(L)
+        v1 = mle_eval_host(self.field, host_ct1is, L, point1)
+        claims = self.circuit.verify_gkr(_pk_output_claims(point0, v0, point1, v1), tr, options)
+        if len(claims) != len(host_inputs):
+            raise HgError("verify: input count mismatch")
+        for vec, cl in zip(host_inputs, claims):
+            for pt, v in cl:
+                if not (mle_eval_host(self.field, vec, pt.shape[0], pt) == v).all():
+                    raise HgError("verify: input claim does not match the input")
+        try:
+            tr.read_felt_ext()
+        except HgError:
+            return claims
+        raise HgError("verify: trailing bytes in proof")
+
+    def verify_batch(self, ctx: Context, inputs_list, ct0is_list, ct1is_list, proofs, options=None):
+        """verify() for a batch of proofs on the device of `ctx` (GkrBatchVerifier), with the same verdicts. inputs_list[p], ct0is_list[p]
+        and ct1is_list[p] belong to proof p: host numpy arrays of canonical limbs, or device buffers in the library's representation.
+        proofs are bytes, or transcripts positioned at the start of the proof. Returns [(ok, reason)] per proof."""
+        n = len(proofs)
+        if n == 0:
+            return []
+        bv = getattr(self, "_batch", None)
+        if bv is None or bv.ctx is not ctx or bv.max_batch < n:
+            if bv is not None:
+                bv.free()
+            bv = self._batch = GkrBatchVerifier(ctx, self.circuit, n)
+        trs = [Keccak256Transcript.from_proof(p, self.field) if isinstance(p, (bytes, bytearray)) else p for p in proofs]
+        L = self.ct_log2_size
+        points = []
+        for t in trs:
+            points += [t.squeeze_challenges(L), t.squeeze_challenges(L)]
+        tables = [c for pair in zip(ct0is_list, ct1is_list) for c in pair]
+        values = mle_eval_multi(ctx, tables, points)
+        oc = [_pk_output_claims(points[2 * p], values[2 * p], points[2 * p + 1], values[2 * p + 1]) for p in range(n)]
+        res = bv.verify_batch(trs, oc, inputs_list, options)
+        out = []
+        for t, pr, (ok, why) in zip(trs, proofs, res):
+            if ok:
+                try:
+                    t.read_felt_ext()
+                    ok, why = False, "verify: trailing bytes in proof"
+                except HgError:
+                    if isinstance(pr, (bytes, bytearray)) and len(pr) % self._el_bytes:
+                        ok, why = False, "verify: trailing bytes in proof"
+            out.append((ok, why))
+        return out

@@ -84,6 +84,11 @@ template <class FP> struct FieldState {
     DevBuf<long long> wg_a;
     DevBuf<i128> wg_hat;
     DevBuf<WitGenStatus> wg_st;
+    // hg_bfv_pk_witness_generate: u, e0, k1, pk0 and hat0 in the buffers above, the second component here
+    DevBuf<signed char> wg_e1;
+    DevBuf<long long> wg_pk1;
+    DevBuf<i128> wg_hat1;
+    DevBuf<WitGenPkStatus> wg_pk_st;
     // hg_mle_eval_batch
     DevBuf<X> mle_pt, mle_eq, mle_partials, mle_out;
     DevBuf<unsigned> mle_counters;
@@ -475,6 +480,78 @@ template <class FP> void witness_generate(hg_ctx* ctx, size_t n, size_t K, const
         throw std::runtime_error("hg_bfv_witness_generate: assertion of circuit_sk.py failed: " + std::to_string(hs.not_multiple_of_cyclo) + " coefficients not a multiple of x^n+1, " +
                                  std::to_string(hs.not_multiple_of_q) + " not divisible by q_i, " + std::to_string(hs.r1_out_of_range) + " r1 out of range, " +
                                  std::to_string(hs.r2_out_of_range) + " r2 out of range");
+}
+
+// hg_bfv_pk_witness_generate: the public-key relation's witness on the device (witness_gen.cuh, k_wit_pk_*). Small host inputs,
+// device outputs in the library's representation.
+template <class FP> void pk_witness_generate(hg_ctx* ctx, size_t n, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1b, const uint64_t* r2b,
+                                             const uint64_t* p1b, const uint64_t* p2b, const int8_t* u, const int8_t* e0, const int8_t* e1, const int32_t* k1,
+                                             const int64_t* pk0, const int64_t* pk1, void* const* d_out) {
+    typedef typename FP::B B;
+    DeviceCtx* dev = &ctx->dev;
+    FieldState<FP>& fs = typed<FP>(ctx);
+    if (n < 2 || (n & (n - 1)) || K < 1 || K > 64) throw std::runtime_error("hg_bfv_pk_witness_generate: n must be a power of two >= 2 and 1 <= K <= 64");
+    WitGenPkParams P;
+    memset(&P, 0, sizeof P);
+    P.n = (int)n; P.K = (int)K;
+    for (size_t i = 0; i < K; i++) {
+        if (qis[i] >= ((uint64_t)1 << 62) || qis[i] < 3) throw std::runtime_error("hg_bfv_pk_witness_generate: modulus out of range");
+        P.q[i] = (long long)qis[i]; P.k0[i] = (long long)k0is[i];
+        P.q1_bound[0][i] = (long long)r1b[i]; P.q2_bound[0][i] = (long long)r2b[i]; P.q1_bound[1][i] = (long long)p1b[i]; P.q2_bound[1][i] = (long long)p2b[i];
+    }
+    // what the 64-bit partial sums of k_wit_pk_conv rely on: u ternary, |pk| < 2^59
+    for (size_t j = 0; j < n; j++) if (u[j] < -1 || u[j] > 1) throw std::runtime_error("hg_bfv_pk_witness_generate: u must be ternary");
+    for (size_t j = 0; j < K * n; j++)
+        if (pk0[j] <= -(1LL << 59) || pk0[j] >= (1LL << 59) || pk1[j] <= -(1LL << 59) || pk1[j] >= (1LL << 59))
+            throw std::runtime_error("hg_bfv_pk_witness_generate: a public-key coefficient is not below 2^59 in magnitude");
+    {   // p as canonical limbs: the limbs of -1 plus one
+        B m1 = FP::b_sub(FP::b_zero(), FP::b_one());
+        u64 l[4] = {0, 0, 0, 0};
+        FP::b_to_limbs(m1, l);
+        u64 c = 1;
+        for (int q = 0; q < 4; q++) { const u64 v = l[q] + c; c = (v < l[q]) ? 1 : 0; P.p[q] = v; }
+    }
+    cudaStream_t st = dev->stream;
+    auto grow = [&](auto& buf, size_t need) { if (buf.n < need) { HG_CUDA(cudaStreamSynchronize(st)); buf.alloc(need); } };
+    grow(fs.wg_s, n); grow(fs.wg_e, n); grow(fs.wg_e1, n); grow(fs.wg_k1, n); grow(fs.wg_a, K * n); grow(fs.wg_pk1, K * n);
+    grow(fs.wg_hat, K * 2 * n); grow(fs.wg_hat1, K * 2 * n); grow(fs.wg_pk_st, 1);
+    HG_CUDA(cudaMemcpyAsync(fs.wg_s.p, u, n, cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemcpyAsync(fs.wg_e.p, e0, n, cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemcpyAsync(fs.wg_e1.p, e1, n, cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemcpyAsync(fs.wg_k1.p, k1, n * sizeof(int), cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemcpyAsync(fs.wg_a.p, pk0, K * n * sizeof(long long), cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemcpyAsync(fs.wg_pk1.p, pk1, K * n * sizeof(long long), cudaMemcpyHostToDevice, st));
+    HG_CUDA(cudaMemsetAsync(fs.wg_pk_st.p, 0, sizeof(WitGenPkStatus), st));
+    const size_t N2 = 2 * n;
+    HG_K(dev, KC_MISC, 2 * K * n * 8 + 2 * K * N2 * 16,
+         k_wit_pk_conv<<<dim3((unsigned)((N2 + HG_WIT_KT - 1) / HG_WIT_KT), (unsigned)K), HG_WIT_KT, 0, st>>>(fs.wg_s.p, fs.wg_a.p, fs.wg_pk1.p, (int)n, fs.wg_hat.p, fs.wg_hat1.p));
+    constexpr int L = FP::B_LIMBS;
+    u64* const* o = (u64* const*)d_out;  // u, e0, e1, k1, pk0is, pk1is, r1is, p1is, r2is, p2is, ct0is, ct1is
+    HG_K(dev, KC_MISC, 2 * K * N2 * (16 + 3 * 8 * L),
+         k_wit_pk_finish<L><<<dim3((unsigned)((N2 + 255) / 256), (unsigned)K), 256, 0, st>>>(P, fs.wg_e.p, fs.wg_e1.p, fs.wg_k1.p, fs.wg_a.p, fs.wg_pk1.p, fs.wg_hat.p,
+                                                                                         fs.wg_hat1.p, o[4], o[5], o[6], o[7], o[8], o[9], o[10], o[11], fs.wg_pk_st.p));
+    HG_K(dev, KC_MISC, N2 * 4 * 8 * L,
+         k_wit_pk_small<L><<<(unsigned)((N2 + 255) / 256), 256, 0, st>>>(P, fs.wg_s.p, fs.wg_e.p, fs.wg_e1.p, fs.wg_k1.p, o[0], o[1], o[2], o[3]));
+    if (FP::FIELD_ID == 1) {  // canonical limbs -> Montgomery form
+        auto enc = [&](void* p, size_t cnt) { k_field_encode<FP><<<(unsigned)((cnt + 255) / 256), 256, 0, st>>>((B*)p, cnt, 0); HG_LAUNCH_CHECK(); };
+        for (int b = 0; b < 4; b++) enc(o[b], N2);
+        for (int b = 4; b < 8; b++) enc(o[b], K * N2);
+        enc(o[8], K * n); enc(o[9], K * n); enc(o[10], K * N2); enc(o[11], K * N2);
+    }
+    WitGenPkStatus hs;
+    HG_CUDA(cudaMemcpyAsync(&hs, fs.wg_pk_st.p, sizeof hs, cudaMemcpyDeviceToHost, st));
+    HG_CUDA(cudaStreamSynchronize(st));  // also keeps the caller's host arrays alive long enough
+    std::string why;
+    const char* names[2][3] = {{"ct0", "r1", "r2"}, {"ct1", "p1", "p2"}};
+    for (int c = 0; c < 2; c++) {
+        const WitGenStatus& s = hs.c[c];
+        auto add = [&](unsigned cnt, const std::string& what) { if (cnt) why += std::string(why.empty() ? "" : ", ") + names[c][0] + ": " + std::to_string(cnt) + " " + what; };
+        add(s.not_multiple_of_cyclo, "coefficients not a multiple of x^n+1");
+        add(s.not_multiple_of_q, "coefficients not divisible by q_i");
+        add(s.r1_out_of_range, std::string(names[c][1]) + " coefficients out of range");
+        add(s.r2_out_of_range, std::string(names[c][2]) + " coefficients out of range");
+    }
+    if (!why.empty()) throw std::runtime_error("hg_bfv_pk_witness_generate: the witness does not satisfy the relation: " + why);
 }
 
 // hg_field_selftest
@@ -1000,6 +1077,32 @@ int hg_bfv_configure(hg_circuit* c, size_t log2_size, size_t K, const uint64_t* 
         if (out_ids6) { out_ids6[0] = id.s; out_ids6[1] = id.e; out_ids6[2] = id.k1; out_ids6[3] = id.lasso_in; out_ids6[4] = id.lasso; out_ids6[5] = id.sum; }
     })
 }
+int hg_bfv_pk_configure(hg_circuit* c, size_t log2_size, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1_bounds, const uint64_t* r2_bounds,
+                        const uint64_t* p1_bounds, const uint64_t* p2_bounds, uint64_t u_bound, uint64_t e_bound, uint64_t k1_bound, hg_lasso_node* lasso_node,
+                        const hg_lasso_pp* lasso_pp, size_t lasso_num_vars, int* out_ids8) {
+    HG_TRY({
+        if (!c || !qis || !k0is || !r1_bounds || !r2_bounds || !p1_bounds || !p2_bounds || K < 1 || K > 4096) throw std::runtime_error("hg_bfv_pk_configure: bad arguments");
+        if (c->ctx) circuit_use_device(c);
+        if (c->ctx && !lasso_node) throw std::runtime_error("hg_bfv_pk_configure: a device circuit needs the Lasso node (hg_lasso_node_new)");
+        if (!c->ctx && !lasso_pp) throw std::runtime_error("hg_bfv_pk_configure: a host-only circuit needs the Lasso preprocessing and num_vars");
+        BfvPkCircuitParams P;
+        P.log2_size = log2_size; P.K = K; P.u_bound = u_bound; P.e_bound = e_bound; P.k1_bound = k1_bound;
+        P.qis.assign(qis, qis + K); P.k0is.assign(k0is, k0is + K); P.r1_bounds.assign(r1_bounds, r1_bounds + K); P.r2_bounds.assign(r2_bounds, r2_bounds + K);
+        P.p1_bounds.assign(p1_bounds, p1_bounds + K); P.p2_bounds.assign(p2_bounds, p2_bounds + K);
+        const BfvPkCircuitIds id = std::visit([&](auto& k) {
+            typedef std::remove_reference_t<decltype(k)> Ckt;
+            typedef field_t<Ckt> FP;
+            std::function<int()> ins;
+            if constexpr (std::is_same_v<Ckt, GkrCircuitDev<FP>>) ins = [&k, n = &typed<FP>(lasso_node)]() { return k.insert_lasso(n); };
+            else ins = [&]() { return k.insert_lasso(lasso_pp->pp, (int)lasso_num_vars); };
+            return bfv_pk_configure<FP::B_LIMBS>(k, P, ins);
+        }, c->c);
+        if (out_ids8) {
+            const int v[8] = {id.u, id.e0, id.e1, id.k1, id.lasso_in, id.lasso, id.sum0, id.sum1};
+            memcpy(out_ids8, v, sizeof v);
+        }
+    })
+}
 
 // ---- circuit-level API: Circuit::{insert, connect, evaluate} + prove_gkr
 int hg_circuit_new(hg_ctx* ctx, hg_circuit** out) {
@@ -1045,6 +1148,22 @@ int hg_bfv_witness_generate(hg_ctx* ctx, size_t n, size_t K, const uint64_t* qis
             throw std::runtime_error("hg_bfv_witness_generate: NULL argument");
         with_field(ctx->field_id, [&](auto fp) {
             witness_generate<decltype(fp)>(ctx, n, K, qis, k0is, r1_bounds, r2_bounds, s, e, k1, a, d_s, d_e, d_k1, d_ais, d_r1is, d_r2is, d_ct0is);
+        });
+    })
+}
+int hg_bfv_pk_witness_generate(hg_ctx* ctx, size_t n, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1_bounds, const uint64_t* r2_bounds,
+                               const uint64_t* p1_bounds, const uint64_t* p2_bounds, const int8_t* u, const int8_t* e0, const int8_t* e1, const int32_t* k1,
+                               const int64_t* pk0, const int64_t* pk1, void* d_u, void* d_e0, void* d_e1, void* d_k1, void* d_pk0is, void* d_pk1is, void* d_r1is,
+                               void* d_p1is, void* d_r2is, void* d_p2is, void* d_ct0is, void* d_ct1is) {
+    HG_TRY({
+        if (!ctx) throw std::runtime_error("hg_bfv_pk_witness_generate: NULL context");
+        void* const outs[12] = {d_u, d_e0, d_e1, d_k1, d_pk0is, d_pk1is, d_r1is, d_p1is, d_r2is, d_p2is, d_ct0is, d_ct1is};
+        bool null = !qis || !k0is || !r1_bounds || !r2_bounds || !p1_bounds || !p2_bounds || !u || !e0 || !e1 || !k1 || !pk0 || !pk1;
+        for (void* p : outs) null = null || !p;
+        if (null) throw std::runtime_error("hg_bfv_pk_witness_generate: NULL argument");
+        HG_CUDA(cudaSetDevice(ctx->dev.device));
+        with_field(ctx->field_id, [&](auto fp) {
+            pk_witness_generate<decltype(fp)>(ctx, n, K, qis, k0is, r1_bounds, r2_bounds, p1_bounds, p2_bounds, u, e0, e1, k1, pk0, pk1, outs);
         });
     })
 }

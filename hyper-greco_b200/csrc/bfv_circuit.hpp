@@ -144,4 +144,152 @@ template <int LIMBS, class Ckt> BfvCircuitIds bfv_configure(Ckt& c, const BfvCir
     return id;
 }
 
+// ---- BFV public-key encryption (Greco's second relation), for every modulus i < K over Z[x]:
+//   ct0_i = pk0_i u + e0 + k0_i k1 + r1_i q_i + r2_i (x^n + 1)
+//   ct1_i = pk1_i u + e1           + p1_i q_i + p2_i (x^n + 1)
+// The topology has no reference implementation: it is the SK circuit's, doubled where the relation doubles (DESIGN.md section 3,
+// assumption A12). Node insertion order fixes the input order, the output order and the proof bytes.
+struct BfvPkCircuitParams {
+    size_t log2_size = 0, K = 0;
+    std::vector<uint64_t> qis, k0is, r1_bounds, r2_bounds, p1_bounds, p2_bounds;
+    uint64_t u_bound = 0, e_bound = 0, k1_bound = 0;
+};
+struct BfvPkCircuitIds { int u = -1, e0 = -1, e1 = -1, k1 = -1, lasso_in = -1, lasso = -1, sum0 = -1, sum1 = -1; };
+
+template <int LIMBS, class Ckt> BfvPkCircuitIds bfv_pk_configure(Ckt& c, const BfvPkCircuitParams& P, const std::function<int()>& insert_lasso) {
+    typedef VanillaBuilder<LIMBS> VB;
+    const size_t L = P.log2_size, K = P.K, N2 = (size_t)1 << L;
+    if (L < 2 || K < 1 || P.qis.size() < K || P.k0is.size() < K || P.r1_bounds.size() < K || P.r2_bounds.size() < K || P.p1_bounds.size() < K ||
+        P.p2_bounds.size() < K)
+        throw std::runtime_error("bfv_pk_configure: bad parameters");
+    size_t log2K = 0;
+    while (((size_t)1 << log2K) < K) log2K++;
+    if (((size_t)1 << log2K) != K) throw std::runtime_error("bfv_pk_configure: K must be a power of two (the outputs are K blocks of 2n)");
+    BfvPkCircuitIds id;
+    id.u = c.insert_input(L, 1); id.e0 = c.insert_input(L, 1); id.e1 = c.insert_input(L, 1); id.k1 = c.insert_input(L, 1);
+    int e0s, e1s, k1kis;
+    {   // e0s, e1s: K copies of e0 / e1; k1kis: k1 * k0_i
+        VB a(1, L, 1), b(1, L, 1), d(1, L, 1);
+        for (size_t i = 0; i < K; i++)
+            for (size_t j = 0; j < N2; j++) { a.gate(false, 0, {{1, 0, j}}); b.gate(false, 0, {{1, 0, j}}); d.gate(false, 0, {{P.k0is[i], 0, j}}); }
+        e0s = c.insert_vanilla(a.d);
+        e1s = c.insert_vanilla(b.d);
+        k1kis = c.insert_vanilla(d.d);
+    }
+    c.connect(id.e0, e0s);
+    c.connect(id.e1, e1s);
+    c.connect(id.k1, k1kis);
+    std::vector<int> pk0is, pk1is, r1is, p1is;
+    for (size_t i = 0; i < K; i++) pk0is.push_back(c.insert_input(L, 1));
+    for (size_t i = 0; i < K; i++) pk1is.push_back(c.insert_input(L, 1));
+    for (size_t i = 0; i < K; i++) r1is.push_back(c.insert_input(L, 1));
+    for (size_t i = 0; i < K; i++) p1is.push_back(c.insert_input(L, 1));
+    int r1iqis, p1iqis;
+    {   // r1_i * q_i, p1_i * q_i
+        VB a(K, L, 1), b(K, L, 1);
+        for (size_t i = 0; i < K; i++) for (size_t j = 0; j < N2; j++) { a.gate(false, 0, {{P.qis[i], (uint32_t)i, j}}); b.gate(false, 0, {{P.qis[i], (uint32_t)i, j}}); }
+        r1iqis = c.insert_vanilla(a.d);
+        p1iqis = c.insert_vanilla(b.d);
+    }
+    for (int r : r1is) c.connect(r, r1iqis);
+    for (int p : p1is) c.connect(p, p1iqis);
+    const size_t n_log2 = L - 1, n = (size_t)1 << n_log2;
+    const int r2is = c.insert_input(n_log2, K), p2is = c.insert_input(n_log2, K);
+    const size_t q2_log2 = n_log2 + log2K;
+    // chunks of 2n of a quotient vector (K blocks of n), the SK circuit's chunking; for K = 1 the second half is zero padding
+    auto chunk = [&](int from, std::vector<int>& out) {
+        for (size_t start = 0; start < ((size_t)1 << q2_log2); start += N2) {
+            const size_t cnt = std::min(N2, ((size_t)1 << q2_log2) - start);
+            VB a(1, q2_log2, 1);
+            for (size_t j = 0; j < N2; j++) {
+                if (j < cnt) a.gate(false, 0, {{1, 0, start + j}});
+                else a.gate(true, 0, {});
+            }
+            const int nd = c.insert_vanilla(a.d);
+            c.connect(from, nd);
+            out.push_back(nd);
+        }
+    };
+    std::vector<int> r2_chunks, p2_chunks;
+    chunk(r2is, r2_chunks);
+    chunk(p2is, p2_chunks);
+    {   // every range-checked element shifted by its own vector's bound: r1is | p1is | r2 chunks | p2 chunks | u | e0 | e1 | k1. A chunk
+        // element at flat index f belongs to modulus f / n (modulus 0 for the zero padding of K = 1)
+        const size_t arity = 2 * K + r2_chunks.size() + p2_chunks.size() + 4;
+        VB a(arity, L, 1);
+        uint32_t in = 0;
+        auto whole = [&](uint64_t shift) { for (size_t j = 0; j < N2; j++) a.gate(true, shift, {{1, in, j}}); in++; };
+        auto chunks = [&](const std::vector<int>& ch, const std::vector<uint64_t>& bounds) {
+            for (size_t q = 0; q < ch.size(); q++, in++)
+                for (size_t j = 0; j < N2; j++) a.gate(true, bounds[std::min((q * N2 + j) / n, K - 1)], {{1, in, j}});
+        };
+        for (size_t i = 0; i < K; i++) whole(P.r1_bounds[i]);
+        for (size_t i = 0; i < K; i++) whole(P.p1_bounds[i]);
+        chunks(r2_chunks, P.r2_bounds);
+        chunks(p2_chunks, P.p2_bounds);
+        whole(P.u_bound); whole(P.e_bound); whole(P.e_bound); whole(P.k1_bound);
+        id.lasso_in = c.insert_vanilla(a.d);
+    }
+    id.lasso = insert_lasso();
+    for (int r : r1is) c.connect(r, id.lasso_in);
+    for (int p : p1is) c.connect(p, id.lasso_in);
+    for (int ch : r2_chunks) c.connect(ch, id.lasso_in);
+    for (int ch : p2_chunks) c.connect(ch, id.lasso_in);
+    c.connect(id.u, id.lasso_in); c.connect(id.e0, id.lasso_in); c.connect(id.e1, id.lasso_in); c.connect(id.k1, id.lasso_in);
+    c.connect(id.lasso_in, id.lasso);
+    const int u_eval = c.insert_fft(L, false);
+    c.connect(id.u, u_eval);
+    int u_copy;
+    {   // one claim on FFT(u), as s_copy gives the SK circuit
+        VB a(1, L, 1);
+        for (size_t j = 0; j < N2; j++) a.gate(false, 0, {{1, 0, j}});
+        u_copy = c.insert_vanilla(a.d);
+        c.connect(u_eval, u_copy);
+    }
+    // a relay of arity K over the products pk_i * u = IFFT(FFT(pk_i) . u_copy)
+    auto products = [&](const std::vector<int>& pks) {
+        VB b(K, L, 1);
+        for (size_t i = 0; i < K; i++) for (size_t j = 0; j < N2; j++) b.gate(false, 0, {{1, (uint32_t)i, j}});
+        const int par = c.insert_vanilla(b.d);
+        for (int pk : pks) {
+            const int pk_eval = c.insert_fft(L, false);
+            VB m(2, L, 1);
+            for (size_t j = 0; j < N2; j++) m.mul_gate(0, j, 1, j);
+            const int pku_eval = c.insert_vanilla(m.d);
+            const int pku = c.insert_fft(L, true);
+            c.connect(pk, pk_eval);
+            c.connect(u_copy, pku_eval);
+            c.connect(pk_eval, pku_eval);
+            c.connect(pku_eval, pku);
+            c.connect(pku, par);
+        }
+        return par;
+    };
+    const int pk0u_par = products(pk0is);
+    const int pk1u_par = products(pk1is);
+    auto cyclo = [&]() {  // q2_i * (x^n + 1): the n-1 coefficients of q2_i twice, each run followed by a zero
+        VB a(1, n_log2, K);
+        for (int half = 0; half < 2; half++) {
+            for (size_t j = 0; j + 1 < n; j++) a.gate(false, 0, {{1, 0, j}});
+            a.gate(true, 0, {});
+        }
+        return c.insert_vanilla(a.d);
+    };
+    const int cyclo0 = cyclo(), cyclo1 = cyclo();
+    c.connect(r2is, cyclo0);
+    c.connect(p2is, cyclo1);
+    {
+        VB a(5, L, K), b(4, L, K);
+        for (size_t j = 0; j < N2; j++) {
+            a.gate(false, 0, {{1, 0, j}, {1, 1, j}, {1, 2, j}, {1, 3, j}, {1, 4, j}});
+            b.gate(false, 0, {{1, 0, j}, {1, 1, j}, {1, 2, j}, {1, 3, j}});
+        }
+        id.sum0 = c.insert_vanilla(a.d);
+        id.sum1 = c.insert_vanilla(b.d);
+    }
+    c.connect(pk0u_par, id.sum0); c.connect(e0s, id.sum0); c.connect(k1kis, id.sum0); c.connect(r1iqis, id.sum0); c.connect(cyclo0, id.sum0);
+    c.connect(pk1u_par, id.sum1); c.connect(e1s, id.sum1); c.connect(p1iqis, id.sum1); c.connect(cyclo1, id.sum1);
+    return id;
+}
+
 }  // namespace hg

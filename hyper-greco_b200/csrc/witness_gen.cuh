@@ -168,4 +168,134 @@ __global__ void k_wit_small(WitGenParams P, const signed char* __restrict__ s, c
     wit_store<LIMBS>(ok1 + (size_t)t * LIMBS, vk, P.p);
 }
 
+// ---- BFV public-key encryption: the same arithmetic for two components per modulus,
+//   ct0_i = pk0_i u + e0 + k0_i k1 + r1_i q_i + r2_i (x^n + 1)      ct1_i = pk1_i u + e1 + p1_i q_i + p2_i (x^n + 1)
+//   k_wit_pk_conv    both exact products pk0_i * u and pk1_i * u over Z from one shared-memory tile of u: 2 (2n-1) n K integer MACs
+//   k_wit_pk_finish  per (i, coefficient) and component: + e (+ k0 k1 for ct0), reduction by x^n + 1, centred mod q, quotients,
+//                    bound checks, output layout
+//   k_wit_pk_small   the layout of u, e0, e1, k1
+struct WitGenPkStatus { WitGenStatus c[2]; };  // c[0]: ct0 (r1, r2), c[1]: ct1 (p1, p2)
+
+// hat0[i][k] = sum_j u[j] pk0[i][k - j], hat1 likewise, k = 0 .. 2n-2 (lowest degree first)
+__global__ void __launch_bounds__(HG_WIT_KT) k_wit_pk_conv(const signed char* __restrict__ u, const long long* __restrict__ pk0, const long long* __restrict__ pk1,
+                                                          int n, i128* __restrict__ hat0, i128* __restrict__ hat1) {
+    __shared__ signed char su[HG_WIT_JT];
+    __shared__ long long s0[HG_WIT_JT + HG_WIT_KT], s1[HG_WIT_JT + HG_WIT_KT];
+    const int i = blockIdx.y, k0 = blockIdx.x * HG_WIT_KT, k = k0 + threadIdx.x;
+    const long long* a0 = pk0 + (size_t)i * n;
+    const long long* a1 = pk1 + (size_t)i * n;
+    i128 acc0 = 0, acc1 = 0;
+    for (int j0 = 0; j0 < n; j0 += HG_WIT_JT) {
+        const int lo = k0 - j0 - HG_WIT_JT + 1;
+        for (int t = threadIdx.x; t < HG_WIT_JT; t += HG_WIT_KT) su[t] = j0 + t < n ? u[j0 + t] : 0;
+        for (int t = threadIdx.x; t < HG_WIT_JT + HG_WIT_KT - 1; t += HG_WIT_KT) {
+            const int idx = lo + t;
+            const bool in = idx >= 0 && idx < n;
+            s0[t] = in ? a0[idx] : 0;
+            s1[t] = in ? a1[idx] : 0;
+        }
+        __syncthreads();
+        long long part0 = 0, part1 = 0;  // |u pk| < 2^59 (checked by the caller): 16 taps fit a 64-bit partial sum before it is widened
+#pragma unroll 16
+        for (int t = 0; t < HG_WIT_JT; t++) {
+            const long long uv = su[t];
+            part0 += uv * s0[threadIdx.x + HG_WIT_JT - 1 - t];
+            part1 += uv * s1[threadIdx.x + HG_WIT_JT - 1 - t];
+            if ((t & 15) == 15) { acc0 += (i128)part0; acc1 += (i128)part1; part0 = 0; part1 = 0; }
+        }
+        __syncthreads();
+    }
+    if (k < 2 * n - 1) { hat0[(size_t)i * (2 * n) + k] = acc0; hat1[(size_t)i * (2 * n) + k] = acc1; }
+}
+
+struct WitGenPkParams {
+    int n, K;
+    long long q[64], k0[64], q1_bound[2][64], q2_bound[2][64];  // [component][i]: r1 / p1 and r2 / p2 bounds
+    u64 p[4];
+};
+// One component of one (modulus i, coefficient k < 2n): ct = (hat mod x^n + 1) centred mod q, q2 = the upper half of (ct - hat) centred,
+// q1 = (ct - hat - q2 (x^n + 1)) / q. `extra(c)` is the part of hat of degree < n added to the product (e, and k0 k1 for ct0).
+// Outputs: pk [N2] (padded), q1 [N2], q2 [n], ct [N2], in the layouts of k_wit_finish.
+template <int LIMBS, class Extra>
+__device__ __forceinline__ void wit_pk_component(const WitGenPkParams& P, int i, int k, const long long* __restrict__ pk, const i128* __restrict__ h, Extra extra,
+                                                 u64* __restrict__ opk, u64* __restrict__ oq1, u64* __restrict__ oq2, u64* __restrict__ oct,
+                                                 long long q1_bound, long long q2_bound, WitGenStatus* st) {
+    const int n = P.n, N2 = 2 * n;
+    const long long q = P.q[i];
+    auto hat_full = [&](int c) -> i128 { i128 v = h[c]; if (c < n) v += extra(c); return v; };
+    auto ct_at = [&](int c) -> i128 {
+        i128 red = hat_full(c);
+        if (c < n - 1) red -= hat_full(c + n);
+        return wit_center(red, q);
+    };
+    auto numc_at = [&](int c) -> i128 {
+        i128 v = -hat_full(c);
+        if (c < n) v += ct_at(c);
+        return wit_center(v, q);
+    };
+    if (k < n) {
+        wit_store<LIMBS>(opk + (size_t)(n - 1 - k) * LIMBS, (i128)pk[k], P.p);
+        wit_store<LIMBS>(opk + (size_t)(n + k) * LIMBS, 0, P.p);
+        wit_store<LIMBS>(oct + (size_t)((n - 1) + (n - 1 - k)) * LIMBS, ct_at(k), P.p);
+        if (k < n - 1) wit_store<LIMBS>(oct + (size_t)k * LIMBS, 0, P.p);
+        if (k == 0) wit_store<LIMBS>(oct + (size_t)(N2 - 1) * LIMBS, 0, P.p);
+    }
+    if (k == N2 - 1) {
+        wit_store<LIMBS>(oq1 + (size_t)(N2 - 1) * LIMBS, 0, P.p);
+        wit_store<LIMBS>(oq2 + (size_t)(n - 1) * LIMBS, 0, P.p);
+        return;
+    }
+    const i128 nc = numc_at(k);
+    i128 q2_hi = 0, q2_lo = 0;
+    if (k >= n) {
+        q2_hi = nc;
+        if ((q2_hi < 0 ? -q2_hi : q2_hi) > (i128)q2_bound) atomicAdd(&st->r2_out_of_range, 1u);
+        wit_store<LIMBS>(oq2 + (size_t)(n - 2 - (k - n)) * LIMBS, q2_hi, P.p);
+    } else if (k < n - 1) {
+        q2_lo = numc_at(k + n);
+        if (nc != q2_lo) atomicAdd(&st->not_multiple_of_cyclo, 1u);
+    } else {
+        if (nc != 0) atomicAdd(&st->not_multiple_of_cyclo, 1u);
+    }
+    i128 rem = -hat_full(k);
+    if (k < n) rem += ct_at(k);
+    rem -= (k >= n) ? q2_hi : q2_lo;
+    if (rem % (i128)q != 0) atomicAdd(&st->not_multiple_of_q, 1u);
+    const i128 q1 = rem / (i128)q;
+    if ((q1 < 0 ? -q1 : q1) > (i128)q1_bound) atomicAdd(&st->r1_out_of_range, 1u);
+    wit_store<LIMBS>(oq1 + (size_t)(N2 - 2 - k) * LIMBS, q1, P.p);
+}
+// one thread per (modulus i, coefficient k < 2n), both components. Outputs (LIMBS words per element, N2 = 2n):
+//   pk0is, pk1is, r1is, p1is, ct0is, ct1is [K][N2];  r2is, p2is [K][n]
+template <int LIMBS>
+__global__ void k_wit_pk_finish(WitGenPkParams P, const signed char* __restrict__ e0, const signed char* __restrict__ e1, const int* __restrict__ k1,
+                                const long long* __restrict__ pk0, const long long* __restrict__ pk1, const i128* __restrict__ hat0, const i128* __restrict__ hat1,
+                                u64* __restrict__ pk0is, u64* __restrict__ pk1is, u64* __restrict__ r1is, u64* __restrict__ p1is, u64* __restrict__ r2is,
+                                u64* __restrict__ p2is, u64* __restrict__ ct0is, u64* __restrict__ ct1is, WitGenPkStatus* st) {
+    const int n = P.n, N2 = 2 * n, i = blockIdx.y;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= N2) return;
+    const size_t wide = (size_t)i * N2 * LIMBS, narrow = (size_t)i * n * LIMBS;
+    const long long k0 = P.k0[i];
+    wit_pk_component<LIMBS>(P, i, k, pk0 + (size_t)i * n, hat0 + (size_t)i * N2, [&](int c) { return (i128)e0[c] + (i128)k1[c] * (i128)k0; },
+                            pk0is + wide, r1is + wide, r2is + narrow, ct0is + wide, P.q1_bound[0][i], P.q2_bound[0][i], &st->c[0]);
+    wit_pk_component<LIMBS>(P, i, k, pk1 + (size_t)i * n, hat1 + (size_t)i * N2, [&](int c) { return (i128)e1[c]; },
+                            pk1is + wide, p1is + wide, p2is + narrow, ct1is + wide, P.q1_bound[1][i], P.q2_bound[1][i], &st->c[1]);
+}
+// u: new_padded -> [u high..low | n zeros];  e0, e1, k1: new_shifted(v, 2n - 1) -> [n-1 zeros | v high..low | one zero]
+template <int LIMBS>
+__global__ void k_wit_pk_small(WitGenPkParams P, const signed char* __restrict__ u, const signed char* __restrict__ e0, const signed char* __restrict__ e1,
+                               const int* __restrict__ k1, u64* __restrict__ ou, u64* __restrict__ oe0, u64* __restrict__ oe1, u64* __restrict__ ok1) {
+    const int n = P.n, N2 = 2 * n;
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= N2) return;
+    i128 vu = 0, v0 = 0, v1 = 0, vk = 0;
+    if (t < n) vu = u[n - 1 - t];
+    if (t >= n - 1 && t < N2 - 1) { const int c = n - 1 - (t - (n - 1)); v0 = e0[c]; v1 = e1[c]; vk = k1[c]; }
+    wit_store<LIMBS>(ou + (size_t)t * LIMBS, vu, P.p);
+    wit_store<LIMBS>(oe0 + (size_t)t * LIMBS, v0, P.p);
+    wit_store<LIMBS>(oe1 + (size_t)t * LIMBS, v1, P.p);
+    wit_store<LIMBS>(ok1 + (size_t)t * LIMBS, vk, P.p);
+}
+
 }  // namespace hg

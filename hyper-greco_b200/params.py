@@ -88,3 +88,55 @@ def by_n(n: int) -> BfvSkEncryptConstants:
         if p.N == n:
             return p
     raise KeyError(n)
+
+
+# ----------------------------------------------------------------------------- public-key encryption
+@dataclass(frozen=True)
+class BfvPkEncryptConstants:
+    """Bounds of the BFV public-key-encryption relation (for every modulus i, over Z[x]):
+        ct0_i = pk0_i u + e0 + k0_i k1 + r1_i q_i + r2_i (x^n + 1)
+        ct1_i = pk1_i u + e1           + p1_i q_i + p2_i (x^n + 1)
+    Derived from the SK set of the same name (pk_from_sk)."""
+    name: str
+    N: int
+    E_BOUND: int
+    U_BOUND: int
+    K1_BOUND: int
+    R1_BOUNDS: tuple
+    R2_BOUNDS: tuple
+    P1_BOUNDS: tuple
+    P2_BOUNDS: tuple
+    QIS: tuple
+    K0IS: tuple
+
+    @property
+    def K(self) -> int:
+        return len(self.QIS)
+
+    @property
+    def N_LOG2(self) -> int:
+        return self.N.bit_length() - 1
+
+    @property
+    def log2_size(self) -> int:
+        return self.N_LOG2 + 1
+
+
+def quotient_bound(n: int, q: int, u_bound: int, e_bound: int, extra: int = 0) -> int:
+    """Bound on the q-quotient of pk u + e (+ extra) - ct: floor((n h U + E + extra + 2h) / q), h = (q - 1) / 2. With
+    extra = K1_BOUND k0_i it reproduces every SK R1_BOUNDS entry; with extra = 0 it is the PK P1 bound."""
+    h = (q - 1) // 2
+    return (n * h * u_bound + e_bound + extra + 2 * h) // q
+
+
+def pk_from_sk(sk: BfvSkEncryptConstants) -> BfvPkEncryptConstants:
+    """N, QIS, K0IS, E_BOUND, K1_BOUND as they are; U_BOUND = S_BOUND; R1 = SK R1; R2 = P2 = SK R2 (kept as given: at n = 32768
+    they differ from (q - 1) / 2 by the float rounding of the generator that produced them); P1 by quotient_bound."""
+    return BfvPkEncryptConstants(
+        name=sk.name, N=sk.N, E_BOUND=sk.E_BOUND, U_BOUND=sk.S_BOUND, K1_BOUND=sk.K1_BOUND,
+        R1_BOUNDS=sk.R1_BOUNDS, R2_BOUNDS=sk.R2_BOUNDS,
+        P1_BOUNDS=tuple(quotient_bound(sk.N, q, sk.S_BOUND, sk.E_BOUND) for q in sk.QIS), P2_BOUNDS=sk.R2_BOUNDS,
+        QIS=sk.QIS, K0IS=sk.K0IS)
+
+
+PK_PARAMS = {name: pk_from_sk(p) for name, p in PARAMS.items()}

@@ -292,6 +292,27 @@ int hg_bfv_configure(hg_circuit* c, size_t log2_size, size_t K, const uint64_t* 
 int hg_bfv_witness_generate(hg_ctx* ctx, size_t n, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1_bounds, const uint64_t* r2_bounds,
                             const int8_t* s, const int8_t* e, const int32_t* k1, const int64_t* a, void* d_s, void* d_e, void* d_k1, void* d_ais, void* d_r1is,
                             void* d_r2is, void* d_ct0is);
+/* ---- BFV PUBLIC-key encryption, Greco's second relation: for every modulus i < K over Z[x],
+ *        ct0_i = pk0_i u + e0 + k0_i k1 + r1_i q_i + r2_i (x^n + 1)      ct1_i = pk1_i u + e1 + p1_i q_i + p2_i (x^n + 1)
+ *      hg_bfv_pk_configure builds its circuit as hg_bfv_configure builds the SK one (same Lasso-node arguments), with the bounds of
+ *      the quotients p1 / p2 and of u added. The public pk coefficients are not range-checked. Node order (DESIGN.md section 3, A12):
+ *      inputs u, e0, e1, k1; pk0is.., pk1is.., r1is.., p1is..; r2is, p2is (n x K each). The Lasso node range-checks r1is | p1is |
+ *      r2 chunks | p2 chunks | u | e0 | e1 | k1, every element shifted by the bound of its own vector and modulus. Outputs in order:
+ *      the Lasso node, sum0 (= ct0is, K x 2n), sum1 (= ct1is). out_ids8 (may be NULL): node ids of u, e0, e1, k1, the Lasso node's
+ *      input layer, the Lasso node, sum0, sum1. */
+int hg_bfv_pk_configure(hg_circuit* c, size_t log2_size, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1_bounds, const uint64_t* r2_bounds,
+                        const uint64_t* p1_bounds, const uint64_t* p2_bounds, uint64_t u_bound, uint64_t e_bound, uint64_t k1_bound, hg_lasso_node* lasso_node,
+                        const hg_lasso_pp* lasso_pp, size_t lasso_num_vars, int* out_ids8);
+/* ---- synthetic witness of the public-key relation on the device, as hg_bfv_witness_generate for the SK one: exact products pk0_i u
+ *      and pk1_i u over Z, centred reductions, the quotients r1 / r2 (ct0) and p1 / p2 (ct1) with their bound checks, in the input
+ *      layout of hg_bfv_pk_configure. Host draws, lowest degree first: u in {-1,0,1}, e0, e1 as int8, k1 as int32, pk0 and pk1 as
+ *      [K][n] int64 with |pk| < 2^59. Device outputs in the library's representation:
+ *        d_u, d_e0, d_e1, d_k1: 2n elements;  d_pk0is, d_pk1is, d_r1is, d_p1is, d_ct0is, d_ct1is: K x 2n;  d_r2is, d_p2is: K x n.
+ *      A witness that does not satisfy the relation is an error naming the component (ct0 / ct1) and the quotient. */
+int hg_bfv_pk_witness_generate(hg_ctx* ctx, size_t n, size_t K, const uint64_t* qis, const uint64_t* k0is, const uint64_t* r1_bounds, const uint64_t* r2_bounds,
+                               const uint64_t* p1_bounds, const uint64_t* p2_bounds, const int8_t* u, const int8_t* e0, const int8_t* e1, const int32_t* k1,
+                               const int64_t* pk0, const int64_t* pk1, void* d_u, void* d_e0, void* d_e1, void* d_k1, void* d_pk0is, void* d_pk1is, void* d_r1is,
+                               void* d_p1is, void* d_r2is, void* d_p2is, void* d_ct0is, void* d_ct1is);
 /* ---- verifier: BfvEncrypt::verify (bfv-gkr/src/sk_encryption_circuit.rs:462-517) on the HOST, no GPU and no context.
  *      hg_circuit_new_host makes a circuit DESCRIPTION: the hg_circuit_insert_input / _fft / _vanilla / _connect calls above build it
  *      exactly as for a device circuit, the Lasso node is described by its preprocessing and num_vars (hg_circuit_insert_lasso_host);
