@@ -251,23 +251,29 @@ template <class FP> void evaluate_host(hg_circuit* hc, GkrCircuitDev<FP>& c, con
     DeviceCtx* dev = &hc->ctx->dev;
     const std::vector<size_t> lens = c.input_lens();
     if (n != lens.size()) throw std::runtime_error("evaluate: wrong number of inputs");
+    // every input starts 32-byte aligned in the arena: the layer kernels read a single input in place with 32-byte vector loads
+    // (load4 of gp_kernels.cuh), so an input after one of 1 or 2 Goldilocks entries must not follow it directly
+    const size_t al = std::max<size_t>(1, 32 / sizeof(B));
     size_t total = 0;
+    std::vector<size_t> offs(n);
     for (size_t i = 0; i < n; i++) {
         if (n_elems[i] != lens[i]) throw std::runtime_error("evaluate: input length does not match the input node");
-        total += lens[i];
+        offs[i] = total;
+        total += (lens[i] + al - 1) / al * al;
     }
-    if (hc->host_arena.n != total * sizeof(B)) hc->host_arena.alloc(total * sizeof(B));
+    if (hc->host_arena.n != total * sizeof(B)) {  // the padding between inputs is zero (and stays zero: only inputs are copied in)
+        hc->host_arena.alloc(total * sizeof(B));
+        HG_CUDA(cudaMemsetAsync(hc->host_arena.p, 0, total * sizeof(B), dev->stream));
+    }
     B* arena = (B*)hc->host_arena.p;  // all inputs back to back, in input-node order
     std::vector<const B*> v;
     // host vectors that are adjacent in memory (one pinned block, as a caller that wants speed lays them out) go in one copy.
     // Adjacent addresses can also belong to two separate page-locked allocations, for which one copy is invalid: then the
     // run is copied vector by vector.
-    size_t off = 0;
-    std::vector<size_t> offs(n);
-    for (size_t i = 0; i < n; i++) { offs[i] = off; v.push_back(arena + off); off += lens[i]; }
+    for (size_t i = 0; i < n; i++) v.push_back(arena + offs[i]);
     for (size_t i = 0; i < n;) {
         size_t k = i + 1, run_len = lens[i];
-        while (k < n && (const char*)in[k] == (const char*)in[i] + run_len * sizeof(B)) { run_len += lens[k]; k++; }
+        while (k < n && offs[k] == offs[i] + run_len && (const char*)in[k] == (const char*)in[i] + run_len * sizeof(B)) { run_len += lens[k]; k++; }
         cudaError_t e = cudaMemcpyAsync(arena + offs[i], in[i], run_len * sizeof(B), cudaMemcpyHostToDevice, dev->stream);
         if (e != cudaSuccess && k > i + 1) {
             cudaGetLastError();

@@ -38,6 +38,8 @@ template <class FP> class GkrCircuitDev {
     GkrCircuitDev(DeviceCtx* ctx, NttEngine<FP>* ntt) : ctx_(ctx), ntt_(ntt) {}
 
     int insert_input(size_t log2_size, size_t num_reps) {
+        // every table the sumchecks fold has a power-of-two length: num_reps 3 would make a 3 << log2_size input
+        if (num_reps < 1 || (num_reps & (num_reps - 1)) != 0) throw std::runtime_error("InputNode: num_reps must be a power of two");
         auto n = std::make_unique<Node>();
         n->kind = GKR_INPUT; n->out_len = num_reps << log2_size;
         nodes_.push_back(std::move(n));
@@ -66,6 +68,7 @@ template <class FP> class GkrCircuitDev {
         const size_t ng = d.n_gates, sub = (size_t)1 << d.log2_sub;
         // the CSR comes from the caller: validate it before it indexes host arrays here and device arrays in the kernels
         if (d.arity < 1 || d.arity > 4096 || d.log2_sub > 40 || d.num_reps < 1 || ng < 1) throw std::runtime_error("VanillaNode: bad shape");
+        if ((d.num_reps & (d.num_reps - 1)) != 0) throw std::runtime_error("VanillaNode: num_reps must be a power of two");
         if (d.add_ptr.size() != ng + 1 || d.mul_ptr.size() != ng + 1 || d.has_const.size() != ng) throw std::runtime_error("VanillaNode: CSR pointer arrays must have n_gates + 1 entries");
         if (d.add_ptr[0] != 0 || d.mul_ptr[0] != 0) throw std::runtime_error("VanillaNode: CSR pointers must start at 0");
         for (size_t g = 0; g < ng; g++)
@@ -83,7 +86,9 @@ template <class FP> class GkrCircuitDev {
         n.is_linear = n_mul == 0;
         n.is_elemmul = false;
         if (!n.is_linear) {
-            bool ok = d.arity == 2 && n_add == 0 && n_mul == ng && d.num_reps == 1;
+            // out[g] = in0[g] * in1[g] for EVERY wire g of the inputs: the product sumcheck runs over pad2(n_gates) entries and hands
+            // its point to the inputs, so it is exact only when the gates cover the inputs one to one; any other shape is general
+            bool ok = d.arity == 2 && n_add == 0 && n_mul == ng && d.num_reps == 1 && ng == sub;
             for (size_t g = 0; ok && g < ng; g++) {
                 ok = !d.has_const[g] && d.mul_ptr[g] == g && d.mul_in0[g] == 0 && d.mul_in1[g] == 1 && d.mul_w0[g] == g && d.mul_w1[g] == g &&
                      FP::b_eq(FP::b_from_limbs(&d.mul_coef[g * FP::B_LIMBS]), FP::b_one());
@@ -227,7 +232,12 @@ template <class FP> class GkrCircuitDev {
         NvtxSpan span("eval circuit");  // sk_encryption_circuit.rs:442
         cudaStream_t s = ctx_->stream;
         size_t next = 0;
-        for (auto& n : nodes_) if (n->kind == GKR_INPUT) { if (next >= inputs.size()) throw std::runtime_error("evaluate: too few inputs"); n->value_ptr = inputs[next++]; }
+        for (auto& n : nodes_) if (n->kind == GKR_INPUT) {
+            if (next >= inputs.size()) throw std::runtime_error("evaluate: too few inputs");
+            // a layer reads a single input in place with 32-byte vector loads
+            if ((uintptr_t)inputs[next] % 32 != 0) throw std::runtime_error("evaluate: every input must start 32-byte aligned");
+            n->value_ptr = inputs[next++];
+        }
         if (next != inputs.size()) throw std::runtime_error("evaluate: too many inputs");
         plan_evaluate();
         for (auto& lvl : eval_levels_) {
@@ -340,6 +350,7 @@ template <class FP> class GkrCircuitDev {
   private:
     struct Claim { bool by_index; size_t idx; std::vector<X> point_host; int nvars; std::shared_ptr<X> value; };
     std::vector<std::vector<Claim>> pending_claims_;
+    std::vector<Claim> general_u_claims_;  // phase 1's claims of the general layer being enqueued (run_job)
     size_t msg_budget_ = 0;
     // the claims that reached the input nodes (what verify() checks, sk_encryption_circuit.rs:512-516), after the messages are on the host
     std::vector<std::vector<InputClaim>> collect() {
@@ -573,12 +584,23 @@ template <class FP> class GkrCircuitDev {
         job.evals_off = ch.alloc_msg(n_ev);  // after the rounds: in interactive mode earlier slots have already been downloaded
         if (mode == kModeInteractive) launch_finals(ch, {job});
         // new claims on the predecessors: (point = the round challenges restricted to the input's variables, value = its evaluation)
+        // A general layer gives input slot k its phase-1 claim and then its phase-2 claim before slot k + 1 gets any, as the
+        // verifier reads them: the order matters when one node fills several slots. Phase 1's claims wait for phase 2's.
         const int in_vars = lin(n) ? log2sz(n.n_in) : job.nv;
         std::vector<std::shared_ptr<X>> outv;
+        std::vector<Claim> mine;
         for (int k = 0; k < n_ev; k++) {
             Claim c; c.by_index = true; c.idx = job.r0_idx; c.nvars = in_vars; c.value = std::make_shared<X>(FP::x_zero());
             outv.push_back(c.value);
-            pending_claims_[n.preds.at(k)].push_back(c);
+            mine.push_back(c);
+        }
+        if (n.is_general && job.phase == 0) {
+            general_u_claims_ = mine;
+        } else {
+            for (int k = 0; k < n_ev; k++) {
+                if (job.phase == 1) pending_claims_[n.preds.at(k)].push_back(general_u_claims_.at(k));
+                pending_claims_[n.preds.at(k)].push_back(mine[k]);
+            }
         }
         {
             const size_t eo = job.evals_off;

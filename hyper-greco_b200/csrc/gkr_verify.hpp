@@ -76,6 +76,7 @@ template <class FP> class GkrVerifierHost {
     struct Claim { std::vector<X> point; X value; };
 
     int insert_input(size_t log2_size, size_t num_reps) {
+        if (num_reps < 1 || (num_reps & (num_reps - 1)) != 0) throw VerifyError("InputNode: num_reps must be a power of two");
         Node n;
         n.kind = GKR_INPUT; n.out_len = num_reps << log2_size;
         nodes_.push_back(std::move(n));
@@ -98,6 +99,7 @@ template <class FP> class GkrVerifierHost {
         const size_t ng = d.n_gates, sub = (size_t)1 << d.log2_sub;
         if (d.arity < 1 || d.num_reps < 1 || ng < 1 || d.add_ptr.size() != ng + 1 || d.mul_ptr.size() != ng + 1 || d.has_const.size() != ng)
             throw VerifyError("VanillaNode: bad descriptor");
+        if ((d.num_reps & (d.num_reps - 1)) != 0) throw VerifyError("VanillaNode: num_reps must be a power of two");
         const size_t n_add = d.add_ptr[ng], n_mul = d.mul_ptr[ng];
         for (size_t g = 0; g < ng; g++) if (d.add_ptr[g + 1] < d.add_ptr[g] || d.mul_ptr[g + 1] < d.mul_ptr[g]) throw VerifyError("VanillaNode: CSR pointers must be non-decreasing");
         for (size_t e = 0; e < n_add; e++) if (d.add_in[e] >= d.arity || d.add_wire[e] >= sub) throw VerifyError("VanillaNode: edge outside the inputs");
@@ -110,7 +112,7 @@ template <class FP> class GkrVerifierHost {
         n.a_pad = pad2(d.arity);
         n.is_linear = n_mul == 0;
         if (!n.is_linear) {
-            bool ok = d.arity == 2 && n_add == 0 && n_mul == ng && d.num_reps == 1;
+            bool ok = d.arity == 2 && n_add == 0 && n_mul == ng && d.num_reps == 1 && ng == sub;  // the prover's rule (gkr_dev.cuh)
             for (size_t g = 0; ok && g < ng; g++)
                 ok = !d.has_const[g] && d.mul_ptr[g] == g && d.mul_in0[g] == 0 && d.mul_in1[g] == 1 && d.mul_w0[g] == g && d.mul_w1[g] == g &&
                      FP::b_eq(FP::b_from_limbs(&d.mul_coef[g * FP::B_LIMBS]), FP::b_one());

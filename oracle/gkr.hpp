@@ -51,8 +51,10 @@ template <class F> struct GkrNode {
         while (p < n) p <<= 1;
         return p;
     }
-    bool elementwise_mul() const {  // the only multiplicative layer of the circuit: out[i] = in0[i] * in1[i] (:246-250)
-        if (kind != NODE_VANILLA || arity != 2) return false;
+    // the only multiplicative layer of the circuit: out[i] = in0[i] * in1[i] (:246-250), one gate per input wire and num_reps 1. With
+    // fewer gates than wires the product sumcheck would prove a sum that misses the unread wires, at a point shorter than the inputs'.
+    bool elementwise_mul() const {
+        if (kind != NODE_VANILLA || arity != 2 || num_reps != 1 || gates.size() != ((size_t)1 << log2_sub_input)) return false;
         for (size_t i = 0; i < gates.size(); i++) {
             auto& g = gates[i];
             if (g.has_const || !g.adds.empty() || g.muls.size() != 1) return false;

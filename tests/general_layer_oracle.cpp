@@ -1,6 +1,6 @@
 // TEST INFRASTRUCTURE ONLY (tests/test_general_layer.py compiles it with g++ next to the oracle; the product never links it).
 // An independent CPU restatement of general Vanilla layers: any layer with a product term other than the element-wise shape
-// out[i] = in0[i] * in1[i] (num_reps 1). It follows Libra's two-phase layer sumcheck as DESIGN.md section 7b states it
+// out[i] = in0[i] * in1[i] over every input wire (num_reps 1). It follows Libra's two-phase layer sumcheck as DESIGN.md section 7b states it
 // (assumption A11) and reuses the oracle (oracle/gkr.hpp) for every other node shape, the transcript and the sumcheck.
 // A C entry builds a generic circuit node by node: insert input / vanilla (the CSR of hg_circuit_insert_vanilla) / fft, connect,
 // evaluate, prove_gkr, verify_gkr, for both fields.
@@ -34,7 +34,7 @@ template <class F> struct GeneralCircuit {
     typedef hgo::Circuit<F> C;
     C c;
 
-    bool general(const GkrNode<F>& nd) const { return nd.kind == NODE_VANILLA && !nd.linear() && !(nd.num_reps == 1 && nd.elementwise_mul()); }
+    bool general(const GkrNode<F>& nd) const { return nd.kind == NODE_VANILLA && !nd.linear() && !nd.elementwise_mul(); }
     // fn(output index, coefficient, x, y) for every gate, rep and product term; x = (in0, r sub + w0), y = (in1, r sub + w1)
     // are positions in the concatenated inputs
     template <class Fn> static void for_each_product(const GkrNode<F>& nd, size_t n_in, Fn fn) {
@@ -155,11 +155,13 @@ template <class F> struct SessionT : Session {
     GeneralCircuit<F> g;
     std::vector<std::vector<F>> val;
     std::vector<std::vector<EvalClaim<F>>> claims;
-    int insert_input(int log2_size, int reps) override { return g.c.insert(BfvEncrypt<F>::input(log2_size, reps)); }
+    static void check_reps(int reps) { if (reps < 1 || (reps & (reps - 1)) != 0) throw OracleError("num_reps must be a power of two"); }
+    int insert_input(int log2_size, int reps) override { check_reps(reps); return g.c.insert(BfvEncrypt<F>::input(log2_size, reps)); }
     int insert_fft(int log2_size, bool inverse) override { return g.c.insert(BfvEncrypt<F>::fft(log2_size, inverse)); }
     int insert_vanilla(int arity, int log2_sub, int reps, size_t ng, const uint8_t* has_const, const uint64_t* consts, const uint64_t* add_ptr,
                        const uint64_t* add_coef, const uint32_t* add_in, const uint64_t* add_wire, const uint64_t* mul_ptr, const uint64_t* mul_coef,
                        const uint32_t* mul_in0, const uint64_t* mul_w0, const uint32_t* mul_in1, const uint64_t* mul_w1) override {
+        check_reps(reps);
         std::vector<VanillaGate<F>> gates(ng);
         for (size_t q = 0; q < ng; q++) {
             VanillaGate<F>& gt = gates[q];
